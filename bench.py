@@ -3,6 +3,7 @@
 nonzeros*K per second, whole job over N GPUs, plus roofline and CPU baseline.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c2|c3|c1] [--impl ours|reference]
+                  [--dump-outputs DIR]
 
 Workload at the default (`c4`, BASELINE.json configs[3], the configuration the north-star target is
 quoted on): scRNA-seq shaped CSR counts, D=20,000 genes, ~5 % density, K=32, S=4 draws, 8,192
@@ -43,6 +44,33 @@ WORKLOADS = {
 # rows of the workload the float64 CPU port is timed on (C4: the reference formulation materialises ~20
 # (S,B,D) float64 tensors, 1 GB each at 1,536 rows; 8,192 rows would need ~100 GB)
 CPU_SAMPLE_ROWS = {"c4": 1536, "c3": 2000, "c2": 5000, "c1": 1000}
+DUMP_BYTES = 64 * 10 ** 6           # --dump-outputs: all files together stay below this
+
+
+def step_outputs(eng, loss):
+    """What a caller of `elbo_step` holds after a step, as host float32 / float64 arrays: the returned loss,
+    the (S,16) energy terms per draw, and the 24 variational tensors with the gradient the step applied to
+    them (reference shapes, '/' in a name becomes '.')."""
+    out = {"loss": loss.detach().double().cpu().numpy(), "parts": eng.ws.parts.view(eng.S, -1).cpu().numpy()}
+    for prefix, flat in (("param", eng.params), ("grad", eng.grads)):
+        for k, v in eng.layout.views(flat).items():
+            out[prefix + "." + k.replace("/", ".")] = v.detach().float().cpu().numpy()
+    return out
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """Writes every array as <out_dir>/<name>.npy.  If together they exceed DUMP_BYTES, every array keeps the
+    same share of its elements, flattened, at positions drawn by a generator seeded with `seed` (same shapes:
+    same positions, so two runs compare element for element)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    share = min(1.0, 0.99 * (DUMP_BYTES - 256 * len(arrays)) / max(total, 1))
+    for name, a in arrays.items():
+        if share < 1.0:
+            idx = np.sort(np.random.default_rng(seed).choice(a.size, max(1, int(a.size * share)), replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler(threading.Thread):
@@ -196,7 +224,14 @@ def main():
     ap.add_argument("--S", type=int, default=None, help="override the number of Monte-Carlo draws")
     ap.add_argument("--hot-density", type=float, default=None,
                     help="column population threshold of the tensor-core hot block (0 = gather kernels only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (loss, energy terms, parameters, gradients; "
+                         "last e2e loss) as DIR/<name>.npy, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     wl = dict(WORKLOADS[args.workload])
     if args.K:
         wl["K"] = args.K
@@ -255,8 +290,10 @@ def main():
         torch.cuda.synchronize()
 
     def run_steps(n, get_batch, lr):
+        loss = None
         for i in range(n):
-            model.elbo_step({"counts": get_batch(i)}, S, learning_rate=lr, variant=args.variant)
+            loss = model.elbo_step({"counts": get_batch(i)}, S, learning_rate=lr, variant=args.variant)
+        return loss
 
     # ------------------------------------------------ device-resident: `value`
     run_steps(args.warmup, lambda i: batches[i % len(batches)], args.lr)
@@ -271,11 +308,13 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     torch.cuda.nvtx.range_push("spmf_timed")
     e0.record()
-    run_steps(args.steps, lambda i: batches[(args.warmup + i) % len(batches)], args.lr)
+    last_loss = run_steps(args.steps, lambda i: batches[(args.warmup + i) % len(batches)], args.lr)
     e1.record()
     torch.cuda.nvtx.range_pop()
     barrier()
     ms = e0.elapsed_time(e1)
+    # copied before the instrumented pass below steps the model further
+    outputs = step_outputs(eng, last_loss) if args.dump_outputs and rank == 0 else None
     launches = eng.launches - launches0
     graph_replays = eng.graph_launches - graphs0
     # per-kernel timings for the roofline: a short instrumented pass AFTER the timed region (CUDA events
@@ -501,6 +540,9 @@ def main():
             "gpu_launches": launches, "graph_replays": graph_replays, "graphs_primed": primed,
             "clocks": clk, "roofline": roofline, "cpu_baseline": cpu,
         }))
+    if outputs is not None:
+        outputs["e2e_loss"] = np.array(losses_read[-1], dtype=np.float64)
+        dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.destroy_process_group()
 
