@@ -209,11 +209,12 @@ int spmf_dense_fill(const float* x, int nrows, int D, const long long* rowptr, i
 /* ---- hybrid path: tcgen05 tensor-core GEMMs on the dense hot-column block + gathers elsewhere ----
  * The two products of the step that touch the counts only (encode x.A', poisson.py:640-643, and its
  * transpose GA' = x^T.dzr in the backward) run on the 5th-gen tensor cores for the H most
- * populated columns; the per-nonzero terms (rate, x/rate) stay on the gather kernels.
+ * populated columns; so do the per-nonzero terms (rate, x/rate) of that block (spmf_hot_tile below),
+ * while the gather kernels handle the remaining entries.
  * Column order: `rank[d]` = table row of feature d (descending column population), so the hot block
  * is rows [0,H) of every operand table.  All *_ranked entry points take rank == NULL as identity. */
-/* 0: none; 2: GEMMs + fused tile kernel (KP in {8,16,32}, REC = KP*SV in {32,64,128});
- * 1: GEMMs only (KP = 64 or 128, wider records run as blocks of 128 channels) */
+/* 0: gather kernels, 2: tile-hybrid (GEMMs + fused tile kernel; KP in {8,16,32} with REC = KP*SV in
+ * {32,64,128}, or KP in {64,128}) */
 int spmf_hybrid_supported(int K, int S);
 int spmf_draw_operands_ranked(const float* params, const float* noise, const float* eta, const int* rank,
                               int D, int K, int S, float* Ap, float* EV, float* PH, double* vsum,
@@ -239,13 +240,13 @@ int spmf_umma_tile_a(const void* src_bf16, long long ld, int M, int Kd, void* ds
 /* CSR batch (original column ids) -> ranked + partitioned CSR (zero-based rowptr_out[nrows+1]; per row
  * the entries covered by the tensor-core products first, stored with a NEGATIVE value as their flag,
  * the others from rowmid[row] on) and the dense hot block as UMMA-tiled bf16: xhot = X[nrows][Hp]
- * (every element of the 128-row-padded block is written here) and, if xthot != NULL, its transpose xthot = X^T[H][Bp] (Hp = ceil64(H),
- * Bp = ceil64(nrows); sizes from spmf_umma_tiled_a_elems).  The step itself needs xhot only.  Covered = rank < H and the count is exactly
- * representable in bf16.  rowsum / lgam (both or neither): also emit the per-row constants of
- * spmf_csr_row_consts in the same pass. */
+ * (Hp = ceil64(H); every element of the 128-row-padded block is written here; size from
+ * spmf_umma_tiled_a_elems).  Covered = rank < H and the count is exactly representable in bf16.
+ * rowsum / lgam (both or neither): also emit the per-row constants of spmf_csr_row_consts in the same
+ * pass. */
 int spmf_hot_split(const long long* rowptr, const int* cols, const float* vals, int nrows, long long nnz,
                    const int* rank, int H, long long* rowptr_out, int* cols_out, float* vals_out, int* rowmid,
-                   void* xhot, void* xthot, float* rowsum, float* lgam, void* stream);
+                   void* xhot, float* rowsum, float* lgam, void* stream);
 /* the same, reading the 2-byte transfer format directly (spmf_csr_unpack8 fused in: column-gap bytes, count
  * bytes, sorted overflow list; entry indices relative to rowptr[0]) */
 int spmf_hot_split_u8(const long long* rowptr, const unsigned char* gaps8, const unsigned char* vals8,
@@ -256,7 +257,7 @@ int spmf_hot_split_u8(const long long* rowptr, const unsigned char* gaps8, const
  * cols / cols16 and one of vals / vals16 is non-NULL */
 int spmf_hot_split_packed(const long long* rowptr, const int* cols, const unsigned short* cols16, const float* vals,
                           const unsigned short* vals16, int nrows, long long nnz, const int* rank, int H,
-                          long long* rowptr_out, int* cols_out, float* vals_out, int* rowmid, void* xhot, void* xthot,
+                          long long* rowptr_out, int* cols_out, float* vals_out, int* rowmid, void* xhot,
                           float* rowsum, float* lgam, void* stream);
 /* Direct dense ingest: a dense [nrows][D] batch of counts in FEATURE order (dtype SPMF_DENSE_*) -> the hybrid
  * form without a CSR round trip: xhot = the UMMA-tiled bf16 block of the H hot columns (rank order), the row
@@ -288,19 +289,6 @@ int spmf_umma_gemm3_at(const void* X, int x_kd, int x_rows, int M, const void* B
 int spmf_umma_probe(const void* a_img, int a_bytes, const void* b_img, int b_bytes, int M, int N, int a_mn,
                     int b_mn, int lbo_a, int sbo_a, int step_a, int lbo_b, int sbo_b, int step_b, int nk,
                     float* out, void* stream);
-/* row / column passes of the hybrid step (same outputs as spmf_csr_rows / spmf_csc_cols): `z` must
- * hold the GEMM's un-scaled hot block of x.A' on entry; GA' of covered entries is left to the GEMM. */
-int spmf_csr_rows_hybrid(const long long* rowptr, const int* cols, const float* vals, const int* rowmid,
-                         const float* rowsum, const float* lgam, float inv_xi, int scale_rows, int nrows,
-                         int D, int K, int S, const float* Ap, const float* EV, const float* PH,
-                         const double* vsum, float* z, float* dzr, float* rowacc, void* gs, void* stream);
-/* column pass over the two CSC copies of a hot-split batch: `hot_*` holds the covered entries (GEV and
- * Gphi only -- their GA' comes from the GEMM), `cold_*` the rest (full column pass).  Zeroes the three
- * tables first.  nnz_bound >= either copy's count (the counts themselves are colptr[D], device side). */
-int spmf_csc_cols_hybrid(const int* hot_colptr, const int* hot_rows, const float* hot_vals,
-                         const int* cold_colptr, const int* cold_rows, const float* cold_vals, int nnz_bound,
-                         int nrows, int D, int K, int S, const float* z, const float* dzr, const float* EV,
-                         const float* PH, float* GAp, float* GEVnz, float* Gphinz, void* stream);
 /* ---- tile-hybrid step: the per-nonzero terms of the hot block on the tensor cores as well ----
  * spmf_hot_tile fuses, per 128-row x 64-column tile and draw: rate = z.EV + phi (tcgen05.mma into
  * tensor memory), x log rate and w = x/rate on the CUDA cores, then dz += w.EV and GEV = w^T.z,
@@ -318,13 +306,14 @@ int spmf_hot_tile(const void* xhot, const void* EVt, const float* z, int nrows, 
                   float* dzacc, float* rowacc, float* GEVnz, float* Gphinz, void* gs, void* stream);
 int spmf_rows_finish(const float* rowsum, const float* lgam, float inv_xi, int scale_rows, int nrows, int K, int S,
                      const double* vsum, const float* z, float* dzr, float* rowacc, void* gs, void* stream);
-/* the pieces of spmf_csc_cols_hybrid, for callers that overlap them on several streams: zero the three
- * column-gradient tables; accumulate (atomics) one CSC copy into them -- covered != 0: GEV and Gphi
- * only (hot copy), covered == 0: full column pass (cold copy). */
+/* column side of the tile-hybrid step, in pieces that callers overlap on several streams: zero the three
+ * column-gradient tables; accumulate (atomics) the CSC copy of the uncovered entries into them (full
+ * column pass; GA' of the covered entries comes from spmf_umma_gemm3_at).  nnz_bound >= the copy's count
+ * (the count itself is colptr[D], device side). */
 int spmf_zero_col_grads(float* GAp, float* GEVnz, float* Gphinz, int D, int K, int S, void* stream);
 int spmf_csc_cols_accum(const int* colptr, const int* rows, const float* vals, int nnz_bound, int nrows, int D,
                         int K, int S, const float* z, const float* dzr, const float* EV, const float* PH,
-                        float* GAp, float* GEVnz, float* Gphinz, int covered, void* stream);
+                        float* GAp, float* GEVnz, float* Gphinz, void* stream);
 /* CSC copy of ONE part of a partitioned CSR (spmf_hot_split): part 0 = the first rowmid[r] entries of
  * every row, part 1 = the rest; values are stored as |x|.  rowmid == NULL: whole rows. */
 int spmf_csr_to_csc_part(const long long* rowptr, const int* rowmid, int part, const int* cols, const float* vals,
@@ -390,24 +379,21 @@ typedef struct spmf_step_args {
   void *caller_stream, *hot_stream, *side_stream;
   void *ev_fork, *ev_join, *ev_done;
   void *ev_rows0, *ev_rows1, *ev_cols0, *ev_cols1;
-  /* hybrid path (hot_cols > 0): rowptr/cols/vals/colptr/crows/cvals above are the ranked, partitioned
-   * arrays of spmf_hot_split (rowptr zero-based); rank maps feature -> table row */
+  /* hybrid path (hot_cols > 0): rowptr/cols/vals above are the ranked, partitioned CSR of spmf_hot_split
+   * (rowptr zero-based) and colptr/crows/cvals the CSC of its uncovered entries; rank maps feature -> table row */
   const int* rank;
   int hot_cols, gemm_splits;
   long long t3_qstride;            /* elements between draw groups in ApT3 / dzrT3 */
   const int* rowmid;
-  const int *hot_colptr, *hot_crows;   /* CSC of the covered entries (colptr/crows/cvals above: the rest) */
-  const float* hot_cvals;
-  const void *xhot, *xthot;        /* UMMA-tiled bf16 hot block (spmf_hot_split); xthot is unused (may be NULL) */
+  const void* xhot;                /* UMMA-tiled bf16 hot block (spmf_hot_split) */
   void *ApT3, *dzrT3;              /* UMMA-tiled bf16 B3 workspaces, [NQ] x spmf_umma_tiled_b_elems */
   void *ev_gemm0, *ev_gemm1;       /* optional events around the tensor-core launches of the column side */
   /* optional: two more streams (+ three events) on which the GA' GEMM and the cold column pass run
-   * concurrently with the hot column pass; NULL = everything in order on the hot stream */
+   * concurrently; NULL = everything in order on the hot stream */
   void *aux_stream1, *aux_stream2;
   void *ev_aux_fork, *ev_aux_join1, *ev_aux_join2;
-  /* hot_mode 2: the per-nonzero terms of the hot block run in the fused tcgen05 tile kernel
-   * (spmf_hot_tile) instead of the gather kernels; EVt = workspace of spmf_hot_tile_scratch_bytes */
-  int hot_mode;
+  /* the per-nonzero terms of the hot block run in the fused tcgen05 tile kernel (spmf_hot_tile);
+   * EVt = its workspace of spmf_hot_tile_scratch_bytes (required when hot_cols > 0) */
   void* EVt;
   void *ev_tile0, *ev_tile1;       /* optional events around spmf_hot_tile (bench instrumentation) */
   /* split backward: with scr_dpre (a second double scratch of spmf_backward_scratch_doubles) and

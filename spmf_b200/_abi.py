@@ -85,13 +85,11 @@ _SIGS = {
     "spmf_umma_tile_a": (i32, [p, i64, i32, i32, p, p]),
     "spmf_umma_gemm3_at": (i32, [p, i32, i32, i32, p, i64, p, i64, i64, i32, i32, i32, p]),
     "spmf_umma_probe": (i32, [p, i32, p, i32, i32, i32, i32, i32, i32, i32, i32, i32, i32, i32, i32, p, p]),
-    "spmf_hot_split": (i32, [p, p, p, i32, i64, p, i32, p, p, p, p, p, p, p, p, p]),
+    "spmf_hot_split": (i32, [p, p, p, i32, i64, p, i32, p, p, p, p, p, p, p, p]),
     "spmf_hot_split_u8": (i32, [p, p, p, p, p, i32, i32, p, i32, p, p, p, p, p, p, p, p]),
-    "spmf_hot_split_packed": (i32, [p, p, p, p, p, i32, i64, p, i32, p, p, p, p, p, p, p, p, p]),
+    "spmf_hot_split_packed": (i32, [p, p, p, p, p, i32, i64, p, i32, p, p, p, p, p, p, p, p]),
     "spmf_split3_transpose": (i32, [p, i64, i64, i32, i32, i32, p, i64, i32, p]),
     "spmf_umma_gemm3": (i32, [p, i64, i32, p, i64, p, i64, i64, i32, i32, i32, i32, p]),
-    "spmf_csr_rows_hybrid": (i32, [p, p, p, p, p, p, f32, i32, i32, i32, i32, i32, p, p, p, p, p, p, p, p, p]),
-    "spmf_csc_cols_hybrid": (i32, [p, p, p, p, p, p, i32, i32, i32, i32, i32, p, p, p, p, p, p, p, p]),
     "spmf_hot_tile_scratch_bytes": (i64, [i32, i32, i32]),
     "spmf_hot_ev_tiles": (i32, [p, p, i32, i32, i32, i32, p, p]),
     "spmf_csr_rows_cold": (i32, [p, p, p, p, p, f32, i32, i32, i32, i32, i32, p, p, p, p, p, p, p, p]),
@@ -110,7 +108,7 @@ _SIGS = {
     "spmf_guard_rows_fix_dense": (i32, [p, i32, p, p, p, f32, i32, i32, i32, i32, i32, p, p, p, p, p, p, p, p]),
     "spmf_dense_hot_split": (i32, [p, i32, i32, i32, p, i32, p, p, p, p, p, p, p, p]),
     "spmf_zero_col_grads": (i32, [p, p, p, i32, i32, i32, p]),
-    "spmf_csc_cols_accum": (i32, [p, p, p, i32, i32, i32, i32, i32, p, p, p, p, p, p, p, i32, p]),
+    "spmf_csc_cols_accum": (i32, [p, p, p, i32, i32, i32, i32, i32, p, p, p, p, p, p, p, p]),
     "spmf_csr_to_csc_part": (i32, [p, p, i32, p, p, i32, i32, p, p, p, p, p]),
 }
 
@@ -152,10 +150,10 @@ class StepArgs(C.Structure):
                             "ev_rows0", "ev_rows1", "ev_cols0", "ev_cols1")]
         + [("rank", p), ("hot_cols", i32), ("gemm_splits", i32)]
         + [("t3_qstride", i64)]
-        + [(n, p) for n in ("rowmid", "hot_colptr", "hot_crows", "hot_cvals", "xhot", "xthot", "ApT3", "dzrT3",
+        + [(n, p) for n in ("rowmid", "xhot", "ApT3", "dzrT3",
                             "ev_gemm0", "ev_gemm1", "aux_stream1", "aux_stream2", "ev_aux_fork", "ev_aux_join1",
                             "ev_aux_join2")]
-        + [("hot_mode", i32), ("EVt", p), ("ev_tile0", p), ("ev_tile1", p), ("scr_dpre", p), ("ev_noise", p)]
+        + [("EVt", p), ("ev_tile0", p), ("ev_tile1", p), ("scr_dpre", p), ("ev_noise", p)]
         + [("link", i32), ("gs", p), ("xdense", p), ("xdense_in", p), ("step_state", p), ("model", i32), ("state_preset", i32), ("dense_raw", p), ("dense_raw_dtype", i32), ("adam_tail_early", i32)]
     )
 

@@ -631,12 +631,7 @@ static int launch_hot_tile(const void* xhot, const void* EVt, const float* z, in
   }
   // one CTA per SM: cut the hot columns into ranges so that the grid is several waves of 148 CTAs
   const int nch = (H + 63) / 64, items = ((nrows + 127) / 128) * S;
-  static int waves = 0;                    // SPMF_TILE_WAVES: tuning knob (default 6 waves of CTAs)
-  if (!waves) {
-    const char* e = getenv("SPMF_TILE_WAVES");
-    waves = e ? atoi(e) : 6;
-    if (waves < 1) waves = 6;
-  }
+  constexpr int waves = 6;
   int splits = (waves * 148 + items - 1) / items;
   if (splits > nch) splits = nch;
   if (splits < 1) splits = 1;

@@ -142,14 +142,13 @@ __device__ __forceinline__ void ld_idx(const int* __restrict__ pc, const float* 
   }
 }
 
-// MODE 0: training row pass.  MODE 1: encode only (z).  MODE 2: hybrid -- the hot-column block of
-// the encode product already sits in z (tcgen05 GEMM, spmf_umma.cu); sweep 1 adds the entries the
-// GEMM does not cover (stored after rowmid[row], positive values) and sweep 2 runs over every entry
-// (covered ones carry a negative sign as their flag).
-// MODE 3: cold part of the tile-hybrid step -- as MODE 2, but sweep 2 also skips the covered entries
-// (the tcgen05 tile kernel, spmf_hot_tile.cu, owns them) and dzr / rowacc receive RAW partial sums
-// (un-scaled sum w.EV, sum x log lambda, #non-finite) that spmf_rows_finish completes.
-constexpr int kRowsTrain = 0, kRowsEncode = 1, kRowsHybrid = 2, kRowsCold = 3;
+// MODE 0: training row pass.  MODE 1: encode only (z).
+// MODE 3: cold part of the tile-hybrid step -- the hot-column block of the encode product already sits
+// in z (tcgen05 GEMM, spmf_umma.cu); both sweeps visit only the entries the tensor cores do not cover
+// (stored after rowmid[row], positive values; the tcgen05 tile kernel, spmf_hot_tile.cu, owns the
+// others) and dzr / rowacc receive RAW partial sums (un-scaled sum w.EV, sum x log lambda,
+// #non-finite) that spmf_rows_finish completes.
+constexpr int kRowsTrain = 0, kRowsEncode = 1, kRowsCold = 3;
 
 template <int KP, int SV, int MODE>
 __device__ __forceinline__ void
@@ -162,8 +161,6 @@ csr_rows_body(const long long* __restrict__ rowptr, const int* __restrict__ cols
               const int* __restrict__ rowmid, int* __restrict__ gflag) {
   constexpr bool ENCODE_ONLY = (MODE == kRowsEncode);
   constexpr bool COLD = (MODE == kRowsCold);
-  constexpr bool ZIN = (MODE == kRowsHybrid) || COLD;     // z holds the GEMM's hot block on entry
-  constexpr bool HYBRID = (MODE == kRowsHybrid);          // sweep 2 sees signed (flagged) values
   using M = Map<KP, SV>;
   constexpr int VW = M::VW, LPN = M::LPN, RG = M::RG, VPL = M::VPL, REC = M::REC, NSLOT = M::NSLOT;
   constexpr int U = VPL >= 4 ? 2 : 4;
@@ -203,9 +200,8 @@ csr_rows_body(const long long* __restrict__ rowptr, const int* __restrict__ cols
   };
   const long long j0 = rowptr[row];
   const int n = (int)(rowptr[row + 1] - j0);
-  const int mid = ZIN ? rowmid[row] : 0;             // sweep 1 starts here in the hybrid modes
-  const Range R1 = make_range(j0 + mid, n - mid);
-  const Range R2 = HYBRID ? make_range(j0, n) : R1;
+  const int mid = COLD ? rowmid[row] : 0;            // both sweeps start here in the cold mode
+  const Range R = make_range(j0 + mid, n - mid);
   const float r = scale_rows ? rowsum[row] * inv_xi : 1.f;   // poisson.py:644-649
 
   // ---- z = r * sum_d x A'_d          (poisson.py:640-643 with 1/eta folded into A')
@@ -218,17 +214,17 @@ csr_rows_body(const long long* __restrict__ rowptr, const int* __restrict__ cols
   {
     int dcur[U];
     float xcur[U];
-    if (R1.my_groups > 0) ld_idx<U>(R1.gc + slot * U, R1.gv + slot * U, dcur, xcur);
-    for (int b = 0; b < R1.my_groups; ++b) {
+    if (R.my_groups > 0) ld_idx<U>(R.gc + slot * U, R.gv + slot * U, dcur, xcur);
+    for (int b = 0; b < R.my_groups; ++b) {
       float a[U][VPL][VW];
 #pragma unroll
       for (int u = 0; u < U; ++u)
 #pragma unroll
         for (int i = 0; i < VPL; ++i) ldv<VW>(a[u][i], Apl + (unsigned)dcur[u] * REC + off[i]);
-      const int gn = slot + min(b + 1, R1.my_groups - 1) * NSLOT;   // last iteration re-reads its own group
+      const int gn = slot + min(b + 1, R.my_groups - 1) * NSLOT;   // last iteration re-reads its own group
       int dn[U];
       float xn[U];
-      ld_idx<U>(R1.gc + gn * U, R1.gv + gn * U, dn, xn);
+      ld_idx<U>(R.gc + gn * U, R.gv + gn * U, dn, xn);
 #pragma unroll
       for (int u = 0; u < U; ++u) {
 #pragma unroll
@@ -239,10 +235,10 @@ csr_rows_body(const long long* __restrict__ rowptr, const int* __restrict__ cols
         xcur[u] = xn[u];
       }
     }
-    for (int e = 0; e < R1.n_extra; ++e) {
-      const int t = R1.extra_index(e);
-      const int d = __ldg(R1.rc + t);
-      const float x = __ldg(R1.rv + t);
+    for (int e = 0; e < R.n_extra; ++e) {
+      const int t = R.extra_index(e);
+      const int d = __ldg(R.rc + t);
+      const float x = __ldg(R.rv + t);
 #pragma unroll
       for (int i = 0; i < VPL; ++i) {
         float a[VW];
@@ -277,7 +273,7 @@ csr_rows_body(const long long* __restrict__ rowptr, const int* __restrict__ cols
   float* zq = z + ((size_t)q * nrows + row) * REC;
 #pragma unroll
   for (int i = 0; i < VPL; ++i) {
-    if constexpr (ZIN) {                    // hot-column block of x.A' from the tensor-core GEMM
+    if constexpr (COLD) {                   // hot-column block of x.A' from the tensor-core GEMM
       float a[VW];
       ldv_s<VW>(a, zq + off[i]);
 #pragma unroll
@@ -286,7 +282,7 @@ csr_rows_body(const long long* __restrict__ rowptr, const int* __restrict__ cols
 #pragma unroll
     for (int w = 0; w < VW; ++w) zz[i][w] *= r;
   }
-  if constexpr (ZIN) __syncthreads();       // every slot has read the GEMM block before slot 0 overwrites it
+  if constexpr (COLD) __syncthreads();      // every slot has read the GEMM block before slot 0 overwrites it
 #pragma unroll
   for (int i = 0; i < VPL; ++i)
     if (slot == 0) stv<VW>(zq + off[i], zz[i]);
@@ -305,12 +301,8 @@ csr_rows_body(const long long* __restrict__ rowptr, const int* __restrict__ cols
   {
     int dcur[U];
     float xcur[U];
-    if (R2.my_groups > 0) ld_idx<U>(R2.gc + slot * U, R2.gv + slot * U, dcur, xcur);
-    if constexpr (HYBRID) {
-#pragma unroll
-      for (int u = 0; u < U; ++u) xcur[u] = fabsf(xcur[u]);
-    }
-    for (int b = 0; b < R2.my_groups; ++b) {
+    if (R.my_groups > 0) ld_idx<U>(R.gc + slot * U, R.gv + slot * U, dcur, xcur);
+    for (int b = 0; b < R.my_groups; ++b) {
       float e[U][VPL][VW], ph[U], p[U];
 #pragma unroll
       for (int u = 0; u < U; ++u) {
@@ -318,14 +310,10 @@ csr_rows_body(const long long* __restrict__ rowptr, const int* __restrict__ cols
         for (int i = 0; i < VPL; ++i) ldv<VW>(e[u][i], EVl + (unsigned)dcur[u] * REC + off[i]);
         ph[u] = __ldg(PHl + (unsigned)dcur[u] * SV);
       }
-      const int gn = slot + min(b + 1, R2.my_groups - 1) * NSLOT;
+      const int gn = slot + min(b + 1, R.my_groups - 1) * NSLOT;
       int dn[U];
       float xn[U];
-      ld_idx<U>(R2.gc + gn * U, R2.gv + gn * U, dn, xn);
-      if constexpr (HYBRID) {
-#pragma unroll
-        for (int u = 0; u < U; ++u) xn[u] = fabsf(xn[u]);
-      }
+      ld_idx<U>(R.gc + gn * U, R.gv + gn * U, dn, xn);
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         p[u] = 0.f;
@@ -352,10 +340,10 @@ csr_rows_body(const long long* __restrict__ rowptr, const int* __restrict__ cols
         xcur[u] = xn[u];
       }
     }
-    for (int ex = 0; ex < R2.n_extra; ++ex) {
-      const int t = R2.extra_index(ex);
-      const int d = __ldg(R2.rc + t);
-      const float x = HYBRID ? fabsf(__ldg(R2.rv + t)) : __ldg(R2.rv + t);
+    for (int ex = 0; ex < R.n_extra; ++ex) {
+      const int t = R.extra_index(ex);
+      const int d = __ldg(R.rc + t);
+      const float x = __ldg(R.rv + t);
       float e[VPL][VW];
       float p = 0.f;
 #pragma unroll
@@ -475,12 +463,9 @@ __global__ void __launch_bounds__(128, 5) csr_rows_cold5_kernel(SPMF_ROWS_PARAMS
 // atomics when the column changes (only columns that straddle slices are contended).
 constexpr int kSliceLen = 256;
 
-// NO_GA: the hot-block variant of the hybrid step -- every entry of this CSC is covered by the
-// tensor-core GEMM for the GA' product (spmf_umma.cu), so only z is gathered (GEV, Gphi); with the
-// dzr record and its accumulators gone the kernel keeps four nonzeros in flight per slot instead of two.
 // `nnz_bound` sizes the grid; the actual count is colptr[D] (known on the device only).
-template <int KP, int SV, bool NO_GA>
-__global__ void __launch_bounds__(128, NO_GA ? 5 : 4)
+template <int KP, int SV>
+__global__ void __launch_bounds__(128, 4)
 csc_cols_kernel(const int* __restrict__ colptr, const int* __restrict__ rows,
                 const float* __restrict__ vals, int nnz_bound, int nrows, int D,
                 const float* __restrict__ z, const float* __restrict__ dzr,
@@ -488,7 +473,7 @@ csc_cols_kernel(const int* __restrict__ colptr, const int* __restrict__ rows,
                 float* __restrict__ GAp, float* __restrict__ GEV, float* __restrict__ Gphi, int slice_len) {
   using M = Map<KP, SV>;
   constexpr int VW = M::VW, LPN = M::LPN, RG = M::RG, VPL = M::VPL, REC = M::REC, NSLOT = M::NSLOT;
-  constexpr int U = (VPL >= 4 && !NO_GA) ? 2 : 4;
+  constexpr int U = VPL >= 4 ? 2 : 4;
   const int lane = threadIdx.x & 31;
   const int slot = threadIdx.x / LPN;
   const int li = threadIdx.x % LPN;
@@ -521,7 +506,7 @@ csc_cols_kernel(const int* __restrict__ colptr, const int* __restrict__ rows,
   int d = lo;
   int next = __ldg(colptr + d + 1);
 
-  float ev[VPL][VW], aEV[VPL][VW], aAp[NO_GA ? 1 : VPL][VW], ph, aPh;
+  float ev[VPL][VW], aEV[VPL][VW], aAp[VPL][VW], ph, aPh;
   auto load_col = [&](int dd) {
 #pragma unroll
     for (int i = 0; i < VPL; ++i) {
@@ -529,7 +514,7 @@ csc_cols_kernel(const int* __restrict__ colptr, const int* __restrict__ rows,
 #pragma unroll
       for (int w = 0; w < VW; ++w) {
         aEV[i][w] = 0.f;
-        if constexpr (!NO_GA) aAp[i][w] = 0.f;
+        aAp[i][w] = 0.f;
       }
     }
     ph = __ldg(PHl + (unsigned)dd * SV);
@@ -542,12 +527,12 @@ csc_cols_kernel(const int* __restrict__ colptr, const int* __restrict__ rows,
 #pragma unroll
       for (int w = 0; w < VW; ++w) {
         atomicAdd(GEVq + o + w, aEV[i][w]);
-        if constexpr (!NO_GA) atomicAdd(GApq + o + w, aAp[i][w]);
+        atomicAdd(GApq + o + w, aAp[i][w]);
       }
     }
     if (kg == 0) atomicAdd(Gphq + (unsigned)dd * SV, aPh);
   };
-  auto one = [&](int j, float x, const float (&zz)[VPL][VW], const float (&dd)[NO_GA ? 1 : VPL][VW]) {
+  auto one = [&](int j, float x, const float (&zz)[VPL][VW], const float (&dd)[VPL][VW]) {
     if (j >= next) {
       flush_col(d);
       do {
@@ -569,7 +554,7 @@ csc_cols_kernel(const int* __restrict__ colptr, const int* __restrict__ rows,
 #pragma unroll
       for (int w = 0; w < VW; ++w) {
         aEV[i][w] = fmaf(gq, zz[i][w], aEV[i][w]);
-        if constexpr (!NO_GA) aAp[i][w] = fmaf(x, dd[i][w], aAp[i][w]);
+        aAp[i][w] = fmaf(x, dd[i][w], aAp[i][w]);
       }
   };
   load_col(d);
@@ -589,13 +574,13 @@ csc_cols_kernel(const int* __restrict__ colptr, const int* __restrict__ rows,
       bb[0] = b2.x; bb[1] = b2.y;
       xx[0] = x2.x; xx[1] = x2.y;
     }
-    float zz[U][VPL][VW], dd[U][NO_GA ? 1 : VPL][VW];
+    float zz[U][VPL][VW], dd[U][VPL][VW];
 #pragma unroll
     for (int u = 0; u < U; ++u)
 #pragma unroll
       for (int i = 0; i < VPL; ++i) {
         ldv<VW>(zz[u][i], zl + (unsigned)bb[u] * REC + off[i]);
-        if constexpr (!NO_GA) ldv<VW>(dd[u][i], dl + (unsigned)bb[u] * REC + off[i]);
+        ldv<VW>(dd[u][i], dl + (unsigned)bb[u] * REC + off[i]);
       }
 #pragma unroll
     for (int u = 0; u < U; ++u) one(jb + u, xx[u], zz[u], dd[u]);
@@ -603,11 +588,11 @@ csc_cols_kernel(const int* __restrict__ colptr, const int* __restrict__ rows,
   for (int j = j0 + nfull * U; j < j1; ++j) {     // tail of the last slice
     const int b = __ldg(rows + j);
     const float x = __ldg(vals + j);
-    float zz[VPL][VW], dd[NO_GA ? 1 : VPL][VW];
+    float zz[VPL][VW], dd[VPL][VW];
 #pragma unroll
     for (int i = 0; i < VPL; ++i) {
       ldv<VW>(zz[i], zl + (unsigned)b * REC + off[i]);
-      if constexpr (!NO_GA) ldv<VW>(dd[i], dl + (unsigned)b * REC + off[i]);
+      ldv<VW>(dd[i], dl + (unsigned)b * REC + off[i]);
     }
     one(j, x, zz, dd);
   }
@@ -939,41 +924,6 @@ __global__ void dense_fill_kernel(const float* __restrict__ x, int nrows, int D,
 
 __device__ __forceinline__ bool hot_covered(int r, float x, int H) {   // rank in the block, x > 0 exact in bf16
   return r < H && x > 0.f && __uint_as_float(__float_as_uint(x) & 0xffff0000u) == x;
-}
-
-// xthot = UMMA-tiled X^T[H][Bp] from xhot = UMMA-tiled X[nrows][Hp]: one CTA per 128 x 64 tile of xhot,
-// transposed through shared memory; the result is two contiguous 8 KiB half-tiles of xthot.  Covers
-// every element of xthot (padding included), so no memset is needed.
-__global__ void __launch_bounds__(256)
-hot_transpose_kernel(const unsigned short* __restrict__ xhot, int hchunks, unsigned short* __restrict__ xthot,
-                     int bchunks, int xt_mtiles) {
-  __shared__ unsigned short t[128][66];                      // [row b][col h], padded
-  const int kcx = blockIdx.x, mtx = blockIdx.y;             // xhot tile: rows 128*mtx.., cols 64*kcx..
-  const unsigned short* src = xhot + ((size_t)mtx * hchunks + kcx) * (kTileABytes / 2);
-  // read the tile in its storage order (16-byte chunks), scatter into t[b][h]
-  for (int ch = threadIdx.x; ch < 1024; ch += blockDim.x) {
-    // (an odd number of column chunks: the grid is rounded up so the last m-tile of xthot is complete)
-    const uint4 v = kcx < hchunks ? *reinterpret_cast<const uint4*>(src + ch * 8) : make_uint4(0u, 0u, 0u, 0u);
-    const int rg = ch >> 6, kc8 = (ch >> 3) & 7, r = rg * 8 + (ch & 7);
-    const unsigned short* e = reinterpret_cast<const unsigned short*>(&v);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) t[r][kc8 * 8 + i] = e[i];
-  }
-  __syncthreads();
-  // xthot rows h = 64*kcx + (0..63) -> m-tile (64*kcx)/128, row offset (kcx & 1) * 64; k = b in chunks 2*mtx, 2*mtx+1
-  const int mt_t = kcx >> 1, rbase = (kcx & 1) * 64;
-  if (mt_t >= xt_mtiles) return;
-  for (int ch = threadIdx.x; ch < 1024; ch += blockDim.x) {   // 64 rows x 16 chunks of 8 k
-    const int hr = ch >> 4, kq = ch & 15;                     // local row h, 8-wide k group (b = 8*kq ..)
-    const int kc_t = 2 * mtx + (kq >> 3);
-    if (kc_t >= bchunks) continue;
-    unsigned short e[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) e[i] = t[kq * 8 + i][hr];
-    unsigned short* dst = xthot + ((size_t)mt_t * bchunks + kc_t) * (kTileABytes / 2) +
-                          (core_off(rbase + hr, kq & 7) >> 1);
-    *reinterpret_cast<uint4*>(dst) = *reinterpret_cast<const uint4*>(e);
-  }
 }
 
 // One CTA per row of the 128-row-padded batch.  STAGED: the row's dense hot vector (Hp bf16) is assembled
@@ -1421,7 +1371,7 @@ static int launch_rows(const long long* rowptr, const int* cols, const float* va
   return SPMF_OK;
 }
 
-template <int KP, int SV, bool NO_GA>
+template <int KP, int SV>
 static int launch_cols(const int* colptr, const int* rows, const float* vals, int nnz, int nrows,
                        int D, int NQ, const float* z, const float* dzr, const float* EV,
                        const float* PH, float* GAp, float* GEV, float* Gphi, cudaStream_t st,
@@ -1430,8 +1380,8 @@ static int launch_cols(const int* colptr, const int* rows, const float* vals, in
   const int nslices = (nnz + slice_len - 1) / slice_len;
   if (nslices == 0) return SPMF_OK;
   dim3 grid((nslices + NSLOT - 1) / NSLOT, NQ);
-  csc_cols_kernel<KP, SV, NO_GA><<<grid, 128, 0, st>>>(colptr, rows, vals, nnz, nrows, D, z, dzr, EV, PH,
-                                                      GAp, GEV, Gphi, slice_len);
+  csc_cols_kernel<KP, SV><<<grid, 128, 0, st>>>(colptr, rows, vals, nnz, nrows, D, z, dzr, EV, PH,
+                                               GAp, GEV, Gphi, slice_len);
   SPMF_CHECK_LAUNCH();
   return SPMF_OK;
 }
@@ -1514,7 +1464,7 @@ int spmf_csc_cols(const int* colptr, const int* rows, const float* vals, int nnz
   if (e == cudaSuccess) e = cudaMemsetAsync(Gphinz, 0, (size_t)NQ * D * SV * sizeof(float), st);
   if (e != cudaSuccess) return (int)e;
   int rc = SPMF_OK;
-#define CALL_COLS(KPC, SVC) rc = launch_cols<KPC, SVC, false>(colptr, rows, vals, nnz, nrows, D, NQ, z, dzr, EV, PH, GAp, GEVnz, Gphinz, st)
+#define CALL_COLS(KPC, SVC) rc = launch_cols<KPC, SVC>(colptr, rows, vals, nnz, nrows, D, NQ, z, dzr, EV, PH, GAp, GEVnz, Gphinz, st)
   SPMF_DISPATCH_KP_SV(KP, SV, CALL_COLS);
 #undef CALL_COLS
   return rc;
@@ -1539,8 +1489,7 @@ int spmf_csc_cols(const int* colptr, const int* rows, const float* vals, int nnz
     else return SPMF_ERR_UNSUPPORTED;                                        \
   } while (0)
 
-/* 0: gather kernels only; 2: tile-hybrid (KP <= 32: GEMMs + fused tile kernel); 1: GEMM-hybrid only
- * (KP = 64, 128: the count products on tcgen05 in blocks of 128 channels, per-nonzero terms gathered) */
+/* 0: gather kernels only; 2: tile-hybrid (GEMMs + fused tile kernel, spmf_hot_tile.cu) */
 int spmf_hybrid_supported(int K, int S) {
   if (K <= 0 || K > SPMF_MAX_K || S <= 0) return 0;
   const int KP = spmf_kpad(K), SV = spmf_draw_vec(S);
@@ -1548,22 +1497,6 @@ int spmf_hybrid_supported(int K, int S) {
     return 2;
   if (KP == 64 || KP == 128) return 2;     // fused tile kernel with 64 / 128 latent dims (spmf_hot_tile.cu)
   return 0;
-}
-
-int spmf_csr_rows_hybrid(const long long* rowptr, const int* cols, const float* vals, const int* rowmid,
-                         const float* rowsum, const float* lgam, float inv_xi, int scale_rows, int nrows,
-                         int D, int K, int S, const float* Ap, const float* EV, const float* PH,
-                         const double* vsum, float* z, float* dzr, float* rowacc, void* gs, void* stream) {
-  if (!rowptr || !cols || !vals || !rowmid || !rowsum || !lgam || !Ap || !EV || !PH || !vsum || !z || !dzr || !rowacc)
-    return SPMF_ERR_BAD_ARG;
-  if (nrows <= 0 || D <= 0 || K <= 0 || K > SPMF_MAX_K || S <= 0) return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
-  cudaStream_t st = (cudaStream_t)stream;
-  int rc = SPMF_OK;
-#define CALL_ROWS_H(KPC, SVC) rc = launch_rows<KPC, SVC, kRowsHybrid>(rowptr, cols, vals, rowsum, lgam, inv_xi, scale_rows, nrows, D, NQ, Ap, EV, PH, vsum, z, dzr, rowacc, rowmid, (int*)gs, st)
-  SPMF_DISPATCH_HYBRID(KP, SV, CALL_ROWS_H);
-#undef CALL_ROWS_H
-  return rc;
 }
 
 int spmf_csr_rows_cold(const long long* rowptr, const int* cols, const float* vals, const int* rowmid,
@@ -1595,35 +1528,16 @@ int spmf_zero_col_grads(float* GAp, float* GEVnz, float* Gphinz, int D, int K, i
 
 int spmf_csc_cols_accum(const int* colptr, const int* rows, const float* vals, int nnz_bound, int nrows, int D,
                         int K, int S, const float* z, const float* dzr, const float* EV, const float* PH,
-                        float* GAp, float* GEVnz, float* Gphinz, int covered, void* stream) {
+                        float* GAp, float* GEVnz, float* Gphinz, void* stream) {
   if (!colptr || !rows || !vals || !z || !dzr || !EV || !PH || !GAp || !GEVnz || !Gphinz) return SPMF_ERR_BAD_ARG;
   if (nnz_bound < 0 || nrows <= 0 || D <= 0 || K <= 0 || K > SPMF_MAX_K || S <= 0) return SPMF_ERR_BAD_ARG;
   const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
   cudaStream_t st = (cudaStream_t)stream;
   int rc = SPMF_OK;
-  if (covered) {     // GEV and Gphi only: GA' of these entries comes from the tensor-core GEMM
-#define CALL_COLS_HOT(KPC, SVC) rc = launch_cols<KPC, SVC, true>(colptr, rows, vals, nnz_bound, nrows, D, NQ, z, dzr, EV, PH, GAp, GEVnz, Gphinz, st)
-    SPMF_DISPATCH_HYBRID(KP, SV, CALL_COLS_HOT);
-#undef CALL_COLS_HOT
-  } else {           // sparse remainder: short slices keep every SM busy on a small stream
-#define CALL_COLS_COLD(KPC, SVC) rc = launch_cols<KPC, SVC, false>(colptr, rows, vals, nnz_bound, nrows, D, NQ, z, dzr, EV, PH, GAp, GEVnz, Gphinz, st, 64)
-    SPMF_DISPATCH_HYBRID(KP, SV, CALL_COLS_COLD);
+  // sparse remainder: short slices keep every SM busy on a small stream
+#define CALL_COLS_COLD(KPC, SVC) rc = launch_cols<KPC, SVC>(colptr, rows, vals, nnz_bound, nrows, D, NQ, z, dzr, EV, PH, GAp, GEVnz, Gphinz, st, 64)
+  SPMF_DISPATCH_HYBRID(KP, SV, CALL_COLS_COLD);
 #undef CALL_COLS_COLD
-  }
-  return rc;
-}
-
-int spmf_csc_cols_hybrid(const int* hot_colptr, const int* hot_rows, const float* hot_vals,
-                         const int* cold_colptr, const int* cold_rows, const float* cold_vals, int nnz_bound,
-                         int nrows, int D, int K, int S, const float* z, const float* dzr, const float* EV,
-                         const float* PH, float* GAp, float* GEVnz, float* Gphinz, void* stream) {
-  int rc = spmf_zero_col_grads(GAp, GEVnz, Gphinz, D, K, S, stream);
-  if (rc == SPMF_OK)
-    rc = spmf_csc_cols_accum(hot_colptr, hot_rows, hot_vals, nnz_bound, nrows, D, K, S, z, dzr, EV, PH, GAp, GEVnz,
-                             Gphinz, 1, stream);
-  if (rc == SPMF_OK)
-    rc = spmf_csc_cols_accum(cold_colptr, cold_rows, cold_vals, nnz_bound, nrows, D, K, S, z, dzr, EV, PH, GAp,
-                             GEVnz, Gphinz, 0, stream);
   return rc;
 }
 
@@ -1631,8 +1545,17 @@ int spmf_csc_cols_hybrid(const int* hot_colptr, const int* hot_rows, const float
 // A nonzero is "covered" by the tensor-core products when its column's rank is < H and its value
 // is exactly representable in bf16 (integer counts <= 256).  Per row, covered entries come first
 // (stored with a negative sign as their flag), the rest after rowmid[row]; column ids become ranks.
-// xhot[b][rank] / xthot[rank][b] receive the covered values (both pre-zeroed here).
+// xhot[b][rank] receives the covered values.
 }  // extern "C"
+
+// test hook: exercise the wide-block fallback (unstaged split kernels) on small inputs
+static bool split_unstaged() {
+  static const bool on = [] {
+    const char* e = getenv("SPMF_SPLIT_UNSTAGED");
+    return e && e[0] == '1';
+  }();
+  return on;
+}
 
 template <typename CT, typename VT>
 static int launch_hot_split(const long long* rowptr, const CT* cols, const VT* vals, int nrows, const int* rank, int H,
@@ -1641,11 +1564,7 @@ static int launch_hot_split(const long long* rowptr, const CT* cols, const VT* v
   const long long hp = (H + 63) / 64 * 64;
   const size_t stash = (size_t)kSplitStash * sizeof(int2);
   const size_t smem = (size_t)hp * 2 + stash;
-  static const bool force_scatter = [] {           // test hook: exercise the wide-block fallback on small inputs
-    const char* e = getenv("SPMF_SPLIT_UNSTAGED");
-    return e && e[0] == '1';
-  }();
-  if (smem <= 112 * 1024 && !force_scatter) {
+  if (smem <= 112 * 1024 && !split_unstaged()) {
     // staged: every 16-byte chunk of the 128-row-padded block is written by the kernel (no memset)
     static bool attr = false;
     if (!attr) {
@@ -1675,28 +1594,16 @@ static int launch_hot_split8(const long long* rowptr, const unsigned char* gaps8
   const long long hp = (H + 63) / 64 * 64;
   const size_t stash = (size_t)kSplitStash * sizeof(int2);
   const size_t smem = (size_t)hp * 2 + stash;
-  if (smem <= 112 * 1024) {
+  if (smem <= 112 * 1024 && !split_unstaged()) {
     static bool attr = false;
     if (!attr) {
-      cudaError_t e = cudaFuncSetAttribute(hot_split_kernel<true, unsigned char, unsigned char, true>,
-                                           cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024);
-      if (e != cudaSuccess) return (int)e;
-      e = cudaFuncSetAttribute(hot_split8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024);
+      cudaError_t e = cudaFuncSetAttribute(hot_split8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024);
       if (e != cudaSuccess) return (int)e;
       attr = true;
     }
-    static const bool two_pass = [] {               // ablation switch: the generic two-sweep kernel
-      const char* e = getenv("SPMF_SPLIT8_TWO_PASS");
-      return e && e[0] == '1';
-    }();
-    if (two_pass)
-      hot_split_kernel<true, unsigned char, unsigned char, true><<<(nrows + 127) / 128 * 128, kSplitThreads, smem, st>>>(
-          rowptr, gaps8, vals8, nrows, rank, H, rowptr_out, cols_out, vals_out, rowmid, (unsigned short*)xhot, hp / 64,
-          rowsum, lgam, ovf_idx, ovf_val, novf);
-    else
-      hot_split8_kernel<<<(nrows + 127) / 128 * 128, kSplitThreads, (size_t)hp * 2, st>>>(
-          rowptr, gaps8, vals8, nrows, rank, H, rowptr_out, cols_out, vals_out, rowmid, (unsigned short*)xhot, hp / 64,
-          rowsum, lgam, ovf_idx, ovf_val, novf);
+    hot_split8_kernel<<<(nrows + 127) / 128 * 128, kSplitThreads, (size_t)hp * 2, st>>>(
+        rowptr, gaps8, vals8, nrows, rank, H, rowptr_out, cols_out, vals_out, rowmid, (unsigned short*)xhot, hp / 64,
+        rowsum, lgam, ovf_idx, ovf_val, novf);
   } else {
     cudaError_t e = cudaMemsetAsync(xhot, 0, (size_t)spmf_umma_tiled_a_elems(nrows, hp) * 2, st);
     if (e != cudaSuccess) return (int)e;
@@ -1723,14 +1630,13 @@ int spmf_hot_split_u8(const long long* rowptr, const unsigned char* gaps8, const
 
 int spmf_hot_split_packed(const long long* rowptr, const int* cols, const unsigned short* cols16, const float* vals,
                           const unsigned short* vals16, int nrows, long long nnz, const int* rank, int H,
-                          long long* rowptr_out, int* cols_out, float* vals_out, int* rowmid, void* xhot, void* xthot,
+                          long long* rowptr_out, int* cols_out, float* vals_out, int* rowmid, void* xhot,
                           float* rowsum, float* lgam, void* stream) {
   if (!rowptr || (!cols == !cols16) || (!vals == !vals16) || !rowptr_out || !cols_out || !vals_out || !rowmid || !xhot)
     return SPMF_ERR_BAD_ARG;
   if ((rowsum == nullptr) != (lgam == nullptr)) return SPMF_ERR_BAD_ARG;
   if (nrows <= 0 || nnz < 0 || H <= 0) return SPMF_ERR_BAD_ARG;
   cudaStream_t st = (cudaStream_t)stream;
-  const long long hp = (H + 63) / 64 * 64, bp = ((long long)nrows + 63) / 64 * 64;
   int rc;
 #define SPMF_SPLIT_ARGS nrows, rank, H, rowptr_out, cols_out, vals_out, rowmid, xhot, rowsum, lgam, st
   if (cols && vals) rc = launch_hot_split(rowptr, cols, vals, SPMF_SPLIT_ARGS);
@@ -1738,22 +1644,15 @@ int spmf_hot_split_packed(const long long* rowptr, const int* cols, const unsign
   else if (vals) rc = launch_hot_split(rowptr, cols16, vals, SPMF_SPLIT_ARGS);
   else rc = launch_hot_split(rowptr, cols16, vals16, SPMF_SPLIT_ARGS);
 #undef SPMF_SPLIT_ARGS
-  if (rc != SPMF_OK) return rc;
-  if (!xthot) return SPMF_OK;      // (the GA' GEMM reads xhot itself as an MN-major operand)
-  // the transpose covers whole 128-row tiles of xhot: rows >= nrows are zero there (written by the split)
-  dim3 tg((unsigned)((hp / 64 + 1) / 2 * 2), (unsigned)((nrows + 127) / 128));
-  hot_transpose_kernel<<<tg, 256, 0, st>>>((const unsigned short*)xhot, (int)(hp / 64), (unsigned short*)xthot,
-                                           (int)(bp / 64), (int)((H + 127) / 128));
-  SPMF_CHECK_LAUNCH();
-  return SPMF_OK;
+  return rc;
 }
 
 int spmf_hot_split(const long long* rowptr, const int* cols, const float* vals, int nrows, long long nnz,
                    const int* rank, int H, long long* rowptr_out, int* cols_out, float* vals_out, int* rowmid,
-                   void* xhot, void* xthot, float* rowsum, float* lgam, void* stream) {
+                   void* xhot, float* rowsum, float* lgam, void* stream) {
   if (!cols || !vals) return SPMF_ERR_BAD_ARG;
   return spmf_hot_split_packed(rowptr, cols, nullptr, vals, nullptr, nrows, nnz, rank, H, rowptr_out, cols_out,
-                               vals_out, rowmid, xhot, xthot, rowsum, lgam, stream);
+                               vals_out, rowmid, xhot, rowsum, lgam, stream);
 }
 
 int spmf_csr_colstats(const int* cols, const float* vals, long long nnz, int D, double* colsum,

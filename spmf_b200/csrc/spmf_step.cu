@@ -46,8 +46,7 @@ int spmf_advi_step(const spmf_step_args* a) {
     STEP_TRY(spmf_gamma_grad(a->params, a->noise, D, K, S, a->dgda, side));
   // ---- hot path
   const bool hybrid = a->hot_cols > 0;
-  if (hybrid && (!a->rank || !a->rowmid || !a->xhot || !a->ApT3 || !a->dzrT3)) return SPMF_ERR_BAD_ARG;
-  if (hybrid && a->hot_mode != 2 && (!a->hot_colptr || !a->hot_crows || !a->hot_cvals)) return SPMF_ERR_BAD_ARG;
+  if (hybrid && (!a->rank || !a->rowmid || !a->xhot || !a->ApT3 || !a->dzrT3 || !a->EVt)) return SPMF_ERR_BAD_ARG;
   if (a->fresh_noise)
     STEP_TRY(spmf_fill_noise_dev(a->noise, a->params, D, K, S, a->seed, a->rng_step, SPMF_NOISE_NORMAL, a->step_state,
                                  hot));
@@ -74,9 +73,9 @@ int spmf_advi_step(const spmf_step_args* a) {
                                   a->adam_t, a->clip_value, 1.0f, a->step_state, side));
   }
   if (side != hot) CUDA_TRY(cudaEventRecord((cudaEvent_t)a->ev_join, side));
-  // (tile mode with auxiliary streams: the fp64 operand sums are first read by spmf_rows_finish, so
+  // (hybrid step with auxiliary streams: the fp64 operand sums are first read by spmf_rows_finish, so
   // they leave the critical path and run next to the encode GEMM)
-  const bool pre_fork = hybrid && a->hot_mode == 2 && a->EVt && a->aux_stream1 && a->ev_aux_fork && a->ev_aux_join1;
+  const bool pre_fork = hybrid && a->aux_stream1 && a->ev_aux_fork && a->ev_aux_join1;
   STEP_TRY(spmf_draw_operands_ranked_m(a->params, a->noise, a->eta, hybrid ? a->rank : nullptr, D, K, S, a->Ap,
                                        a->EV, a->PH, pre_fork ? nullptr : a->vsum, pre_fork ? nullptr : a->phisum,
                                        a->scr_d, a->model, hot));
@@ -130,27 +129,20 @@ int spmf_advi_step(const spmf_step_args* a) {
     STEP_TRY(spmf_umma_gemm3(a->xhot, 0, a->nrows, a->ApT3, a->t3_qstride, a->z, REC, (long long)a->nrows * REC,
                              REC, Hp, NQ, a->gemm_splits, hot));
     if (pre_fork) CUDA_TRY(cudaStreamWaitEvent(hot, (cudaEvent_t)a->ev_aux_join1, 0));
-    if (a->hot_mode == 2) {
-      // per-nonzero terms of the hot block in the fused tcgen05 tile kernel; the gather kernel keeps
-      // the uncovered entries only
-      if (!a->EVt) return SPMF_ERR_BAD_ARG;
-      if (!pre_fork) {
-        STEP_TRY(spmf_hot_ev_tiles(a->EV, a->PH, D, H, K, S, a->EVt, hot));
-        STEP_TRY(spmf_zero_col_grads(a->GAp, a->GEV, a->Gph, D, K, S, hot));
-      }
-      STEP_TRY(spmf_csr_rows_cold(a->rowptr, a->cols, a->vals, a->rowmid, a->rowsum, a->inv_xi, a->scale_rows,
-                                  a->nrows, D, K, S, a->Ap, a->EV, a->PH, a->z, a->dzr, a->rowacc, a->gs, hot));
-      if (a->ev_tile0) CUDA_TRY(cudaEventRecord((cudaEvent_t)a->ev_tile0, hot));
-      STEP_TRY(spmf_hot_tile(a->xhot, a->EVt, a->z, a->nrows, D, H, K, S, a->dzr, a->rowacc, a->GEV, a->Gph, a->gs,
-                             hot));
-      if (a->ev_tile1) CUDA_TRY(cudaEventRecord((cudaEvent_t)a->ev_tile1, hot));
-      STEP_TRY(spmf_rows_finish(a->rowsum, a->lgam, a->inv_xi, a->scale_rows, a->nrows, K, S, a->vsum, a->z, a->dzr,
-                                a->rowacc, a->gs, hot));
-    } else {
-      STEP_TRY(spmf_csr_rows_hybrid(a->rowptr, a->cols, a->vals, a->rowmid, a->rowsum, a->lgam, a->inv_xi,
-                                    a->scale_rows, a->nrows, D, K, S, a->Ap, a->EV, a->PH, a->vsum, a->z, a->dzr,
-                                    a->rowacc, a->gs, hot));
+    // per-nonzero terms of the hot block in the fused tcgen05 tile kernel; the gather kernel keeps
+    // the uncovered entries only
+    if (!pre_fork) {
+      STEP_TRY(spmf_hot_ev_tiles(a->EV, a->PH, D, H, K, S, a->EVt, hot));
+      STEP_TRY(spmf_zero_col_grads(a->GAp, a->GEV, a->Gph, D, K, S, hot));
     }
+    STEP_TRY(spmf_csr_rows_cold(a->rowptr, a->cols, a->vals, a->rowmid, a->rowsum, a->inv_xi, a->scale_rows,
+                                a->nrows, D, K, S, a->Ap, a->EV, a->PH, a->z, a->dzr, a->rowacc, a->gs, hot));
+    if (a->ev_tile0) CUDA_TRY(cudaEventRecord((cudaEvent_t)a->ev_tile0, hot));
+    STEP_TRY(spmf_hot_tile(a->xhot, a->EVt, a->z, a->nrows, D, H, K, S, a->dzr, a->rowacc, a->GEV, a->Gph, a->gs,
+                           hot));
+    if (a->ev_tile1) CUDA_TRY(cudaEventRecord((cudaEvent_t)a->ev_tile1, hot));
+    STEP_TRY(spmf_rows_finish(a->rowsum, a->lgam, a->inv_xi, a->scale_rows, a->nrows, K, S, a->vsum, a->z, a->dzr,
+                              a->rowacc, a->gs, hot));
   }
   // exact guard of poisson.py:606-616: if a row pass met a non-finite log-likelihood, the data term of
   // this step is re-evaluated densely with the reference's replacement semantics (conditional launch:
@@ -173,16 +165,15 @@ int spmf_advi_step(const spmf_step_args* a) {
     STEP_TRY(spmf_csc_cols(a->colptr, a->crows, a->cvals, a->nnz, a->nrows, D, K, S, a->z, a->dzr, a->EV, a->PH,
                            a->GAp, a->GEV, a->Gph, 0, hot));
   } else {
-    // three independent accumulations into the (zeroed) column-gradient tables:
-    //   hot CSC (covered entries): GEV, Gphi          -- gather kernel, hot stream
+    // two independent accumulations into the column-gradient tables (zeroed before the tile kernel,
+    // which has added GEV / Gphi of the covered entries):
     //   GA'[0:H] += X_hot^T . dzr                     -- tcgen05 GEMM, aux stream 1
-    //   cold CSC (everything else): GEV, Gphi, GA'    -- gather kernel, aux stream 2
+    //   cold CSC (the uncovered entries): GEV, Gphi, GA'  -- gather kernel, aux stream 2
     const int H = a->hot_cols;
     const int Bp = (a->nrows + 127) / 128 * 128;     // whole 128-row tiles of the count block
     const bool fork = cols_fork;
     cudaStream_t s1 = fork ? (cudaStream_t)a->aux_stream1 : hot;
     cudaStream_t s2 = fork ? (cudaStream_t)a->aux_stream2 : hot;
-    if (a->hot_mode != 2) STEP_TRY(spmf_zero_col_grads(a->GAp, a->GEV, a->Gph, D, K, S, hot));
     if (fork) {
       CUDA_TRY(cudaEventRecord((cudaEvent_t)a->ev_aux_fork, hot));
       CUDA_TRY(cudaStreamWaitEvent(s1, (cudaEvent_t)a->ev_aux_fork, 0));
@@ -197,10 +188,7 @@ int spmf_advi_step(const spmf_step_args* a) {
                                 (long long)D * REC, REC, NQ, a->gemm_splits, s1));
     if (a->ev_gemm1) CUDA_TRY(cudaEventRecord((cudaEvent_t)a->ev_gemm1, s1));
     STEP_TRY(spmf_csc_cols_accum(a->colptr, a->crows, a->cvals, a->nnz, a->nrows, D, K, S, a->z, a->dzr, a->EV,
-                                 a->PH, a->GAp, a->GEV, a->Gph, 0, s2));
-    if (a->hot_mode != 2)      // (mode 2: GEV / Gphi of the covered entries came from the tile kernel)
-      STEP_TRY(spmf_csc_cols_accum(a->hot_colptr, a->hot_crows, a->hot_cvals, a->nnz, a->nrows, D, K, S, a->z,
-                                   a->dzr, a->EV, a->PH, a->GAp, a->GEV, a->Gph, 1, hot));
+                                 a->PH, a->GAp, a->GEV, a->Gph, s2));
     if (fork) {
       CUDA_TRY(cudaEventRecord((cudaEvent_t)a->ev_aux_join1, s1));
       CUDA_TRY(cudaEventRecord((cudaEvent_t)a->ev_aux_join2, s2));

@@ -52,22 +52,17 @@ class StepGraphs:
 
 @dataclass
 class HotSplit:
-    """Hybrid form of a minibatch (spmf_hot_split): ranked + partitioned CSR, its CSC copy, and the
-    dense bf16 hot-column block with its transpose -- the operands of the tcgen05 GEMMs."""
+    """Hybrid form of a minibatch (spmf_hot_split): ranked + partitioned CSR, the CSC copy of its uncovered
+    entries, and the dense bf16 hot-column block -- the operand of the tcgen05 kernels."""
     H: int
     rowptr: torch.Tensor          # int64 [nrows+1], zero-based
     cols: torch.Tensor            # int32 [nnz]   column RANKS
     vals: torch.Tensor            # fp32 [nnz]    negative = covered by the tensor-core products
     rowmid: torch.Tensor          # int32 [nrows] first uncovered entry of each row (row-local)
     xhot: torch.Tensor            # bf16, UMMA-tiled X[nrows][ceil64(H)]   (see include/spmf_b200.h)
-    xthot: Optional[torch.Tensor] # bf16, UMMA-tiled X^T[H][ceil64(nrows)] (only on request; the step reads xhot)
     colptr: torch.Tensor          # CSC of the entries NOT covered by the GEMMs: int32 [D+1]
     crows: torch.Tensor
     cvals: torch.Tensor
-    hcolptr: torch.Tensor         # CSC of the covered entries (valid only if has_hot_csc)
-    hcrows: torch.Tensor
-    hcvals: torch.Tensor
-    has_hot_csc: bool = True
     version: int = 0              # column-ordering version this form was built for
 
 
@@ -89,42 +84,32 @@ class DeviceBatch:
     dense_raw: Optional[torch.Tensor] = None   # dense-ingested batch: the raw [nrows][D] upload (feature order)
     dense_dtype: int = 0                       # SPMF_DENSE_* of dense_raw
 
-    def ensure_hot(self, rank, H, bufs=None, hot_csc=True, row_consts=False, build_xt=False, packed=None,
-                   version=0):
+    def ensure_hot(self, rank, H, bufs=None, row_consts=False, packed=None, version=0):
         """Build (once) the hybrid form for the column ordering `rank` (int32 [D] device tensor) with
-        H hot columns.  `bufs` may supply reusable staging (the streaming uploader).  `hot_csc`: also
-        build the CSC copy of the covered entries (only the GEMM-only hybrid mode reads it; the tile
-        mode gets those gradients from the tensor-core kernel).  `packed` = (cols16, vals16): read the
-        compact upload format instead of self.cols / self.vals (either may be None = use the wide array)."""
-        if (self.hot is not None and self.hot.H == H and self.hot.version == version
-                and (self.hot.has_hot_csc or not hot_csc)):
+        H hot columns.  `bufs` may supply reusable staging (the streaming uploader).  `packed` =
+        (cols16, vals16): read the compact upload format instead of self.cols / self.vals (either may be
+        None = use the wide array)."""
+        if self.hot is not None and self.hot.H == H and self.hot.version == version:
             return self.hot
         dev = self.rowptr.device
         n, nnz = self.nrows, self.nnz
         m = max(nnz, 1) + 8
         na = _abi._lib.spmf_umma_tiled_a_elems(n, _ceil64(H))
-        nt = _abi._lib.spmf_umma_tiled_a_elems(H, _ceil64(n))
         if bufs is None:
             bufs = dict(rowptr=torch.empty(n + 1, dtype=torch.int64, device=dev),
                         cols=torch.empty(m, dtype=torch.int32, device=dev),
                         vals=torch.empty(m, dtype=torch.float32, device=dev),
                         rowmid=torch.empty(n, dtype=torch.int32, device=dev),
                         xhot=torch.empty(na, dtype=torch.bfloat16, device=dev),
-                        xthot=torch.empty(nt, dtype=torch.bfloat16, device=dev) if build_xt else None,
                         colptr=torch.empty(self.D + 1, dtype=torch.int32, device=dev),
                         crows=torch.empty(m, dtype=torch.int32, device=dev),
                         cvals=torch.empty(m, dtype=torch.float32, device=dev),
-                        hcolptr=torch.empty(self.D + 1, dtype=torch.int32, device=dev),
-                        hcrows=torch.empty(m, dtype=torch.int32, device=dev),
-                        hcvals=torch.empty(m, dtype=torch.float32, device=dev),
                         scratch=torch.empty(_abi._lib.spmf_csc_scratch_ints(self.D), dtype=torch.int32, device=dev))
         st = _stream()
         rs, lg = (_ptr(self.rowsum), _ptr(self.lgam)) if row_consts else (None, None)
         if packed is not None and len(packed) == 5:
             # 2-byte transfer format: (gaps8, vals8, ovf_idx, ovf_val, novf) -- expanded inside the split
             g8, v8, oi, ov, novf = packed
-            if bufs.get("xthot") is not None:
-                raise _abi.SpmfError("the 2-byte split does not build the transposed block")
             _abi.call("spmf_hot_split_u8", _ptr(self.rowptr), _ptr(g8), _ptr(v8), _ptr(oi) if novf else None,
                       _ptr(ov) if novf else None, int(novf), n, _ptr(rank), H, _ptr(bufs["rowptr"]), _ptr(bufs["cols"]),
                       _ptr(bufs["vals"]), _ptr(bufs["rowmid"]), _ptr(bufs["xhot"]), rs, lg, st)
@@ -133,18 +118,14 @@ class DeviceBatch:
             _abi.call("spmf_hot_split_packed", _ptr(self.rowptr), None if c16 is not None else _ptr(self.cols), _ptr(c16),
                       None if v16 is not None else _ptr(self.vals), _ptr(v16), n, nnz, _ptr(rank), H,
                       _ptr(bufs["rowptr"]), _ptr(bufs["cols"]), _ptr(bufs["vals"]), _ptr(bufs["rowmid"]),
-                      _ptr(bufs["xhot"]), _ptr(bufs.get("xthot")), rs, lg, st)
-        for part, pre in ((0, "h"), (1, "")):       # covered entries / the rest
-            if part == 0 and not hot_csc:
-                continue
-            _abi.call("spmf_csr_to_csc_part", _ptr(bufs["rowptr"]), _ptr(bufs["rowmid"]), part, _ptr(bufs["cols"]),
-                      _ptr(bufs["vals"]), n, self.D, _ptr(bufs[pre + "colptr"]), _ptr(bufs[pre + "crows"]),
-                      _ptr(bufs[pre + "cvals"]), _ptr(bufs["scratch"]), st)
+                      _ptr(bufs["xhot"]), rs, lg, st)
+        # CSC copy of the uncovered entries (part 1 of the partitioned CSR)
+        _abi.call("spmf_csr_to_csc_part", _ptr(bufs["rowptr"]), _ptr(bufs["rowmid"]), 1, _ptr(bufs["cols"]),
+                  _ptr(bufs["vals"]), n, self.D, _ptr(bufs["colptr"]), _ptr(bufs["crows"]), _ptr(bufs["cvals"]),
+                  _ptr(bufs["scratch"]), st)
         self.hot = HotSplit(H=H, rowptr=bufs["rowptr"], cols=bufs["cols"], vals=bufs["vals"],
-                            rowmid=bufs["rowmid"], xhot=bufs["xhot"], xthot=bufs.get("xthot"),
-                            colptr=bufs["colptr"], crows=bufs["crows"], cvals=bufs["cvals"],
-                            hcolptr=bufs["hcolptr"], hcrows=bufs["hcrows"], hcvals=bufs["hcvals"],
-                            has_hot_csc=bool(hot_csc), version=version)
+                            rowmid=bufs["rowmid"], xhot=bufs["xhot"],
+                            colptr=bufs["colptr"], crows=bufs["crows"], cvals=bufs["cvals"], version=version)
         return self.hot
 
     def ensure_csc(self):
@@ -511,10 +492,9 @@ class BatchUploader:
 
     def __init__(self, device, D, max_rows=0, max_nnz=0, hot=None):
         self.device, self.D = torch.device(device), int(D)
-        # hot = (rank, H[, need_hot_csc])
+        # hot = (rank, H[, version])
         self.hot = hot if (hot is not None and hot[0] is not None and hot[1] > 0) else None
-        self.hot_csc = bool(hot[2]) if (self.hot is not None and len(hot) > 2) else True
-        self.hot_version = int(hot[3]) if (self.hot is not None and len(hot) > 3) else 0
+        self.hot_version = int(hot[2]) if (self.hot is not None and len(hot) > 2) else 0
         self.graphs = StepGraphs()          # CUDA-graph replays of the step on this staging slot (engine.py)
         self._alloc(max_rows, max_nnz)
 
@@ -542,17 +522,12 @@ class BatchUploader:
         if self.hot is not None:
             H = int(self.hot[1])
             na = _abi._lib.spmf_umma_tiled_a_elems(max(rows, 1), _ceil64(H))
-            nt = _abi._lib.spmf_umma_tiled_a_elems(H, _ceil64(max(rows, 1)))
             self.hot_bufs = dict(rowptr=torch.empty(rows + 1, dtype=torch.int64, device=dev),
                                  cols=torch.empty(n, dtype=torch.int32, device=dev),
                                  vals=torch.empty(n, dtype=torch.float32, device=dev),
                                  rowmid=torch.empty(max(rows, 1), dtype=torch.int32, device=dev),
                                  xhot=torch.empty(na, dtype=torch.bfloat16, device=dev),
-                                 xthot=None,
-                                 colptr=self.colptr, crows=self.crows, cvals=self.cvals,
-                                 hcolptr=torch.empty(self.D + 1, dtype=torch.int32, device=dev),
-                                 hcrows=torch.empty(n, dtype=torch.int32, device=dev),
-                                 hcvals=torch.empty(n, dtype=torch.float32, device=dev), scratch=self.cursor)
+                                 colptr=self.colptr, crows=self.crows, cvals=self.cvals, scratch=self.cursor)
 
     def upload_dense(self, hb: HostDenseBatch) -> DeviceBatch:
         """Dense batch: one H2D copy of the slab, then straight to the hybrid form (tile-hybrid engines), or
@@ -567,8 +542,8 @@ class BatchUploader:
             self.graphs.drop(None)
         rawv = raw[:n * self.D].view(n, self.D)
         rawv.copy_(hb.x, non_blocking=True)
-        if self.hot is None or self.hot_csc:
-            # no fused tile kernel on the consuming engine: compact to CSR on the device (host sync for nnz)
+        if self.hot is None:
+            # the consuming engine runs the gather step: compact to CSR on the device (host sync for nnz)
             sh = CsrShard.from_dense(rawv, self.device)
             return sh.batch(0, n, cache=False)
         H, hb_ = int(self.hot[1]), self.hot_bufs
@@ -581,8 +556,7 @@ class BatchUploader:
         db = DeviceBatch(rowptr=None, cols=None, vals=None, rowsum=self.rowsum[:n], lgam=self.lgam[:n], nrows=n,
                          nnz=nnz, D=self.D, dense_raw=raw, dense_dtype=_DENSE_CODE[dt])
         db.hot = HotSplit(H=H, rowptr=hb_["rowptr"], cols=hb_["cols"], vals=hb_["vals"], rowmid=hb_["rowmid"],
-                          xhot=hb_["xhot"], xthot=None, colptr=hb_["colptr"], crows=hb_["crows"], cvals=hb_["cvals"],
-                          hcolptr=hb_["hcolptr"], hcrows=hb_["hcrows"], hcvals=hb_["hcvals"], has_hot_csc=False,
+                          xhot=hb_["xhot"], colptr=hb_["colptr"], crows=hb_["crows"], cvals=hb_["cvals"],
                           version=self.hot_version)
         db._resident, db._step_graphs, db._nnz_bound = True, self.graphs, self.cap_nnz
         return db
@@ -617,7 +591,7 @@ class BatchUploader:
                 else:
                     self.ovf_i[:novf].copy_(hb.ovf_idx, non_blocking=True)
                 self.ovf_v[:novf].copy_(hb.ovf_val, non_blocking=True)
-            if self.hot is not None and os.environ.get("SPMF_FUSED_UNPACK8", "1") != "0":
+            if self.hot is not None:
                 packed8 = (self.g8, self.v8, self.ovf_i, self.ovf_v, novf)       # ... inside the hot split
             else:
                 _abi.call("spmf_csr_unpack8", _ptr(self.rowptr), _ptr(self.g8), _ptr(self.v8), n, _ptr(self.ovf_i),
@@ -644,7 +618,7 @@ class BatchUploader:
             db = DeviceBatch(rowptr=self.rowptr[:n + 1], cols=None if (c16 is not None or packed8) else self.cols,
                              vals=None if (v16 is not None or packed8) else self.vals, rowsum=self.rowsum[:n],
                              lgam=self.lgam[:n], nrows=n, nnz=nnz, D=self.D)
-            db.ensure_hot(self.hot[0], int(self.hot[1]), bufs=self.hot_bufs, hot_csc=self.hot_csc,
+            db.ensure_hot(self.hot[0], int(self.hot[1]), bufs=self.hot_bufs,
                           row_consts=True,          # row constants come out of the split's first pass
                           packed=packed8 or (c16, v16), version=self.hot_version)
             # same device arrays for every batch through this slot: the step may be replayed as a graph

@@ -144,14 +144,9 @@ class AdviEngine:
         self.graph_launches = 0
         self.rank = None          # int32 [D]: table row of each feature (hot-column ordering), or None
         self.hot_cols = 0         # H > 0 enables the hybrid (tensor-core hot block + gather) step
-        cap = int(_abi._lib.spmf_hybrid_supported(self.K, self.S)) if self.link == 0 else 0
-        # cap 2: GEMMs + fused tile kernel (default on).  cap 1 (latent dims 64 / 128): only the count
-        # products have a tensor-core path; measured at K=128 it does not beat the gather kernels yet
-        # (5.43 vs 5.39 ms/step), so it is opt-in.
-        self.hybrid_ok = cap == 2 or (cap == 1 and os.environ.get("SPMF_WIDE_HYBRID", "0") == "1")
-        # 1: tensor cores for the two count products only; 2: also the per-nonzero terms of the hot block
-        # (fused tile kernel; latent dims <= 32 -- wider records use mode 1)
-        self.hot_mode = min(int(os.environ.get("SPMF_HOT_MODE", "2")), cap) if cap else 0
+        # tile-hybrid step: GEMMs for the count products + fused tile kernel for the per-nonzero terms
+        self.hybrid_ok = self.link == 0 and _abi._lib.spmf_hybrid_supported(self.K, self.S) != 0
+        self.hot_mode = 2 if self.hybrid_ok else 0    # spmf_hybrid_supported's code for the tile-hybrid step
         self.inv_xi = 1.0
         self._ws = None
         self._side = None
@@ -466,14 +461,16 @@ class AdviEngine:
         """Build (once) the form of `batch` this engine's step reads: the hybrid form (ranked CSR/CSC + dense
         bf16 hot block) or the plain CSC copy.  step() does it on first use; resident training loops call
         this up front so that no step pays for it."""
-        hybrid = (self.link == 0 and self.hot_cols > 0 and self.hybrid_ok and self.rank is not None
-                  and batch.nnz > 0)
+        hybrid = self._runs_hybrid(batch)
         if hybrid:
-            batch.ensure_hot(self.rank, self.hot_cols, hot_csc=(self.hot_mode != 2),
-                             version=getattr(self, "rank_version", 0))
+            batch.ensure_hot(self.rank, self.hot_cols, version=getattr(self, "rank_version", 0))
         elif self.link == 0:
             batch.ensure_csc()
         return hybrid
+
+    def _runs_hybrid(self, batch: DeviceBatch):
+        """Whether this engine steps `batch` in the hybrid form."""
+        return self.hybrid_ok and self.hot_cols > 0 and self.rank is not None and batch.nnz > 0
 
     def prime_graph(self, batch: DeviceBatch, fresh_noise=True, lr=None, clip_value=0.0):
         """Capture (without running it) the CUDA graph of this batch's step for the given configuration, so
@@ -495,11 +492,9 @@ class AdviEngine:
             w.ensure_rows(batch.nrows)
             self._args = None
             self._ws_gen += 1
-        hybrid = (self.link == 0 and self.hot_cols > 0 and self.hybrid_ok and self.rank is not None
-                  and batch.nnz > 0)
+        hybrid = self._runs_hybrid(batch)
         if hybrid:
-            h = batch.ensure_hot(self.rank, self.hot_cols, hot_csc=(self.hot_mode != 2),
-                                 version=getattr(self, "rank_version", 0))
+            h = batch.ensure_hot(self.rank, self.hot_cols, version=getattr(self, "rank_version", 0))
             if w.ensure_hybrid(self.hot_cols, batch.nrows):
                 self._args = None
                 self._ws_gen += 1
@@ -531,12 +526,11 @@ class AdviEngine:
         if hybrid:
             a.rowptr, a.cols, a.vals = _ptr(h.rowptr), _ptr(h.cols), _ptr(h.vals)
             a.colptr, a.crows, a.cvals = _ptr(h.colptr), _ptr(h.crows), _ptr(h.cvals)
-            a.hot_colptr, a.hot_crows, a.hot_cvals = _ptr(h.hcolptr), _ptr(h.hcrows), _ptr(h.hcvals)
             a.rank, a.hot_cols, a.gemm_splits = _ptr(self.rank), int(self.hot_cols), 0
-            a.rowmid, a.xhot, a.xthot = _ptr(h.rowmid), _ptr(h.xhot), _ptr(h.xthot)
+            a.rowmid, a.xhot = _ptr(h.rowmid), _ptr(h.xhot)
             a.t3_qstride = w.t3_qstride
             a.ApT3, a.dzrT3 = _ptr(w.ApT3), _ptr(w.dzrT3)
-            a.hot_mode, a.EVt = int(self.hot_mode), _ptr(w.EVt)
+            a.EVt = _ptr(w.EVt)
         else:
             a.rowptr, a.cols, a.vals = _ptr(batch.rowptr), _ptr(batch.cols), _ptr(batch.vals)
             a.colptr, a.crows, a.cvals = _ptr(batch.colptr), _ptr(batch.crows), _ptr(batch.cvals)
@@ -562,11 +556,8 @@ class AdviEngine:
             if hybrid:
                 a.ev_gemm0, a.ev_gemm1 = tev[4].cuda_event, tev[5].cuda_event
                 ev.setdefault("umma_gemm_gradA", []).append((tev[4], tev[5], batch.nnz, batch.nrows))
-                if self.hot_mode == 2:
-                    a.ev_tile0, a.ev_tile1 = tev[6].cuda_event, tev[7].cuda_event
-                    ev.setdefault("hot_tile", []).append((tev[6], tev[7], batch.nnz, batch.nrows))
-                else:
-                    a.ev_tile0 = a.ev_tile1 = None
+                a.ev_tile0, a.ev_tile1 = tev[6].cuda_event, tev[7].cuda_event
+                ev.setdefault("hot_tile", []).append((tev[6], tev[7], batch.nnz, batch.nrows))
             else:
                 a.ev_gemm0 = a.ev_gemm1 = a.ev_tile0 = a.ev_tile1 = None
         else:
@@ -580,9 +571,8 @@ class AdviEngine:
         if do_adam:
             self.opt_step += 1
         # kernels issued by spmf_advi_step (counted against the ncu launch lists under profiles/):
-        # 17 in gather mode with the split backward (16 with the one-pass backward), +5 GEMM-hybrid
-        # (2 splits, 2 GEMMs, second column kernel), +7 tile-hybrid (2 splits, 2 GEMMs, EV tiles, tile
-        # kernel, row finalisation); +1 Adam
+        # 17 in gather mode with the split backward (16 with the one-pass backward), +7 tile-hybrid
+        # (2 splits, 2 GEMMs, EV tiles, tile kernel, row finalisation); +1 Adam
         self._last_adam = (float(lr), beta1, beta2, eps, float(clip_value)) if do_adam else None
         self.tail_stepped = bool(a.adam_tail_early)     # (multi-GPU tail: the exchange skips those tensors)
         base = 17 if a.scr_dpre else 16
@@ -591,7 +581,7 @@ class AdviEngine:
         elif xd is not None:
             base += 2              # the two conditional guard launches
         n_adam = (1 if (a.adam_lr > 0 and self.world_size == 1) else 0) + (1 if a.adam_tail_early else 0)
-        self.launches += base + n_adam + ((7 if self.hot_mode == 2 else 5) if hybrid else 0)
+        self.launches += base + n_adam + (7 if hybrid else 0)
         return w.parts.view(self.S, _abi.NUM_PARTS)
 
     def _launch_step(self, a, batch, graphable, hybrid, fresh_noise, capture_only=False):
@@ -599,7 +589,7 @@ class AdviEngine:
         arrays every epoch) -- one CUDA graph launch (spmf_step_graph_launch).  The first step of every
         configuration runs eagerly: it performs the kernels' lazy one-time initialisation, which must
         not happen under stream capture."""
-        cfg = (int(fresh_noise), a.adam_lr > 0, bool(hybrid), int(self.hot_mode), int(self.link), int(a.adam_tail_early))
+        cfg = (int(fresh_noise), a.adam_lr > 0, bool(hybrid), int(self.link), int(a.adam_tail_early))
         warm = cfg in self._warm_cfgs
         if not (self.use_graphs and graphable and warm and getattr(batch, "_resident", False)):
             if capture_only:

@@ -318,11 +318,11 @@ class PoissonFactorization:
         self._set_scales_from_stats(colsum.cpu(), colnnz.cpu())
 
     def _hot_spec(self, eng):
-        """(rank, H, need_hot_csc) for the streaming uploader, decided by the engine that will consume
+        """(rank, H, version) for the streaming uploader, decided by the engine that will consume
         the batches: the hybrid form is only built when THAT engine (its S decides KP*SV) runs the
         hybrid step; otherwise batches keep their plain CSR + CSC form."""
         if eng.hybrid_ok and eng.hot_cols > 0 and eng.rank is not None:
-            return (eng.rank, int(eng.hot_cols), eng.hot_mode != 2, getattr(eng, "rank_version", 0))
+            return (eng.rank, int(eng.hot_cols), getattr(eng, "rank_version", 0))
         return None
 
     def _choose_hot_columns(self, colnnz, nrows):

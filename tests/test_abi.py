@@ -107,7 +107,7 @@ def test_step_args_struct_matches_header(tmp_path):
     from spmf_b200 import _abi
     src = tmp_path / "sz.c"
     fields = ["seed", "params", "n_params", "vsum", "rowptr", "nrows", "adam_lr", "adam_t", "caller_stream", "ev_cols1",
-              "rank", "hot_cols", "t3_qstride", "rowmid", "hot_cvals", "dzrT3", "ev_gemm1", "aux_stream2", "ev_aux_join2", "hot_mode", "EVt", "ev_tile1", "scr_dpre", "ev_noise", "step_state", "dense_raw", "dense_raw_dtype", "adam_tail_early"]
+              "rank", "hot_cols", "t3_qstride", "rowmid", "xhot", "dzrT3", "ev_gemm1", "aux_stream2", "ev_aux_join2", "EVt", "ev_tile1", "scr_dpre", "ev_noise", "link", "step_state", "dense_raw", "dense_raw_dtype", "adam_tail_early"]
     prints = "".join(f'printf("%zu\\n", offsetof(spmf_step_args, {f}));' for f in fields)
     src.write_text('#include <stdio.h>\n#include <stddef.h>\n#include "%s"\nint main(){printf("%%zu\\n", sizeof(spmf_step_args));%s return 0;}\n'
                    % (HEADER, prints))
