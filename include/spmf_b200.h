@@ -16,7 +16,7 @@
  *  - `gs` (where present, may be NULL) = device guard state (see "dense evaluation" below): the row passes
  *    raise its flag when they meet a non-finite log-likelihood, the backward / loss-part kernels read it.
  *
- * Device layouts (KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S/SV; draw s = q*SV + sv):
+ * Device layouts (KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S/SV; draw s = q*SV + sv):
  *   params / grads / adam moments : flat fp32, tensor offsets from spmf_layout()
  *                                   (order: v,w,u,s | u_eta,u_tau,s_eta,s_tau,u_eta_a,u_tau_a,s_eta_a,s_tau_a;
  *                                    each as (loc|conc_raw , scale_raw); v stored transposed as (D,K))
@@ -38,14 +38,18 @@ extern "C" {
 #define SPMF_ERR_BAD_ARG (-1)
 #define SPMF_ERR_UNSUPPORTED (-2)
 #define SPMF_ERR_PEER_TIMEOUT (-3)   /* a peer rank never reached the step's exchange (spmf_p2p_status) */
-#define SPMF_MAX_K 128
+#define SPMF_MAX_K 512        /* latent dimensions of the gather and dense paths */
+#define SPMF_MAX_TILE_K 128   /* latent dimensions of the tensor-core (tcgen05) hybrid path */
 #define SPMF_NUM_TENSORS 24
 #define SPMF_NUM_VARS 12
 #define SPMF_NUM_PARTS 16
 
 /* ---- layout helpers (host only, no device work) ---- */
 int spmf_kpad(int K);       /* latent dim padded to a power of two */
-int spmf_draw_vec(int S);   /* draws processed per vector lane: 4, 2 or 1 */
+int spmf_draw_vec(int S);   /* draws processed per vector lane: 4, 2 or 1 (the rule for K <= 128) */
+/* draws per gather record for latent dim K: the largest SV in {4,2,1} that divides S with
+ * spmf_kpad(K)*SV <= 512 floats.  Equals spmf_draw_vec(S) for K <= 128; every layout below uses it. */
+int spmf_draw_vec_k(int K, int S);
 /* position of (draw sv, latent k) inside one SV*KP-float gather record (k-vector-major, see
  * csrc/spmf_record.cuh); negative on bad arguments. */
 int spmf_rec_pos(int KP, int SV, int sv, int k);
@@ -214,7 +218,9 @@ int spmf_dense_fill(const float* x, int nrows, int D, const long long* rowptr, i
  * Column order: `rank[d]` = table row of feature d (descending column population), so the hot block
  * is rows [0,H) of every operand table.  All *_ranked entry points take rank == NULL as identity. */
 /* 0: gather kernels, 2: tile-hybrid (GEMMs + fused tile kernel; KP in {8,16,32} with REC = KP*SV in
- * {32,64,128}, or KP in {64,128}) */
+ * {32,64,128}, or KP in {64,128}).  Always 0 for K > SPMF_MAX_TILE_K: the tensor-core entry points of
+ * the tile-hybrid step (spmf_hot_ev_tiles, spmf_hot_tile, spmf_csr_rows_cold, spmf_rows_finish,
+ * spmf_csc_cols_accum) reject such K with SPMF_ERR_BAD_ARG. */
 int spmf_hybrid_supported(int K, int S);
 int spmf_draw_operands_ranked(const float* params, const float* noise, const float* eta, const int* rank,
                               int D, int K, int S, float* Ap, float* EV, float* PH, double* vsum,

@@ -14,7 +14,8 @@ LIB_PATH = os.path.join(_HERE, "lib", "libspmf_b200.so")
 NUM_TENSORS = 24
 NUM_VARS = 12
 NUM_PARTS = 16
-MAX_K = 128
+MAX_K = 512        # latent dimensions of the gather / dense kernels (SPMF_MAX_K)
+MAX_TILE_K = 128   # latent dimensions of the tensor-core hybrid path (SPMF_MAX_TILE_K)
 
 
 class SpmfError(RuntimeError):
@@ -41,6 +42,7 @@ u32 = C.c_uint
 _SIGS = {
     "spmf_kpad": (i32, [i32]),
     "spmf_draw_vec": (i32, [i32]),
+    "spmf_draw_vec_k": (i32, [i32, i32]),
     "spmf_rec_pos": (i32, [i32, i32, i32, i32]),
     "spmf_layout": (i32, [i32, i32, i32, C.POINTER(i64), C.POINTER(i64)]),
     "spmf_backward_scratch_floats": (i64, [i32, i32, i32]),
@@ -219,6 +221,11 @@ def kpad(K):
 
 def draw_vec(S):
     return _lib.spmf_draw_vec(S)
+
+
+def draw_vec_k(K, S):
+    """Draws per gather record for latent dim K (what every device layout uses)."""
+    return _lib.spmf_draw_vec_k(K, S)
 
 
 _REC_PERM = {}

@@ -667,7 +667,7 @@ int spmf_dense_encode(const float* xd, const float* eta_enc, const float* rowsum
                       int nrows, int D, int K, int S, int link, const float* Ap, float* z, void* stream) {
   if (!xd || !rowsum || !Ap || !z || !dense_shape_ok(nrows, D, K, S)) return SPMF_ERR_BAD_ARG;
   if ((link & 1) && !eta_enc) return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV;
   DenseBatch b{xd, rowsum, nullptr, eta_enc, inv_xi, scale_rows, nrows, D};
   cudaStream_t st = (cudaStream_t)stream;
 #define CALL_L(KC, L)                                                                             \
@@ -692,7 +692,7 @@ int spmf_dense_rows(const float* xd, const float* rowsum, const float* lgam, flo
   if (!xd || !rowsum || !lgam || !EV || !PH || !z || !dzr || !rowacc || !gs || !dense_shape_ok(nrows, D, K, S))
     return SPMF_ERR_BAD_ARG;
   if (mode < SPMF_DENSE_OPTIMISTIC || mode > SPMF_DENSE_GUARDED) return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV;
   DenseBatch b{xd, rowsum, lgam, nullptr, inv_xi, scale_rows, nrows, D};
   cudaStream_t st = (cudaStream_t)stream;
 #define CALL_L(KC, L)                                                                                     \
@@ -719,7 +719,7 @@ int spmf_dense_cols(const float* xd, const float* eta_enc, int nrows, int D, int
   if (!xd || !z || !EV || !PH || !GEV || !Gph || !dense_shape_ok(nrows, D, K, S)) return SPMF_ERR_BAD_ARG;
   if (with_ga && (!dzr || !GAp)) return SPMF_ERR_BAD_ARG;
   if ((link & 1) && !eta_enc) return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV;
   DenseBatch b{xd, nullptr, nullptr, eta_enc, 1.f, 0, nrows, D};
   cudaStream_t st = (cudaStream_t)stream;
 #define CALL_L(KC, L)                                                                                       \
@@ -802,7 +802,7 @@ static int guard_rows_fix_impl(const long long* rowptr, const int* cols, const f
   if (false || !rowsum || !lgam || !EV || !PH || !z || !dzr || !rowacc || !xd || !gs ||
       !dense_shape_ok(nrows, D, K, S))
     return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV;
   GuardFixArgs a{};
   a.b = DenseBatch{xd, rowsum, lgam, nullptr, inv_xi, scale_rows, nrows, D};
   a.rowptr = rowptr; a.cols = cols; a.vals = vals; a.xd = xd;
@@ -823,7 +823,7 @@ static int guard_rows_fix_impl(const long long* rowptr, const int* cols, const f
 int spmf_guard_cols_fix(int nrows, int D, int K, int S, const float* EV, const float* PH, const float* z,
                         float* GEV, float* Gph, const float* xd, void* gs, void* stream) {
   if (!EV || !PH || !z || !GEV || !Gph || !xd || !gs || !dense_shape_ok(nrows, D, K, S)) return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV;
   GuardFixArgs a{};
   a.b = DenseBatch{xd, nullptr, nullptr, nullptr, 1.f, 0, nrows, D};
   a.xd = const_cast<float*>(xd);

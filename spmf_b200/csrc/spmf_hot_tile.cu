@@ -654,8 +654,8 @@ long long spmf_hot_tile_scratch_bytes(int H, int K, int S) {
 }
 
 int spmf_hot_ev_tiles(const float* EV, const float* PH, int D, int H, int K, int S, void* EVt, void* stream) {
-  if (!EV || !PH || !EVt || D <= 0 || H <= 0 || H > D || K <= 0 || K > SPMF_MAX_K || S <= 0) return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S);
+  if (!EV || !PH || !EVt || D <= 0 || H <= 0 || H > D || K <= 0 || K > SPMF_MAX_TILE_K || S <= 0) return SPMF_ERR_BAD_ARG;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S);
   dim3 grid((H + 63) / 64, S);
   cudaStream_t st = (cudaStream_t)stream;
 #define CALL_EVT(KPC, SVC) hot_ev_tiles_kernel<KPC, SVC><<<grid, 256, 0, st>>>(EV, PH, D, H, (unsigned char*)EVt)
@@ -668,8 +668,8 @@ int spmf_hot_ev_tiles(const float* EV, const float* PH, int D, int H, int K, int
 int spmf_hot_tile(const void* xhot, const void* EVt, const float* z, int nrows, int D, int H, int K, int S,
                   float* dzacc, float* rowacc, float* GEVnz, float* Gphinz, void* gs, void* stream) {
   if (!xhot || !EVt || !z || !dzacc || !rowacc || !GEVnz || !Gphinz) return SPMF_ERR_BAD_ARG;
-  if (nrows <= 0 || D <= 0 || H <= 0 || H > D || K <= 0 || K > SPMF_MAX_K || S <= 0) return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S);
+  if (nrows <= 0 || D <= 0 || H <= 0 || H > D || K <= 0 || K > SPMF_MAX_TILE_K || S <= 0) return SPMF_ERR_BAD_ARG;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S);
   cudaStream_t st = (cudaStream_t)stream;
   int rc = SPMF_OK;
 #define CALL_HT(KPC, SVC) rc = launch_hot_tile<KPC, SVC>(xhot, EVt, z, nrows, D, H, S, dzacc, rowacc, GEVnz, Gphinz, (int*)gs, st)
@@ -680,9 +680,9 @@ int spmf_hot_tile(const void* xhot, const void* EVt, const float* z, int nrows, 
 
 int spmf_rows_finish(const float* rowsum, const float* lgam, float inv_xi, int scale_rows, int nrows, int K, int S,
                      const double* vsum, const float* z, float* dzr, float* rowacc, void* gs, void* stream) {
-  if (!rowsum || !lgam || !vsum || !z || !dzr || !rowacc || nrows <= 0 || K <= 0 || K > SPMF_MAX_K || S <= 0)
+  if (!rowsum || !lgam || !vsum || !z || !dzr || !rowacc || nrows <= 0 || K <= 0 || K > SPMF_MAX_TILE_K || S <= 0)
     return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV;
   dim3 grid((unsigned)((nrows + 3) / 4), NQ);
   cudaStream_t st = (cudaStream_t)stream;
 #define CALL_RF(KPC, SVC) rows_finish_kernel<KPC, SVC><<<grid, 128, 0, st>>>(rowsum, lgam, inv_xi, scale_rows, nrows, vsum, z, dzr, rowacc, (int*)gs)

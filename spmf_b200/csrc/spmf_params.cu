@@ -126,9 +126,10 @@ gamma_kernel(Layout L, const float* __restrict__ P, float* __restrict__ N, float
 // ------------------------------------------------------------------ draw -> operands
 // Only the four Normal-based variables enter the operands (u, v per (d,k); w, s per feature), so this
 // kernel initialises just those -- no lgamma / digamma of the InverseGamma factors (that was 80 % of
-// its instructions) -- and needs softplus(t) alone, not its derivatives.
+// its instructions) -- and needs softplus(t) alone, not its derivatives.  (Launch bounds: 0 = no
+// occupancy target; the wide instantiations, KK >= 8, ask for 3 CTAs per SM, which keeps them free of spills.)
 template <int KK>
-__global__ void __launch_bounds__(128)
+__global__ void __launch_bounds__(128, KK >= 8 ? 3 : 0)
 draw_operands_kernel(Layout L, const float* __restrict__ P, const float* __restrict__ N,
                      const float* __restrict__ eta, const int* __restrict__ rank, int SV, int KP,
                      float* __restrict__ Ap, float* __restrict__ EV, float* __restrict__ PH, int vw_identity) {
@@ -230,16 +231,21 @@ __global__ void sample_kernel(Layout L, const float* __restrict__ P, const float
 // factors the data half needs -- cu = a_d sigmoid'(u)/eta_d, cv = eta_d sigmoid'(v), uy = u/eta_d -- so
 // that backward_dk_post_kernel is a pure streaming pass.  The gradient is linear in the upstream
 // terms, so pre + post == the one-pass kernel.  PRE runs on the side stream under the data term.
+// Latent dims k0 + [0, 32*KK) of feature d: a warp covers a wide latent space in 128-wide chunks
+// (backward_dk_wide_kernel) with the register budget of KK = 4.  The first chunk stores the per-(s,d)
+// sums (da, prior / log q parts), later chunks add to them.  `lane` below is the latent index of lane 0
+// of the chunk plus the lane, as the spmf_model.cuh bodies expect (k = lane + 32 * i).
+#define SPMF_DK_PARAMS                                                                                  \
+  Layout L, Hyper h, const float *__restrict__ P, const float *__restrict__ N, const float *__restrict__ G, \
+      const float *__restrict__ eta, const int *__restrict__ rank, int SV, int KP,                       \
+      const float *__restrict__ GAp, const float *__restrict__ GEVnz, const double *__restrict__ zcolsum, \
+      float *__restrict__ grads, float *__restrict__ scr_utau, float *__restrict__ scr_parts,            \
+      float *__restrict__ scr_da, float *__restrict__ fac, const int *__restrict__ gflag
+#define SPMF_DK_ARGS L, h, P, N, G, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, fac, gflag
+
 template <int KK, bool PRE>
-__global__ void __launch_bounds__(128, KK == 1 ? 6 : 3)
-backward_dk_kernel(Layout L, Hyper h, const float* __restrict__ P, const float* __restrict__ N,
-                   const float* __restrict__ G, const float* __restrict__ eta,
-                   const int* __restrict__ rank, int SV, int KP,
-                   const float* __restrict__ GAp, const float* __restrict__ GEVnz,
-                   const double* __restrict__ zcolsum, float* __restrict__ grads,
-                   float* __restrict__ scr_utau, float* __restrict__ scr_parts,
-                   float* __restrict__ scr_da, float* __restrict__ fac, const int* __restrict__ gflag) {
-  const int lane = threadIdx.x & 31;
+__device__ __forceinline__ void backward_dk_body(SPMF_DK_PARAMS, int k0, bool first) {
+  const int wlane = threadIdx.x & 31, lane = k0 + wlane;
   const int d = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (d >= L.D) return;
   const int dr = (!PRE && rank) ? rank[d] : d;
@@ -256,7 +262,7 @@ backward_dk_kernel(Layout L, Hyper h, const float* __restrict__ P, const float* 
   float a_mine[2] = {0.f, 0.f};                    // a_d of draws lane, lane + 32 (S <= 64 on this path)
 #pragma unroll
   for (int h2 = 0; h2 < 2; ++h2) {
-    const int sm = lane + 32 * h2;
+    const int sm = wlane + 32 * h2;
     if (sm < L.S) {
       const float y0 = ndraw(s0, N[L.noff[VAR_S] + (long long)sm * 2 * L.D + d]).y;
       const float y1 = ndraw(s1, N[L.noff[VAR_S] + (long long)sm * 2 * L.D + L.D + d]).y;
@@ -308,12 +314,16 @@ backward_dk_kernel(Layout L, Hyper h, const float* __restrict__ P, const float* 
     da = warp_sum(da);
 #pragma unroll
     for (int j = 0; j < 5; ++j) pp[j] = warp_sum(pp[j]);
-    if (lane == 0) {
+    if (wlane == 0 && first) {
       if constexpr (!PRE) scr_da[(long long)s * L.D + d] = da;
       float* o = scr_parts + ((long long)d * L.S + s) * NUM_PARTS;
 #pragma unroll
       for (int j = 0; j < NUM_PARTS; ++j) o[j] = 0.f;
       o[P_U] = pp[0]; o[P_V] = pp[1]; o[P_UETA] = pp[2]; o[P_UETAA] = pp[3]; o[P_LOGQ] = pp[4];
+    } else if (wlane == 0) {
+      if constexpr (!PRE) scr_da[(long long)s * L.D + d] += da;
+      float* o = scr_parts + ((long long)d * L.S + s) * NUM_PARTS;
+      o[P_U] += pp[0]; o[P_V] += pp[1]; o[P_UETA] += pp[2]; o[P_UETAA] += pp[3]; o[P_LOGQ] += pp[4];
     }
   }
   const float invS = 1.f / (float)L.S;
@@ -329,6 +339,18 @@ backward_dk_kernel(Layout L, Hyper h, const float* __restrict__ P, const float* 
       gparam_finish(st.ua[i], P[L.toff[UETAA_C] + e], P[L.toff[UETAA_B] + e], invS, &grads[L.toff[UETAA_C] + e], &grads[L.toff[UETAA_B] + e]);
     }
   }
+}
+
+template <int KK, bool PRE>
+__global__ void __launch_bounds__(128, KK == 1 ? 6 : 3) backward_dk_kernel(SPMF_DK_PARAMS) {
+  backward_dk_body<KK, PRE>(SPMF_DK_ARGS, 0, true);
+}
+
+// KP in {256, 512}: the warp of feature d walks the latent space in chunks of 128
+template <bool PRE>
+__global__ void __launch_bounds__(128, 3) backward_dk_wide_kernel(SPMF_DK_PARAMS) {
+  if (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5) >= L.D) return;
+  for (int k0 = 0; k0 < L.K; k0 += 128) backward_dk_body<4, PRE>(SPMF_DK_ARGS, k0, k0 == 0);
 }
 
 // Data half of the backward: u and v per (d,k) -- grads += (1/S) sum_s of the upstream terms times the
@@ -786,6 +808,16 @@ int spmf_kpad(int K) {
 
 int spmf_draw_vec(int S) { return (S % 4 == 0) ? 4 : (S % 2 == 0) ? 2 : 1; }
 
+// A gather record holds at most 512 floats (one warp-wide slot of 16 floats per lane, spmf_sparse.cu):
+// wide latent spaces take fewer draws per record.  KP <= 128 always fits 4 draws, so there this is
+// spmf_draw_vec(S).
+int spmf_draw_vec_k(int K, int S) {
+  const int KP = spmf_kpad(K);
+  for (int sv = 4; sv > 1; sv >>= 1)
+    if (S % sv == 0 && (long long)KP * sv <= 512) return sv;
+  return 1;
+}
+
 int spmf_rec_pos(int KP, int SV, int sv, int k) {
   if (KP <= 0 || (KP & (KP - 1)) || SV <= 0 || sv < 0 || sv >= SV || k < 0 || k >= KP) return SPMF_ERR_BAD_ARG;
   return rec_pos(KP, SV, sv, k);
@@ -864,11 +896,14 @@ int spmf_draw_operands_ranked_m(const float* params, const float* noise, const f
   if (D <= 0 || K <= 0 || S <= 0 || K > SPMF_MAX_K) return SPMF_ERR_BAD_ARG;
   cudaStream_t st = (cudaStream_t)stream;
   Layout L = make_layout(D, K, S);
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S);
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S);
   dim3 grid((D + 3) / 4);
   if (KP <= 32) draw_operands_kernel<1><<<grid, 128, 0, st>>>(L, params, noise, eta, rank, SV, KP, Ap, EV, PH, vwid);
   else if (KP <= 64) draw_operands_kernel<2><<<grid, 128, 0, st>>>(L, params, noise, eta, rank, SV, KP, Ap, EV, PH, vwid);
-  else draw_operands_kernel<4><<<grid, 128, 0, st>>>(L, params, noise, eta, rank, SV, KP, Ap, EV, PH, vwid);
+  else if (KP <= 128) draw_operands_kernel<4><<<grid, 128, 0, st>>>(L, params, noise, eta, rank, SV, KP, Ap, EV, PH, vwid);
+  else if (KP == 256) draw_operands_kernel<8><<<grid, 128, 0, st>>>(L, params, noise, eta, rank, SV, KP, Ap, EV, PH, vwid);
+  else if (KP == 512) draw_operands_kernel<16><<<grid, 128, 0, st>>>(L, params, noise, eta, rank, SV, KP, Ap, EV, PH, vwid);
+  else return SPMF_ERR_UNSUPPORTED;
   SPMF_CHECK_LAUNCH();
   if (!vsum) return SPMF_OK;        // the caller runs spmf_operand_sums itself (on another stream)
   return spmf_operand_sums(EV, PH, D, K, S, vsum, phisum, scratch, stream);
@@ -879,7 +914,7 @@ int spmf_operand_sums(const float* EV, const float* PH, int D, int K, int S, dou
                       double* scratch, void* stream) {
   if (!EV || !PH || !vsum || !phisum || !scratch) return SPMF_ERR_BAD_ARG;
   if (D <= 0 || K <= 0 || S <= 0 || K > SPMF_MAX_K) return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV;
   return reduce_rows_pair(EV, vsum, D, KP * SV, NQ, PH, phisum, D, SV, NQ, scratch, (cudaStream_t)stream);
 }
 
@@ -948,7 +983,7 @@ int spmf_backward_params_ranked_m(const float* params, const float* noise, const
   cudaStream_t st = (cudaStream_t)stream;
   Layout L = make_layout(D, K, S);
   Hyper h = make_hyper(u_tau_scale, s_tau_scale, decay, w_entropy, w_prior, world_size, batch_rows, model);
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S);
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S);
   // float scratch: scr_utau [S][D][K] | scr_parts [D][S*16] | scr_lat [K][S*16] | scr_da [S][D]
   float* scr_utau = scr_f;
   float* scr_parts = scr_utau + (long long)S * D * K;
@@ -962,7 +997,9 @@ int spmf_backward_params_ranked_m(const float* params, const float* noise, const
   dim3 grid((D + 3) / 4);
   if (KP <= 32) backward_dk_kernel<1, false><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, nullptr, (const int*)gs);
   else if (KP <= 64) backward_dk_kernel<2, false><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, nullptr, (const int*)gs);
-  else backward_dk_kernel<4, false><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, nullptr, (const int*)gs);
+  else if (KP <= 128) backward_dk_kernel<4, false><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, nullptr, (const int*)gs);
+  else if (KP <= 512) backward_dk_wide_kernel<false><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, nullptr, (const int*)gs);
+  else return SPMF_ERR_UNSUPPORTED;
   backward_feat_kernel<<<(int)(((long long)D * SV + 127) / 128), 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, Gphinz, scr_da, grads, scr_parts, 0, (const int*)gs);
   SPMF_CHECK_LAUNCH();
   int rc = reduce_rows_pair(scr_utau, dutau, D, K, S, scr_parts, featparts, D, S * NUM_PARTS, 1, rscr, st);
@@ -1002,7 +1039,7 @@ int spmf_backward_pre_m(const float* params, const float* noise, const float* dg
   cudaStream_t st = (cudaStream_t)stream;
   Layout L = make_layout(D, K, S);
   Hyper h = make_hyper(u_tau_scale, s_tau_scale, decay, w_entropy, w_prior, world_size, batch_rows, model);
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S);
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S);
   float* scr_utau = scr_f;
   float* scr_parts = scr_utau + (long long)S * D * K;
   float* scr_lat = scr_parts + (long long)D * S * NUM_PARTS;
@@ -1015,7 +1052,9 @@ int spmf_backward_pre_m(const float* params, const float* noise, const float* dg
   dim3 grid((D + 3) / 4);
   if (KP <= 32) backward_dk_kernel<1, true><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, KP, nullptr, nullptr, nullptr, grads, scr_utau, scr_parts, scr_da, fac, nullptr);
   else if (KP <= 64) backward_dk_kernel<2, true><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, KP, nullptr, nullptr, nullptr, grads, scr_utau, scr_parts, scr_da, fac, nullptr);
-  else backward_dk_kernel<4, true><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, KP, nullptr, nullptr, nullptr, grads, scr_utau, scr_parts, scr_da, fac, nullptr);
+  else if (KP <= 128) backward_dk_kernel<4, true><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, KP, nullptr, nullptr, nullptr, grads, scr_utau, scr_parts, scr_da, fac, nullptr);
+  else if (KP <= 512) backward_dk_wide_kernel<true><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, KP, nullptr, nullptr, nullptr, grads, scr_utau, scr_parts, scr_da, fac, nullptr);
+  else return SPMF_ERR_UNSUPPORTED;
   backward_feat_kernel<<<(int)(((long long)D * SV + 127) / 128), 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, nullptr, nullptr, grads, scr_parts, 1, nullptr);
   SPMF_CHECK_LAUNCH();
   int rc = reduce_rows_pair(scr_utau, dutau, D, K, S, scr_parts, featparts, D, S * NUM_PARTS, 1, rscr, st);
@@ -1048,7 +1087,7 @@ int spmf_backward_post_m(const float* params, const float* noise, const float* e
   cudaStream_t st = (cudaStream_t)stream;
   Layout L = make_layout(D, K, S);
   Hyper h = make_hyper(u_tau_scale, s_tau_scale, decay, w_entropy, w_prior, world_size, batch_rows, model);
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S);
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S);
   float* scr_da = scr_f + (long long)S * D * K + (long long)D * S * NUM_PARTS + (long long)K * S * NUM_PARTS;
   const float* fac = scr_da + (long long)S * D;
   const double* featparts = scr_d + (long long)S * K;
@@ -1057,7 +1096,10 @@ int spmf_backward_post_m(const float* params, const float* noise, const float* e
   if (S > 64) return SPMF_ERR_BAD_ARG;
   if (KP <= 32) backward_dk_post_kernel<1><<<grid, 128, 0, st>>>(L, h, params, noise, eta, rank, SV, KP, GAp, GEVnz, Gphinz, zcolsum, fac, grads, (const int*)gs);
   else if (KP <= 64) backward_dk_post_kernel<2><<<grid, 128, 0, st>>>(L, h, params, noise, eta, rank, SV, KP, GAp, GEVnz, Gphinz, zcolsum, fac, grads, (const int*)gs);
-  else backward_dk_post_kernel<4><<<grid, 128, 0, st>>>(L, h, params, noise, eta, rank, SV, KP, GAp, GEVnz, Gphinz, zcolsum, fac, grads, (const int*)gs);
+  else if (KP <= 128) backward_dk_post_kernel<4><<<grid, 128, 0, st>>>(L, h, params, noise, eta, rank, SV, KP, GAp, GEVnz, Gphinz, zcolsum, fac, grads, (const int*)gs);
+  else if (KP == 256) backward_dk_post_kernel<8><<<grid, 128, 0, st>>>(L, h, params, noise, eta, rank, SV, KP, GAp, GEVnz, Gphinz, zcolsum, fac, grads, (const int*)gs);
+  else if (KP == 512) backward_dk_post_kernel<16><<<grid, 128, 0, st>>>(L, h, params, noise, eta, rank, SV, KP, GAp, GEVnz, Gphinz, zcolsum, fac, grads, (const int*)gs);
+  else return SPMF_ERR_UNSUPPORTED;
   finalize_parts_kernel<<<1, ((S + 31) / 32) * 32, 0, st>>>(S, SV, K, featparts, latparts, datasums, phisum,
                                                            (double)batch_rows, (double)w_entropy, (double)w_prior,
                                                            parts, grads + L.comm_off, (GuardState*)gs);
@@ -1163,7 +1205,7 @@ int spmf_batch_sums(const float* z, const float* rowacc, int nrows, int K, int S
                     double* datasums, double* scratch, void* stream) {
   if (!z || !rowacc || !zcolsum || !datasums || !scratch || nrows <= 0 || K <= 0 || K > SPMF_MAX_K || S <= 0)
     return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV;
   return reduce_rows_pair(z, zcolsum, nrows, KP * SV, NQ, rowacc, datasums, nrows, 4 * SV, NQ, scratch,
                           (cudaStream_t)stream);
 }

@@ -38,6 +38,7 @@ struct Map {
   static constexpr int VPL = NV < 4 ? NV : 4;            // vectors per lane (<= 16 latent dims)
   static constexpr int RG = NV / VPL;                    // lanes sharing one draw
   static constexpr int LPN = SV * RG;                    // lanes per nonzero slot (<= 32)
+  static_assert(LPN <= 32, "a nonzero slot must fit in one warp (REC = SV*KP <= 512)");
   static constexpr int REC = SV * KP;                    // floats per record
   static constexpr int THREADS = 128;
   static constexpr int NSLOT = THREADS / LPN;            // slots per CTA
@@ -465,7 +466,7 @@ constexpr int kSliceLen = 256;
 
 // `nnz_bound` sizes the grid; the actual count is colptr[D] (known on the device only).
 template <int KP, int SV>
-__global__ void __launch_bounds__(128, 4)
+__global__ void __launch_bounds__(128, KP > 128 ? 3 : 4)
 csc_cols_kernel(const int* __restrict__ colptr, const int* __restrict__ rows,
                 const float* __restrict__ vals, int nnz_bound, int nrows, int D,
                 const float* __restrict__ z, const float* __restrict__ dzr,
@@ -1397,6 +1398,14 @@ static int launch_cols(const int* colptr, const int* rows, const float* vals, in
       case 32: SPMF_DISPATCH_SV(32, SV, CALL); break;                        \
       case 64: SPMF_DISPATCH_SV(64, SV, CALL); break;                        \
       case 128: SPMF_DISPATCH_SV(128, SV, CALL); break;                      \
+      /* wide records: SV = spmf_draw_vec_k(K, S) keeps SV*KP <= 512 */       \
+      case 256:                                                              \
+        if (SV == 2) { CALL(256, 2); } else if (SV == 1) { CALL(256, 1); }   \
+        else return SPMF_ERR_UNSUPPORTED;                                    \
+        break;                                                               \
+      case 512:                                                              \
+        if (SV == 1) { CALL(512, 1); } else return SPMF_ERR_UNSUPPORTED;     \
+        break;                                                               \
       default: return SPMF_ERR_UNSUPPORTED;                                  \
     }                                                                        \
   } while (0)
@@ -1427,7 +1436,7 @@ int spmf_csr_rows(const long long* rowptr, const int* cols, const float* vals, c
     return SPMF_ERR_BAD_ARG;
   if (nrows <= 0 || D <= 0 || K <= 0 || K > SPMF_MAX_K || S <= 0) return SPMF_ERR_BAD_ARG;
   if (variant != 0) return SPMF_ERR_UNSUPPORTED;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV;
   cudaStream_t st = (cudaStream_t)stream;
   int rc = SPMF_OK;
 #define CALL_ROWS(KPC, SVC) rc = launch_rows<KPC, SVC, kRowsTrain>(rowptr, cols, vals, rowsum, lgam, inv_xi, scale_rows, nrows, D, NQ, Ap, EV, PH, vsum, z, dzr, rowacc, nullptr, (int*)gs, st)
@@ -1441,7 +1450,7 @@ int spmf_csr_encode(const long long* rowptr, const int* cols, const float* vals,
                     float* z, void* stream) {
   if (!rowptr || !cols || !vals || !rowsum || !Ap || !z) return SPMF_ERR_BAD_ARG;
   if (nrows <= 0 || D <= 0 || K <= 0 || K > SPMF_MAX_K || S <= 0) return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV;
   cudaStream_t st = (cudaStream_t)stream;
   int rc = SPMF_OK;
 #define CALL_ENC(KPC, SVC) rc = launch_rows<KPC, SVC, kRowsEncode>(rowptr, cols, vals, rowsum, nullptr, inv_xi, scale_rows, nrows, D, NQ, Ap, nullptr, nullptr, nullptr, z, nullptr, nullptr, nullptr, nullptr, st)
@@ -1456,7 +1465,7 @@ int spmf_csc_cols(const int* colptr, const int* rows, const float* vals, int nnz
   if (!colptr || !rows || !vals || !z || !dzr || !EV || !PH || !GAp || !GEVnz || !Gphinz) return SPMF_ERR_BAD_ARG;
   if (nnz < 0 || nrows <= 0 || D <= 0 || K <= 0 || K > SPMF_MAX_K || S <= 0) return SPMF_ERR_BAD_ARG;
   if (variant != 0) return SPMF_ERR_UNSUPPORTED;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV;
   cudaStream_t st = (cudaStream_t)stream;
   const size_t nb = (size_t)NQ * D * KP * SV * sizeof(float);
   cudaError_t e = cudaMemsetAsync(GAp, 0, nb, st);
@@ -1491,8 +1500,8 @@ int spmf_csc_cols(const int* colptr, const int* rows, const float* vals, int nnz
 
 /* 0: gather kernels only; 2: tile-hybrid (GEMMs + fused tile kernel, spmf_hot_tile.cu) */
 int spmf_hybrid_supported(int K, int S) {
-  if (K <= 0 || K > SPMF_MAX_K || S <= 0) return 0;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S);
+  if (K <= 0 || K > SPMF_MAX_TILE_K || S <= 0) return 0;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S);
   if ((KP == 32 && (SV == 4 || SV == 2 || SV == 1)) || (KP == 16 && (SV == 4 || SV == 2)) || (KP == 8 && SV == 4))
     return 2;
   if (KP == 64 || KP == 128) return 2;     // fused tile kernel with 64 / 128 latent dims (spmf_hot_tile.cu)
@@ -1505,8 +1514,8 @@ int spmf_csr_rows_cold(const long long* rowptr, const int* cols, const float* va
                        void* gs, void* stream) {
   if (!rowptr || !cols || !vals || !rowmid || !rowsum || !Ap || !EV || !PH || !z || !dzacc || !rowacc)
     return SPMF_ERR_BAD_ARG;
-  if (nrows <= 0 || D <= 0 || K <= 0 || K > SPMF_MAX_K || S <= 0) return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
+  if (nrows <= 0 || D <= 0 || K <= 0 || K > SPMF_MAX_TILE_K || S <= 0) return SPMF_ERR_BAD_ARG;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV;
   cudaStream_t st = (cudaStream_t)stream;
   int rc = SPMF_OK;
 #define CALL_ROWS_C(KPC, SVC) rc = launch_rows<KPC, SVC, kRowsCold>(rowptr, cols, vals, rowsum, nullptr, inv_xi, scale_rows, nrows, D, NQ, Ap, EV, PH, nullptr, z, dzacc, rowacc, rowmid, (int*)gs, st)
@@ -1517,7 +1526,7 @@ int spmf_csr_rows_cold(const long long* rowptr, const int* cols, const float* va
 
 int spmf_zero_col_grads(float* GAp, float* GEVnz, float* Gphinz, int D, int K, int S, void* stream) {
   if (!GAp || !GEVnz || !Gphinz || D <= 0 || K <= 0 || K > SPMF_MAX_K || S <= 0) return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV;
   cudaStream_t st = (cudaStream_t)stream;
   const size_t nb = (size_t)NQ * D * KP * SV * sizeof(float);
   cudaError_t e = cudaMemsetAsync(GAp, 0, nb, st);
@@ -1530,8 +1539,8 @@ int spmf_csc_cols_accum(const int* colptr, const int* rows, const float* vals, i
                         int K, int S, const float* z, const float* dzr, const float* EV, const float* PH,
                         float* GAp, float* GEVnz, float* Gphinz, void* stream) {
   if (!colptr || !rows || !vals || !z || !dzr || !EV || !PH || !GAp || !GEVnz || !Gphinz) return SPMF_ERR_BAD_ARG;
-  if (nnz_bound < 0 || nrows <= 0 || D <= 0 || K <= 0 || K > SPMF_MAX_K || S <= 0) return SPMF_ERR_BAD_ARG;
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV;
+  if (nnz_bound < 0 || nrows <= 0 || D <= 0 || K <= 0 || K > SPMF_MAX_TILE_K || S <= 0) return SPMF_ERR_BAD_ARG;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV;
   cudaStream_t st = (cudaStream_t)stream;
   int rc = SPMF_OK;
   // sparse remainder: short slices keep every SM busy on a small stream

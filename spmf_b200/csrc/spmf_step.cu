@@ -79,7 +79,7 @@ int spmf_advi_step(const spmf_step_args* a) {
   STEP_TRY(spmf_draw_operands_ranked_m(a->params, a->noise, a->eta, hybrid ? a->rank : nullptr, D, K, S, a->Ap,
                                        a->EV, a->PH, pre_fork ? nullptr : a->vsum, pre_fork ? nullptr : a->phisum,
                                        a->scr_d, a->model, hot));
-  const int KP = spmf_kpad(K), SV = spmf_draw_vec(S), NQ = S / SV, REC = KP * SV;
+  const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S), NQ = S / SV, REC = KP * SV;
   if (a->ev_rows0) CUDA_TRY(cudaEventRecord((cudaEvent_t)a->ev_rows0, hot));
   const bool dense_link = a->link != SPMF_LINK_POISSON;
   if (dense_link) {

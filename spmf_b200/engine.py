@@ -24,7 +24,7 @@ class StepWorkspace:
 
     def __init__(self, D, K, S, max_rows, device):
         self.D, self.K, self.S = D, K, S
-        self.KP, self.SV = _abi.kpad(K), _abi.draw_vec(S)
+        self.KP, self.SV = _abi.kpad(K), _abi.draw_vec_k(K, S)
         self.NQ = S // self.SV
         self.max_rows = 0
         self.device = device

@@ -334,7 +334,7 @@ class PoissonFactorization:
             return                      # dense links: no closed form, no hot / cold split
         self._rank_version = getattr(self, "_rank_version", 0) + 1     # invalidates cached hybrid forms
         # (whether a given engine uses the hot block is its own decision: hybrid_ok depends on S)
-        if self.hot_density <= 0 or nrows <= 0 or self.latent_dim > _abi.MAX_K:
+        if self.hot_density <= 0 or nrows <= 0 or self.latent_dim > _abi.MAX_TILE_K:
             return
         order = torch.argsort(colnnz.to(torch.float64), descending=True, stable=True)
         H = int((colnnz.to(torch.float64) >= self.hot_density * nrows).sum().item())
