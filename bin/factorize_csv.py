@@ -8,7 +8,9 @@ followed by the row's encoding), written after ADVI calibration.  Differences: t
 `spmf_b200.PoissonFactorization` (current API of mederrata_spmf/poisson.py instead of the legacy
 `PoissonMatrixFactorization` the reference script still imports); the count matrix is held on the
 device as CSR; the forest-plot PDF of the reference (matplotlib + arviz, bin/factorize_csv.py:141-183)
-is not produced; `--log-transform` is rejected (no CUDA path).
+is not produced; `--log-transform` is rejected (no CUDA path).  `--checkpoint PATH` writes a training
+checkpoint every `--checkpoint-every` epochs and, when PATH exists, resumes the run from it (`-e` counts the
+epochs of the whole run); the output files are the same either way.
 """
 import argparse
 import csv
@@ -34,6 +36,11 @@ def build_parser():
     parser.add_argument('-rn', '--row-normalize', help='Row normalize based on counts?', action='store_true')
     parser.add_argument('--sample-size', type=int, default=8, help='Monte-Carlo draws per step (not in the reference CLI)')
     parser.add_argument('--device', type=str, default='cuda', help='CUDA device (not in the reference CLI)')
+    parser.add_argument('--checkpoint', type=str, default=None,
+                        help='Checkpoint file: written during training; if it exists, training resumes from it '
+                             '(-e counts the epochs of the whole run) (not in the reference CLI)')
+    parser.add_argument('--checkpoint-every', type=int, default=1,
+                        help='Epochs between checkpoints. Default: 1 (not in the reference CLI)')
     return parser
 
 
@@ -75,7 +82,8 @@ def main(argv=None):
     factor.calibrate_advi(
         lambda: ({'counts': b} for b in shard.iter_batches(batch, drop_remainder=drop)),
         num_steps=args.epoch, rel_tol=1e-4, clip_value=args.clip_value, learning_rate=args.learning_rate,
-        sample_size=args.sample_size)                            # :121-124
+        sample_size=args.sample_size,                            # :121-124
+        checkpoint_path=args.checkpoint, checkpoint_every=args.checkpoint_every, resume=True)
 
     enc_name, model_name, rep_name = output_names(args.csv_file, args.dimension, args.log_transform, args.row_normalize)
     print("Saving the encoding matrix")

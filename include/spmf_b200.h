@@ -186,6 +186,12 @@ int spmf_p2p_close(void* ptr);
 long long spmf_p2p_flag_bytes(void);
 int spmf_p2p_status(const void* flags, void* stream);
 int spmf_p2p_reduce_adam(const spmf_p2p_args* args, void* stream);
+/* Host-only: the floats [*lo, *hi) of the reduced block [0, comm_off) whose sum, Adam update and moments belong
+ * to `rank` in spmf_p2p_reduce_adam (comm_off a multiple of 4, 1 <= world <= SPMF_P2P_MAX_WORLD).  The ranges of
+ * ranks 0..world-1 follow each other and cover the block once; a rank may own an empty range.  With the
+ * peer-memory exchange, adam_m / adam_v of a rank are current only inside its own range: a checkpoint gathers
+ * them by it. */
+int spmf_p2p_owned_range(long long comm_off, int world, int rank, long long* lo, long long* hi);
 
 /* ---- data formats either side of the path ---- */
 /* compute_scales (poisson.py:113-154): colsum[D] (double) and colnnz[D] (float, as the reference

@@ -188,6 +188,7 @@ _SIGS["spmf_p2p_close"] = (i32, [p])
 _SIGS["spmf_p2p_flag_bytes"] = (i64, [])
 _SIGS["spmf_p2p_status"] = (i32, [p, p])
 _SIGS["spmf_p2p_reduce_adam"] = (i32, [p, p])
+_SIGS["spmf_p2p_owned_range"] = (i32, [i64, i32, i32, C.POINTER(i64), C.POINTER(i64)])
 
 EXPORTS = tuple(_SIGS)
 
@@ -247,6 +248,14 @@ def layout(D, K, S):
     n = (i64 * (NUM_VARS + 1))()
     _check(_lib.spmf_layout(D, K, S, t, n), "spmf_layout")
     return list(t), list(n)
+
+
+def p2p_owned_range(comm_off, world, rank):
+    """Floats [lo, hi) of the reduced block whose Adam moments `rank` holds under the peer-memory exchange."""
+    lo, hi = i64(), i64()
+    _check(_lib.spmf_p2p_owned_range(int(comm_off), int(world), int(rank), C.byref(lo), C.byref(hi)),
+           "spmf_p2p_owned_range")
+    return lo.value, hi.value
 
 
 def backward_scratch(D, K, S):

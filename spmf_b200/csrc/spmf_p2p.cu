@@ -53,6 +53,18 @@ __device__ __forceinline__ unsigned ld_acquire_sys(const unsigned* p) {
 // wrap-safe "flag has reached epoch"
 __device__ __forceinline__ bool reached(unsigned flag, unsigned epoch) { return (int)(flag - epoch) >= 0; }
 
+// float4 vectors [v0, v1) of the reduced block (nvec vectors) whose sum, Adam update and moments belong to
+// `rank`: ceil(nvec / world) consecutive vectors per rank, in rank order.  The exchange kernel and
+// spmf_p2p_owned_range (checkpoints gather the moments by it) both use this one definition.  (`rank` by
+// reference: the kernel then reads a.rank where the product needs it, and compiles to the same SASS as with
+// the formula written inline.)
+__host__ __device__ __forceinline__ void owned_vecs(long long nvec, int world, const int& rank, long long* v0,
+                                                   long long* v1) {
+  const long long per = (nvec + world - 1) / world;
+  *v0 = min(nvec, per * rank);
+  *v1 = min(nvec, *v0 + per);
+}
+
 struct P2PArgs {
   int world, rank, S, slack;
   unsigned epoch;
@@ -104,8 +116,8 @@ p2p_reduce_adam_kernel(const P2PArgs a) {
   if (live) {
     // ---- 2. my slice of the reduced block, 4 floats at a time
     const long long nvec = a.comm_off / 4;                      // (comm_off is a multiple of 4: checked on the host)
-    const long long per = (nvec + W - 1) / W;
-    const long long v0 = min(nvec, per * a.rank), v1 = min(nvec, v0 + per);
+    long long v0, v1;
+    owned_vecs(nvec, W, a.rank, &v0, &v1);
     for (long long i = v0 + tid; i < v1; i += nthr) {
       float4 g[SPMF_P2P_MAX_WORLD];
 #pragma unroll
@@ -221,6 +233,16 @@ int spmf_p2p_open(const unsigned char* handle64, void** ptr) {
 int spmf_p2p_close(void* ptr) { return ptr ? (int)cudaIpcCloseMemHandle(ptr) : SPMF_OK; }
 
 long long spmf_p2p_flag_bytes(void) { return 4096; }
+
+int spmf_p2p_owned_range(long long comm_off, int world, int rank, long long* lo, long long* hi) {
+  if (comm_off < 0 || (comm_off & 3) || world < 1 || world > SPMF_P2P_MAX_WORLD || rank < 0 || rank >= world || !lo || !hi)
+    return SPMF_ERR_BAD_ARG;
+  long long v0, v1;
+  owned_vecs(comm_off / 4, world, rank, &v0, &v1);
+  *lo = 4 * v0;
+  *hi = 4 * v1;
+  return SPMF_OK;
+}
 
 int spmf_p2p_status(const void* flags, void* stream) {
   // host-synchronous read of the give-up flag (diagnostics; not on the step path)

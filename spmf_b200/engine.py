@@ -9,6 +9,7 @@ launches over five streams in hybrid mode) instead of a TensorFlow graph, never 
 """
 from __future__ import annotations
 
+import itertools
 import os
 from typing import Optional
 
@@ -17,6 +18,10 @@ import torch
 from . import _abi
 from .data import DeviceBatch, StepGraphs as _StepGraphs, _ptr, _stream
 from .variables import VariableLayout, PART_NAMES
+
+# engine serial numbers: the key of an engine's cached step graphs (an id() may be reused by a later engine, e.g.
+# one loaded from a checkpoint in the same process, whose graphs would then replay the freed engine's buffers)
+_ENGINE_SERIAL = itertools.count()
 
 
 class StepWorkspace:
@@ -142,6 +147,7 @@ class AdviEngine:
         self._ws_gen = 0                  # bumped whenever a workspace buffer moves: invalidates graphs
         self._warm_cfgs = set()
         self.graph_launches = 0
+        self._serial = next(_ENGINE_SERIAL)
         self.rank = None          # int32 [D]: table row of each feature (hot-column ordering), or None
         self.hot_cols = 0         # H > 0 enables the hybrid (tensor-core hot block + gather) step
         # tile-hybrid step: GEMMs for the count products + fused tile kernel for the per-nonzero terms
@@ -601,7 +607,7 @@ class AdviEngine:
         cache = batch.__dict__.get("_step_graphs")
         if cache is None:
             cache = batch.__dict__["_step_graphs"] = _StepGraphs()
-        key = (id(self), self._ws_gen) + cfg + (batch.nrows, int(a.nnz), getattr(self, "rank_version", 0),
+        key = (self._serial, self._ws_gen) + cfg + (batch.nrows, int(a.nnz), getattr(self, "rank_version", 0),
                                                   a.inv_xi, a.scale_rows, a.rowptr, a.xhot)
         h = cache.handles.get(key)
         if h is None:

@@ -73,6 +73,24 @@ def exchange_kind(eng):
     return "p2p-kernel" if (link is not None and link.ok) else "nccl-allreduce"
 
 
+def gather_owned(eng, t, group=None):
+    """Full copy of a per-parameter buffer (adam_m / adam_v or a snapshot of them) of which, under the peer-memory
+    exchange, each rank holds only its owned slice of the reduced block current (spmf_p2p_owned_range); the
+    replicated tail [n_data_block, n_params) is the same on every rank and is taken from this one.  Collective."""
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    spans = [_abi.p2p_owned_range(eng.layout.comm_off, world, q) for q in range(world)]
+    width = max(hi - lo for lo, hi in spans)
+    lo, hi = spans[rank]
+    mine = torch.zeros(width, dtype=t.dtype, device=t.device)
+    mine[:hi - lo] = t[lo:hi]
+    pieces = [torch.empty_like(mine) for _ in range(world)]
+    dist.all_gather(pieces, mine, group=group)
+    full = t.clone()
+    for (a, b), piece in zip(spans, pieces):
+        full[a:b] = piece[:b - a]
+    return full
+
+
 def allreduce_step(eng, parts, group=None, adam=False):
     """All-reduce gradients + data parts in one collective; returns the global loss (0-d tensor).
     adam=True: the optimiser step (all 24 tensors; the 16 replicated ones are bit-identical on every rank)

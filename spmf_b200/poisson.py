@@ -37,6 +37,20 @@ from .engine import AdviEngine
 from .variables import VAR_LIST, NORMAL_VARS, var_shapes
 
 LINK_CUSTOM = 64      # host-side only: user-supplied encoder / decoder callables (data term in torch, engine.custom_forward)
+CHECKPOINT_VERSION = 1   # layout of the 'training' entry that save_checkpoint adds to state()
+
+
+def _pickle_module():
+    try:
+        import dill as _pk          # (custom encoder / decoder callables are dill pickles)
+    except ImportError:             # pragma: no cover - dill ships with the image
+        _pk = pickle
+    return _pk
+
+
+def _read_state(filename):
+    with open(filename, 'rb') as f:
+        return _pickle_module().load(f)
 
 
 def waic_terms(ll):
@@ -186,6 +200,7 @@ class PoissonFactorization:
         self.calibrated_expectations = {}
         self._last_data_factory = None
         self._engines: Dict[int, AdviEngine] = {}
+        self._pending_counters = {}     # S -> (opt_step, rng_step) of a loaded checkpoint, for engines not created yet
         self._params = None
         if initialize_distributions:
             self.create_distributions()
@@ -221,6 +236,7 @@ class PoissonFactorization:
         self.bijectors = {k: 'softplus' for k in VAR_LIST}          # all Softplus, poisson.py:215-224,297-301
         self.var_list = list(VAR_LIST)                               # poisson.py:572
         self._engines = {}
+        self._pending_counters = {}
         self._params = None
         eng = self._engine_for(1)
         self._params = eng.params
@@ -251,6 +267,8 @@ class PoissonFactorization:
                 eng.adam_m, eng.adam_v = first.adam_m, first.adam_v
             self._engines[S] = eng
             self._push_scales(eng)
+            if S in self._pending_counters:
+                eng.opt_step, eng.rng_step = self._pending_counters.pop(S)
         return self._engines[S]
 
     def _push_scales(self, eng):
@@ -640,19 +658,41 @@ class PoissonFactorization:
     def fit(self, batched_data_factory, batch_size=None, dataset_size=None, num_steps=100,
             learning_rate=0.01, rel_tol=1e-4, abs_tol=None, clip_value=0.0, sample_size=8,
             sample_batches=1, max_decay_steps=25, lr_decay_factor=0.99, patience=5, verbose=True,
-            **kwargs):
+            checkpoint_path=None, checkpoint_every=1, resume=False, **kwargs):
         """Minibatch ADVI (call site tests/spmf_test.py:35-43).  [EXT] behaviour restated from the
         reference's notebook logs (SURVEY.md section 5): an epoch is one pass over
         `batched_data_factory()`; the mean batch loss is tracked; on improvement the parameters are
         snapshotted, on a plateau the learning rate decays by `lr_decay_factor` and the best
         snapshot is restored; stops on rel_tol / abs_tol / max_decay_steps / num_steps.
-        Returns the list of epoch losses."""
+        Returns the list of epoch losses.
+
+        `checkpoint_path`: write a checkpoint (save_checkpoint, plus the state of this loop) after every
+        `checkpoint_every` epochs, after the last epoch and when the loop stops early.  `resume=True` with an
+        existing `checkpoint_path`: continue the run stored there (parameters, optimiser, counters, column
+        ranking, epoch, losses, learning rate, best snapshot); `num_steps` counts the epochs of the whole run and
+        the returned list includes the epochs before the resume."""
         self._last_data_factory = batched_data_factory
         S = int(sample_size) * int(sample_batches)
         eng = self._engine_for(S)
         losses, best, best_state = [], float('inf'), None
         lr, decays, since_best = float(learning_rate), 0, 0
-        for epoch in range(int(num_steps)):
+        if checkpoint_path is not None and int(checkpoint_every) < 1:
+            raise ValueError("checkpoint_every must be >= 1")
+        start, stopped = 0, False
+        if resume and checkpoint_path is not None and os.path.exists(checkpoint_path):
+            loop = self._apply_checkpoint(_read_state(checkpoint_path))
+            if loop is not None:
+                start, stopped, losses = int(loop['epoch']), bool(loop['stopped']), list(loop['losses'])
+                lr, decays, since_best, best = float(loop['lr']), int(loop['decays']), int(loop['since_best']), float(loop['best'])
+                bs = loop['best_state']
+                if bs is not None:
+                    best_state = tuple(t.to(self.device) for t in bs[:3]) + (int(bs[3]),)
+                if verbose:
+                    print(f"Resuming from {checkpoint_path} at epoch {start}")
+        if stopped:                    # the stored run had already met its stopping rule
+            self.set_calibration_expectations()
+            return losses
+        for epoch in range(start, int(num_steps)):
             acc = torch.zeros((), dtype=torch.float64, device=self.device)
             nb, last = 0, None
             batches = batched_data_factory()
@@ -672,6 +712,7 @@ class PoissonFactorization:
             losses.append(mean_loss)
             if verbose:
                 print(f"Epoch {epoch}: average-batch loss: {mean_loss} last batch loss: {float(last.item())}")
+            stop = False
             if not math.isfinite(mean_loss):
                 if best_state is not None:
                     if verbose:
@@ -686,9 +727,9 @@ class PoissonFactorization:
                 best_state = self._snapshot(eng)
                 if math.isfinite(prev_best):
                     if abs_tol is not None and improved < abs_tol:
-                        break
-                    if rel_tol is not None and improved < rel_tol * abs(prev_best):
-                        break
+                        stop = True
+                    elif rel_tol is not None and improved < rel_tol * abs(prev_best):
+                        stop = True
             else:
                 since_best += 1
                 if since_best >= patience:
@@ -699,6 +740,13 @@ class PoissonFactorization:
                         print(f"New learning rate: {lr}")
                     self._restore(eng, best_state)
             if decays >= max_decay_steps:
+                stop = True
+            if checkpoint_path is not None and (stop or epoch + 1 == int(num_steps)
+                                                or (epoch + 1) % int(checkpoint_every) == 0):
+                self._write_checkpoint(checkpoint_path, dict(
+                    epoch=epoch + 1, stopped=stop, losses=list(losses), lr=lr, decays=decays,
+                    since_best=since_best, best=best, best_state=best_state))
+            if stop:
                 break
         else:
             if verbose:
@@ -766,12 +814,115 @@ class PoissonFactorization:
     def save(self, filename):
         """[EXT] BayesianModel.save (a dill pickle in the reference; bin/factorize_csv.py:136-139).  The
         state is plain tensors / floats, so the file loads with either dill or pickle."""
-        try:
-            import dill as _pk
-        except ImportError:          # pragma: no cover - dill ships with the image
-            _pk = pickle
         with open(filename, 'wb') as f:
-            _pk.dump(self.state(), f)
+            _pickle_module().dump(self.state(), f)
+
+    def save_checkpoint(self, path):
+        """Write what training needs to continue exactly where it stands: state() plus a 'training' entry with
+        the flat parameters, the Adam moments, the optimiser and Philox counters of every engine, and the
+        hot-column ranking (see _training_state).  `load` restores all of it.  The file is written to
+        `path + '.tmp'` and renamed, so an interrupted write leaves the previous checkpoint intact.  Under
+        torch.distributed the call is collective: every rank calls it, rank 0 writes."""
+        self._write_checkpoint(path, None)
+
+    def _moment_gatherer(self, eng):
+        """t -> full copy of a moment buffer.  With the peer-memory exchange a rank keeps the moments of its own
+        slice of the data block only (csrc/spmf_p2p.cu): the slices are gathered from all ranks (collective)."""
+        if eng.world_size > 1:
+            from .parallel import exchange_kind, gather_owned
+            if exchange_kind(eng) == "p2p-kernel":
+                return lambda t: gather_owned(eng, t, self.process_group)
+        return lambda t: t
+
+    def _training_state(self, loop=None):
+        """The 'training' entry of a checkpoint (CPU tensors and plain values).  `loop`: the state of fit()."""
+        eng = self._engine_for(1)
+        full = self._moment_gatherer(eng)
+        counters = dict(self._pending_counters)
+        counters.update({S: (int(e.opt_step), int(e.rng_step)) for S, e in self._engines.items()})
+        tr = {
+            'version': CHECKPOINT_VERSION, 'model': int(self._model_id), 'link': int(self.link),
+            'params': eng.params.detach().to('cpu', copy=True),
+            'adam_m': full(eng.adam_m).to('cpu', copy=True), 'adam_v': full(eng.adam_v).to('cpu', copy=True),
+            'counters': counters,
+            'col_rank': None if self.col_rank is None else self.col_rank.to('cpu', torch.int32, copy=True),
+            'hot_cols': int(self.hot_cols), 'hot_density': float(self.hot_density),
+            'exact_guard': bool(self.exact_guard), 'rank_version': int(getattr(self, '_rank_version', 0)),
+        }
+        if loop is not None:
+            loop = dict(loop)
+            bs = loop['best_state']
+            if bs is not None:
+                loop['best_state'] = (bs[0].to('cpu', copy=True), full(bs[1]).to('cpu', copy=True),
+                                      full(bs[2]).to('cpu', copy=True), int(bs[3]))
+            tr['fit'] = loop
+        return tr
+
+    def _write_checkpoint(self, path, loop):
+        path = os.fspath(path)
+        ck = self.state()
+        ck['training'] = self._training_state(loop)
+        dist_on = torch.distributed.is_available() and torch.distributed.is_initialized()
+        err = None
+        if not dist_on or torch.distributed.get_rank(self.process_group) == 0:
+            try:
+                tmp = path + ".tmp"
+                with open(tmp, 'wb') as f:
+                    _pickle_module().dump(ck, f)
+                    f.flush()
+                    os.fsync(f.fileno())
+                os.replace(tmp, path)
+            except Exception as e:     # noqa: BLE001 -- re-raised below, after the other ranks learn of it
+                err = e
+        if dist_on:                    # every rank returns once the file is in place, or raises with rank 0
+            ok = torch.tensor([0.0 if err else 1.0], device=self.device)
+            torch.distributed.all_reduce(ok, op=torch.distributed.ReduceOp.MIN, group=self.process_group)
+            if err is None and float(ok.item()) == 0.0:
+                raise _abi.SpmfError(f"rank 0 could not write the checkpoint {path}")
+        if err is not None:
+            raise err
+
+    def _restore_training(self, tr):
+        """Take over the 'training' entry of a checkpoint: parameters, moments (full on every rank: only a rank's
+        owned slice is read under the peer-memory exchange), ranking, and the counters of every engine -- those
+        of engines not created yet are applied when _engine_for creates them."""
+        if tr.get('version') != CHECKPOINT_VERSION:
+            raise _abi.SpmfError(f"checkpoint format {tr.get('version')} is not {CHECKPOINT_VERSION}")
+        if int(tr['model']) != self._model_id or int(tr['link']) != self.link:
+            raise _abi.SpmfError(f"checkpoint of model {tr['model']} / link {tr['link']} cannot resume "
+                                 f"{type(self).__name__} (model {self._model_id} / link {self.link})")
+        eng = self._engine_for(1)
+        n = eng.layout.n_params
+        if any(tuple(tr[k].shape) != (n,) for k in ('params', 'adam_m', 'adam_v')):
+            raise _abi.SpmfError(f"checkpoint holds {tuple(tr['params'].shape)} parameters, this model {n}")
+        eng.params.copy_(tr['params'])
+        eng.adam_m.copy_(tr['adam_m'])
+        eng.adam_v.copy_(tr['adam_v'])
+        self.hot_density, self.exact_guard = float(tr['hot_density']), bool(tr['exact_guard'])
+        rank = tr['col_rank']
+        self.col_rank = None if rank is None else rank.to(device=self.device, dtype=torch.int32)
+        self.hot_cols, self._rank_version = int(tr['hot_cols']), int(tr['rank_version'])
+        counters = {int(S): (int(a), int(b)) for S, (a, b) in tr['counters'].items()}
+        for S, e in self._engines.items():
+            self._push_scales(e)
+            e.exact_guard = self.exact_guard
+            e.opt_step, e.rng_step = counters.pop(S, (0, 0))
+        self._pending_counters = counters
+
+    def _apply_checkpoint(self, state):
+        """fit(resume=True): take over the scales and training state of a checkpoint; returns fit's loop state
+        (None when the checkpoint was written by save_checkpoint)."""
+        tr = state.get('training')
+        if tr is None:
+            raise _abi.SpmfError("the file has no training state (written by save(), not save_checkpoint())")
+        hy = state['hyper']
+        if (int(hy['feature_dim']), int(hy['latent_dim'])) != (self.feature_dim, self.latent_dim):
+            raise _abi.SpmfError(f"checkpoint of D={hy['feature_dim']}, K={hy['latent_dim']} cannot resume a model "
+                                 f"of D={self.feature_dim}, K={self.latent_dim}")
+        self.eta_i = torch.as_tensor(state['eta_i'], dtype=torch.float64).reshape(1, -1)
+        self.xi_u_global = float(state.get('xi_u_global', 1.0))
+        self._restore_training(tr)
+        return tr.get('fit')
 
     def reconstitute(self, state):
         """poisson.py:711-717: re-create distributions, then assign the saved tensors in order."""
@@ -786,13 +937,18 @@ class PoissonFactorization:
 
     @classmethod
     def load(cls, filename, device=None):
-        with open(filename, 'rb') as f:
-            try:
-                import dill as _pk          # (custom encoder / decoder callables are dill pickles)
-            except ImportError:             # pragma: no cover
-                _pk = pickle
-            state = _pk.load(f)
-        m = cls(device=device, **state['hyper'])
+        """A model from a save() file, or -- from a save_checkpoint() file -- one that continues training exactly
+        where the saved model stood (parameters, Adam moments and step, Philox counters, column ranking)."""
+        state = _read_state(filename)
+        tr = state.get('training')
+        extra = {}
+        if tr is not None:
+            if int(tr['model']) != cls._model_id:
+                raise _abi.SpmfError(f"checkpoint of model {tr['model']} cannot be loaded as {cls.__name__}")
+            extra = dict(hot_density=tr['hot_density'], exact_guard=tr['exact_guard'])
+        m = cls(device=device, **state['hyper'], **extra)
         m.reconstitute(state)
+        if tr is not None:
+            m._restore_training(tr)
         m.set_calibration_expectations()
         return m
