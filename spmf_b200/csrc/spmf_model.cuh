@@ -231,7 +231,7 @@ template <int KK>
 struct LaneState {
   NParam u[KK], v[KK];
   GParam ue[KK], ua[KK];
-  GParam ut[KK];   // u_tau[k] (replicated per lane, accumulators unused here)
+  float utb[KK];   // softplus(scale_raw) of u_tau[k]: read by the host form of lane_step only
   float ck[KK];    // symmetry_breaking_decay^k (poisson.py:225-226)
 };
 struct FeatState {
@@ -261,10 +261,7 @@ SPMF_HD void lane_init(LaneState<KK>& st, const Layout& L, const float* P, int d
       st.v[i] = nparam_init(P[L.toff[V_LOC] + e], P[L.toff[V_RHO] + e]);
       st.ue[i] = gparam_init(P[L.toff[UETA_C] + e], P[L.toff[UETA_B] + e]);
       st.ua[i] = gparam_init(P[L.toff[UETAA_C] + e], P[L.toff[UETAA_B] + e]);
-      // u_tau[k] enters the (d,k) program through its draw y = softplus(beta / g) only: beta is all it needs
-      // (its own gradient / log q terms are backward_lat_kernel's) -- no lgamma / digamma per (d,k)
-      st.ut[i].beta = softplusf(P[L.toff[UTAU_B] + k]);
-      st.ut[i].alpha = 0.f; st.ut[i].psi = 0.f; st.ut[i].c0 = 0.f; st.ut[i].acc_da = 0.f; st.ut[i].acc_db = 0.f;
+      st.utb[i] = softplusf(P[L.toff[UTAU_B] + k]);
     }
   }
 }
@@ -311,14 +308,23 @@ SPMF_HD void lane_operands(const LaneState<KK>& st, const Layout& L, const float
   if (v_out) *v_out = v.y;
 }
 
+// u_tau[k] enters the (d,k) programs through its draw y = softplus(beta_k / g_sk) only, a function of
+// (s,k): the kernels evaluate it once per step into an [S][K] table (utau_table_kernel) instead of once
+// per (d,k,s).  beta = softplus(scale_raw[k]).
+SPMF_HD float utau_y(float beta, float g) { return softplus4(beta * SPMF_RCPF(g)).y; }
+
 // Upstream gradients of the data term for one (d,k,s)
 struct DkUp { float GAp, GEV; };   // dL/dA'_dk (sum over rows), dL/dEV_dk (closed form already applied)
-struct DkOut { float da; float dutau; float parts[5]; };  // parts: U, V, UETA, UETAA, LOGQ
+// parts: U, V, UETA, UETAA, LOGQ; uy, usg, vsg: the u draw, sigmoid'(u) and sigmoid'(v) of this (d,k,s),
+// which the split backward stores for its data half
+struct DkOut { float da; float dutau; float parts[5]; float uy, usg, vsg; };
 
+// One (d,k,s) of the (d,k) program.  eta_dec = eta[d], ieta = 1 / eta[D + d] (the encoder divisor) and
+// ut_y = utau_y of (s,k) are per-feature / per-draw values the caller holds.
 template <int KK>
 SPMF_HD DkOut lane_step(LaneState<KK>& st, const Layout& L, const Hyper& h, const float* N,
-                        const float* G, const float* eta, int d, int lane, int i, int s, float a_d,
-                        DkUp up) {
+                        const float* G, float eta_dec, float ieta, int d, int lane, int i, int s, float a_d,
+                        float ut_y, DkUp up) {
   DkOut o;
   int k = lane + 32 * i;
   const long long DK = (long long)L.D * L.K;
@@ -328,20 +334,18 @@ SPMF_HD DkOut lane_step(LaneState<KK>& st, const Layout& L, const Hyper& h, cons
   NDraw v = ndraw_sel(st.v[i], eps_v, h.vw_identity);
   GDraw ue = gdraw(st.ue[i], N[L.noff[VAR_UETA] + e]);
   GDraw ua = gdraw(st.ua[i], N[L.noff[VAR_UETAA] + e]);
-  GDraw ut = gdraw(st.ut[i], N[L.noff[VAR_UTAU] + (long long)s * L.K + k]);
   const float ck = st.ck[i];
-  float sigma = ue.y * ut.y * ck;
+  float sigma = ue.y * ut_y * ck;
   float du, dsig, dv, dtmp, due, dua, dua2;
   float pu = halfnormal(u.y, sigma, &du, &dsig);                 // poisson.py:247-251
   float pv = h.vw_identity ? normal0(v.y, 0.1f, &dv)             // bernoulli.py:200-208
                            : halfnormal(v.y, 0.1f, &dv, &dtmp);  // poisson.py:229-235
   float pue = sqrt_ig_half(ue.y, ua.y, &due, &dua);              // poisson.py:303-311
   float pua = ig_half(ua.y, 1.0f, &dua2);                        // poisson.py:312-322
-  float ieta = 1.f / eta[L.D + d];
   const float wpr = h.w_prior * h.rep_scale, wer = h.w_entropy * h.rep_scale;
   float Gy_u = -(wpr * du + up.GAp * a_d * ieta);
-  float Gy_v = -(wpr * dv + eta[d] * up.GEV);
-  float Gy_ue = -h.w_prior * (dsig * ut.y * ck + due);
+  float Gy_v = -(wpr * dv + eta_dec * up.GEV);
+  float Gy_ue = -h.w_prior * (dsig * ut_y * ck + due);
   float Gy_ua = -h.w_prior * (dua + dua2);
   nparam_bwd(st.u[i], u, eps_u, Gy_u, wer);
   nparam_bwd(st.v[i], v, eps_v, Gy_v, wer);
@@ -352,7 +356,18 @@ SPMF_HD DkOut lane_step(LaneState<KK>& st, const Layout& L, const Hyper& h, cons
   o.parts[0] = pu; o.parts[1] = pv; o.parts[2] = pue; o.parts[3] = pua;
   o.parts[4] = nlogq(st.u[i], u, eps_u) + nlogq(st.v[i], v, eps_v) + glogq(st.ue[i], ue) +
                glogq(st.ua[i], ua);
+  o.uy = u.y; o.usg = u.sg; o.vsg = v.sg;
   return o;
+}
+
+// Host form (tests/hostcheck): draws u_tau from the lane state and reads eta itself.
+template <int KK>
+SPMF_HD DkOut lane_step(LaneState<KK>& st, const Layout& L, const Hyper& h, const float* N,
+                        const float* G, const float* eta, int d, int lane, int i, int s, float a_d,
+                        DkUp up) {
+  const int k = lane + 32 * i;
+  const float ut_y = utau_y(st.utb[i], N[L.noff[VAR_UTAU] + (long long)s * L.K + k]);
+  return lane_step<KK>(st, L, h, N, G, eta[d], 1.f / eta[L.D + d], d, lane, i, s, a_d, ut_y, up);
 }
 
 // per-feature step (lane 0): w, s, s_eta, s_tau, s_eta_a, s_tau_a.  da = sum_k GAp u / eta (reduced),

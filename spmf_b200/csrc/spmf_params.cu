@@ -59,15 +59,30 @@ __global__ void fill_normal_kernel(Layout L, float* __restrict__ noise, uint32_t
 // The continued-fraction regime of the gradient (draws well above alpha, ~20 % of them) is not evaluated
 // in place -- that would run its long loop once per draw slot with a fifth of the lanes active -- but
 // queued in shared memory and worked off by the whole CTA with (nearly) full warps.
+// The grid is the concatenation of each variable's ceil(vsize / 128) CTAs (gamma_grid_blocks): the
+// variables range from K to D*K elements, and a grid of 8 x the largest left ~70 % of the CTAs with
+// nothing to do.
+static unsigned gamma_grid_blocks(const Layout& L) {
+  long long nb = 0;
+  for (int v = VAR_UETA; v < NUM_VARS; ++v) nb += (L.vsize[v] + 127) / 128;
+  return (unsigned)nb;
+}
+
 __global__ void __launch_bounds__(128)
 gamma_kernel(Layout L, const float* __restrict__ P, float* __restrict__ N, float* __restrict__ G,
              int draw, int grad, uint32_t step, uint32_t k0, uint32_t k1, const StepState* __restrict__ sst) {
   if (sst) step = sst->rng_step;
   __shared__ float4 cfq[128 * 4];              // (alpha, digamma(alpha), draw, slot = draw index * 128 + thread)
   __shared__ int cfn;
-  const int v = VAR_UETA + blockIdx.y;
+  int v = VAR_UETA;
+  long long blk = blockIdx.x;
+  for (; v < NUM_VARS - 1; ++v) {
+    const long long nb = (L.vsize[v] + 127) / 128;
+    if (blk < nb) break;
+    blk -= nb;
+  }
   const long long nelem = L.vsize[v];
-  const long long e0 = (long long)blockIdx.x * blockDim.x;
+  const long long e0 = blk * blockDim.x;
   const long long e = e0 + threadIdx.x;
   const bool live = e < nelem;
   if (threadIdx.x == 0) cfn = 0;
@@ -78,6 +93,7 @@ gamma_kernel(Layout L, const float* __restrict__ P, float* __restrict__ N, float
   float* Gv = G + L.noff[v];
   for (int s0 = 0; s0 < L.S; s0 += 4) {
     const int ns = L.S - s0 < 4 ? L.S - s0 : 4;
+    bool queued = false;
     if (live) {
       float g[4] = {1.f, 1.f, 1.f, 1.f}, o[4];
 #pragma unroll
@@ -96,6 +112,7 @@ gamma_kernel(Layout L, const float* __restrict__ P, float* __restrict__ N, float
       }
       if (grad) {
         const unsigned cf = gamma_der_series4(alpha, psi, g, ns, o);
+        queued = cf != 0u;
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           if (j < ns) {
@@ -108,17 +125,19 @@ gamma_kernel(Layout L, const float* __restrict__ P, float* __restrict__ N, float
         }
       }
     }
-    if (grad) {
-      __syncthreads();
+    // the queue is worked off (and emptied for the next group of draws) only when some lane filled it
+    if (grad && __syncthreads_or(queued)) {
       const int nq = cfn;
       for (int t = threadIdx.x; t < nq; t += blockDim.x) {
         const float4 q = cfq[t];
         const int slot = __float_as_int(q.w);
         Gv[(long long)(s0 + (slot >> 7)) * nelem + e0 + (slot & 127)] = gamma_der_cf(q.x, q.y, q.z);
       }
-      __syncthreads();
-      if (threadIdx.x == 0) cfn = 0;
-      __syncthreads();
+      if (s0 + 4 < L.S) {
+        __syncthreads();
+        if (threadIdx.x == 0) cfn = 0;
+        __syncthreads();
+      }
     }
   }
 }
@@ -222,6 +241,20 @@ __global__ void sample_kernel(Layout L, const float* __restrict__ P, const float
   }
 }
 
+// ------------------------------------------------------------------ u_tau draws, per (s,k)
+// utab[s][k] = utau_y (spmf_model.cuh): the one value of u_tau the (d,k) programs read, evaluated once
+// per step here rather than D times per (s,k) inside them.
+__global__ void utau_table_kernel(Layout L, const float* __restrict__ P, const float* __restrict__ N,
+                                  float* __restrict__ utab) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= L.S * L.K) return;
+  utab[i] = utau_y(softplusf(P[L.toff[UTAU_B] + i % L.K]), N[L.noff[VAR_UTAU] + i]);
+}
+
+static void launch_utau_table(const Layout& L, const float* P, const float* N, float* utab, cudaStream_t st) {
+  utau_table_kernel<<<(L.S * L.K + 127) / 128, 128, 0, st>>>(L, P, N, utab);
+}
+
 // ------------------------------------------------------------------ backward, (d,k)-shaped tensors
 // One warp per feature d, lanes over k: u, v, u_eta, u_eta_a.  Emits da[s][d] = sum_k GA' u / eta
 // (needed by the per-feature kernel), the per-(s,d,k) contribution to d prior_u / d u_tau, and
@@ -240,8 +273,9 @@ __global__ void sample_kernel(Layout L, const float* __restrict__ P, const float
       const float *__restrict__ eta, const int *__restrict__ rank, int SV, int KP,                       \
       const float *__restrict__ GAp, const float *__restrict__ GEVnz, const double *__restrict__ zcolsum, \
       float *__restrict__ grads, float *__restrict__ scr_utau, float *__restrict__ scr_parts,            \
-      float *__restrict__ scr_da, float *__restrict__ fac, const int *__restrict__ gflag
-#define SPMF_DK_ARGS L, h, P, N, G, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, fac, gflag
+      float *__restrict__ scr_da, float *__restrict__ fac, const float *__restrict__ utab,               \
+      const int *__restrict__ gflag
+#define SPMF_DK_ARGS L, h, P, N, G, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, fac, utab, gflag
 
 template <int KK, bool PRE>
 __device__ __forceinline__ void backward_dk_body(SPMF_DK_PARAMS, int k0, bool first) {
@@ -254,6 +288,7 @@ __device__ __forceinline__ void backward_dk_body(SPMF_DK_PARAMS, int k0, bool fi
   lane_init<KK>(st, L, P, d, lane, h.decay);
   const NParam s0 = nparam_init(P[L.toff[S_LOC] + d], P[L.toff[S_RHO] + d]);
   const NParam s1 = nparam_init(P[L.toff[S_LOC] + L.D + d], P[L.toff[S_RHO] + L.D + d]);
+  const float eta_dec = eta[d], ieta = 1.f / eta[L.D + d];   // decoder scale, 1 / encoder divisor
   const RecMap rmap = rec_map(KP);                 // rec_pos(sv, k) = rec_pos(0, k) + sv * RG * VW
   const int sv_stride = rmap.RG * rmap.VW;
   int pos0[KK];
@@ -294,16 +329,13 @@ __device__ __forceinline__ void backward_dk_body(SPMF_DK_PARAMS, int k0, bool fi
           up.GAp = GAp[idx];
           up.GEV = GEVnz[idx] - (dense ? 0.f : (float)zcolsum[(long long)q * SV * KP + rp]);
         }
-        DkOut o = lane_step<KK>(st, L, h, N, G, eta, d, lane, i, s, a_d, up);
+        DkOut o = lane_step<KK>(st, L, h, N, G, eta_dec, ieta, d, lane, i, s, a_d, __ldg(&utab[s * L.K + k]), up);
         if constexpr (PRE) {
           const long long e = ((long long)s * L.D + d) * L.K + k;
           const long long nsdk = (long long)L.S * L.D * L.K;
-          const NDraw ud = ndraw(st.u[i], N[L.noff[VAR_U] + e]);
-          const NDraw vd = ndraw_sel(st.v[i], N[L.noff[VAR_V] + e], h.vw_identity);
-          const float ieta = 1.f / eta[L.D + d];       // encoder divisor
-          fac[e] = a_d * ieta * ud.sg;
-          fac[nsdk + e] = eta[d] * vd.sg;
-          fac[2 * nsdk + e] = ud.y * ieta;
+          fac[e] = a_d * ieta * o.usg;
+          fac[nsdk + e] = eta_dec * o.vsg;
+          fac[2 * nsdk + e] = o.uy * ieta;
         }
         da += o.da;
         scr_utau[((long long)s * L.D + d) * L.K + k] = o.dutau;
@@ -850,9 +882,7 @@ int spmf_fill_noise_dev(float* noise, const float* params, int D, int K, int S, 
     fill_normal_kernel<<<grid, 256, 0, st>>>(L, noise, step, k0, k1, sst);
   }
   if (which & SPMF_NOISE_GAMMA) {
-    long long emax = (long long)D * K > 2LL * D ? (long long)D * K : 2LL * D;
-    dim3 grid((unsigned)((emax + 127) / 128), NUM_VARS - VAR_UETA);
-    gamma_kernel<<<grid, 128, 0, st>>>(L, params, noise, noise, 1, 0, step, k0, k1, sst);
+    gamma_kernel<<<gamma_grid_blocks(L), 128, 0, st>>>(L, params, noise, noise, 1, 0, step, k0, k1, sst);
   }
   SPMF_CHECK_LAUNCH();
   return SPMF_OK;
@@ -922,9 +952,7 @@ int spmf_gamma_grad(const float* params, const float* noise, int D, int K, int S
                     void* stream) {
   if (!params || !noise || !dgda || D <= 0 || K <= 0 || S <= 0 || K > SPMF_MAX_K) return SPMF_ERR_BAD_ARG;
   Layout L = make_layout(D, K, S);
-  long long emax = (long long)D * K > 2LL * D ? (long long)D * K : 2LL * D;
-  dim3 grid((unsigned)((emax + 127) / 128), NUM_VARS - VAR_UETA);
-  gamma_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(L, params, const_cast<float*>(noise), dgda, 0, 1, 0, 0, 0, nullptr);
+  gamma_kernel<<<gamma_grid_blocks(L), 128, 0, (cudaStream_t)stream>>>(L, params, const_cast<float*>(noise), dgda, 0, 1, 0, 0, 0, nullptr);
   SPMF_CHECK_LAUNCH();
   return SPMF_OK;
 }
@@ -939,9 +967,7 @@ int spmf_gamma_draw_grad_dev(const float* params, float* noise, float* dgda, int
                              unsigned long long seed, unsigned int step, const void* step_state, void* stream) {
   if (!params || !noise || !dgda || D <= 0 || K <= 0 || S <= 0 || K > SPMF_MAX_K) return SPMF_ERR_BAD_ARG;
   Layout L = make_layout(D, K, S);
-  long long emax = (long long)D * K > 2LL * D ? (long long)D * K : 2LL * D;
-  dim3 grid((unsigned)((emax + 127) / 128), NUM_VARS - VAR_UETA);
-  gamma_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(L, params, noise, dgda, 1, 1, step,
+  gamma_kernel<<<gamma_grid_blocks(L), 128, 0, (cudaStream_t)stream>>>(L, params, noise, dgda, 1, 1, step,
                                                       (uint32_t)(seed & 0xffffffffu), (uint32_t)(seed >> 32),
                                                       (const StepState*)step_state);
   SPMF_CHECK_LAUNCH();
@@ -984,7 +1010,8 @@ int spmf_backward_params_ranked_m(const float* params, const float* noise, const
   Layout L = make_layout(D, K, S);
   Hyper h = make_hyper(u_tau_scale, s_tau_scale, decay, w_entropy, w_prior, world_size, batch_rows, model);
   const int KP = spmf_kpad(K), SV = spmf_draw_vec_k(K, S);
-  // float scratch: scr_utau [S][D][K] | scr_parts [D][S*16] | scr_lat [K][S*16] | scr_da [S][D]
+  // float scratch: scr_utau [S][D][K] | scr_parts [D][S*16] | scr_lat [K][S*16] | scr_da [S][D] |
+  // (fac [3][S][D][K], split backward only) | utab [S][K]
   float* scr_utau = scr_f;
   float* scr_parts = scr_utau + (long long)S * D * K;
   float* scr_lat = scr_parts + (long long)D * S * NUM_PARTS;
@@ -994,11 +1021,13 @@ int spmf_backward_params_ranked_m(const float* params, const float* noise, const
   double* latparts = featparts + (long long)S * NUM_PARTS;
   double* rscr = latparts + (long long)S * NUM_PARTS;
   float* scr_da = scr_lat + (long long)K * S * NUM_PARTS;
+  float* utab = scr_da + (long long)S * D + 3LL * S * D * K;
   dim3 grid((D + 3) / 4);
-  if (KP <= 32) backward_dk_kernel<1, false><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, nullptr, (const int*)gs);
-  else if (KP <= 64) backward_dk_kernel<2, false><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, nullptr, (const int*)gs);
-  else if (KP <= 128) backward_dk_kernel<4, false><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, nullptr, (const int*)gs);
-  else if (KP <= 512) backward_dk_wide_kernel<false><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, nullptr, (const int*)gs);
+  launch_utau_table(L, params, noise, utab, st);
+  if (KP <= 32) backward_dk_kernel<1, false><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, nullptr, utab, (const int*)gs);
+  else if (KP <= 64) backward_dk_kernel<2, false><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, nullptr, utab, (const int*)gs);
+  else if (KP <= 128) backward_dk_kernel<4, false><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, nullptr, utab, (const int*)gs);
+  else if (KP <= 512) backward_dk_wide_kernel<false><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, KP, GAp, GEVnz, zcolsum, grads, scr_utau, scr_parts, scr_da, nullptr, utab, (const int*)gs);
   else return SPMF_ERR_UNSUPPORTED;
   backward_feat_kernel<<<(int)(((long long)D * SV + 127) / 128), 128, 0, st>>>(L, h, params, noise, dgda, eta, rank, SV, Gphinz, scr_da, grads, scr_parts, 0, (const int*)gs);
   SPMF_CHECK_LAUNCH();
@@ -1017,8 +1046,9 @@ int spmf_backward_params_ranked_m(const float* params, const float* noise, const
 }
 
 long long spmf_backward_scratch_floats(int D, int K, int S) {
-  // scr_utau | scr_parts | scr_lat | scr_da | fac (3 factors per (s,d,k), split backward only)
-  return 4LL * S * D * K + (long long)D * S * NUM_PARTS + (long long)K * S * NUM_PARTS + (long long)S * D;
+  // scr_utau | scr_parts | scr_lat | scr_da | fac (3 factors per (s,d,k), split backward only) | utab
+  return 4LL * S * D * K + (long long)D * S * NUM_PARTS + (long long)K * S * NUM_PARTS + (long long)S * D +
+         (long long)S * K;
 }
 
 /* Split backward: spmf_backward_pre = everything that does not depend on the data term (runs under it on
@@ -1045,15 +1075,17 @@ int spmf_backward_pre_m(const float* params, const float* noise, const float* dg
   float* scr_lat = scr_parts + (long long)D * S * NUM_PARTS;
   float* scr_da = scr_lat + (long long)K * S * NUM_PARTS;
   float* fac = scr_da + (long long)S * D;
+  float* utab = fac + 3LL * S * D * K;
   double* dutau = scr_d;
   double* featparts = dutau + (long long)S * K;
   double* latparts = featparts + (long long)S * NUM_PARTS;
   double* rscr = latparts + (long long)S * NUM_PARTS;
   dim3 grid((D + 3) / 4);
-  if (KP <= 32) backward_dk_kernel<1, true><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, KP, nullptr, nullptr, nullptr, grads, scr_utau, scr_parts, scr_da, fac, nullptr);
-  else if (KP <= 64) backward_dk_kernel<2, true><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, KP, nullptr, nullptr, nullptr, grads, scr_utau, scr_parts, scr_da, fac, nullptr);
-  else if (KP <= 128) backward_dk_kernel<4, true><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, KP, nullptr, nullptr, nullptr, grads, scr_utau, scr_parts, scr_da, fac, nullptr);
-  else if (KP <= 512) backward_dk_wide_kernel<true><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, KP, nullptr, nullptr, nullptr, grads, scr_utau, scr_parts, scr_da, fac, nullptr);
+  launch_utau_table(L, params, noise, utab, st);
+  if (KP <= 32) backward_dk_kernel<1, true><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, KP, nullptr, nullptr, nullptr, grads, scr_utau, scr_parts, scr_da, fac, utab, nullptr);
+  else if (KP <= 64) backward_dk_kernel<2, true><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, KP, nullptr, nullptr, nullptr, grads, scr_utau, scr_parts, scr_da, fac, utab, nullptr);
+  else if (KP <= 128) backward_dk_kernel<4, true><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, KP, nullptr, nullptr, nullptr, grads, scr_utau, scr_parts, scr_da, fac, utab, nullptr);
+  else if (KP <= 512) backward_dk_wide_kernel<true><<<grid, 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, KP, nullptr, nullptr, nullptr, grads, scr_utau, scr_parts, scr_da, fac, utab, nullptr);
   else return SPMF_ERR_UNSUPPORTED;
   backward_feat_kernel<<<(int)(((long long)D * SV + 127) / 128), 128, 0, st>>>(L, h, params, noise, dgda, eta, nullptr, SV, nullptr, nullptr, grads, scr_parts, 1, nullptr);
   SPMF_CHECK_LAUNCH();
