@@ -151,6 +151,8 @@ int spmf_unpack_adam(float* comm_slack, int slack_floats, int S, float w_entropy
                      double* loss_out, const float* grads, long long n_data, const spmf_adam_args* adam,
                      void* stream);
 int spmf_colsum(const float* in, long long n, int c, int q, double* out, double* scratch, void* stream);
+/* the same over fp64 input: out[q][c] = sum over rows of in[q][n][c] in a fixed order; scratch: 64*q*c doubles */
+int spmf_colsum_f64(const double* in, long long n, int c, int q, double* out, double* scratch, void* stream);
 
 /* ---- multi-GPU tail over NVLink peer memory (net-new, SURVEY.md 8e; replaces ncclAllReduce -> spmf_unpack_adam) ----
  * One process per GPU.  Gradient, parameter and flag buffers come from spmf_p2p_alloc (cudaMalloc, zeroed) and
@@ -534,6 +536,33 @@ int spmf_guard_rows_fix_dense(const void* raw, int raw_dtype, const int* rank, c
                               void* stream);
 int spmf_guard_cols_fix(int nrows, int D, int K, int S, const float* EV, const float* PH, const float* z,
                         float* GEV, float* Gph, const float* xd, void* gs, void* stream);
+
+/* ---- posterior predictive check (csrc/spmf_ppc.cu) ----
+ * One pass over every (draw, row, feature) entry of a batch: the rate of the entry as the data term forms it
+ * (any link; xd, z, EV, PH as for spmf_dense_rows, z from spmf_csr_encode / spmf_dense_encode), a replicate
+ * x_rep ~ Poisson(rate) or Bernoulli(sigmoid(rate)) drawn from the Philox stream keyed by (seed, draw s,
+ * global row = row_offset + local row, feature d) -- independent of the batch split, the launch geometry and the
+ * training streams -- and its statistics:
+ *   row_total[S][nrows] (sum_d x_rep), row_nnz[S][nrows], row_disc[S][nrows][2] = (D(x_rep), D(x)) in fp64
+ *   summed in feature order, D = sum_d (y - rate)^2 / rate (Poisson) or (y - p)^2 / (p (1 - p)) (Bernoulli);
+ *   disc_sum[S][2] = the sums of row_disc over the rows (fixed order; scratch: 128*S doubles);
+ *   accumulated (zeroed by the caller): col_total / col_sumsq [S][D] (uint64), col_nnz [S][D] (uint32) by
+ *   integer atomics, draw_max[S] (largest replicate) and draw_invalid[S] (entries whose Poisson rate is negative,
+ *   not finite or above 2^24, or whose logit is not finite: replicate 0, left out of both discrepancies);
+ *   out[S][nrows][D] (int32, may be NULL) = the replicates themselves.
+ * Every output is bit-identical from run to run.  1 <= S <= SPMF_PPC_MAX_S, row_offset + nrows <= SPMF_PPC_MAX_ROW. */
+#define SPMF_PPC_MAX_S 65535
+#define SPMF_PPC_MAX_ROW (1LL << 48)
+int spmf_ppc_rows(const float* xd, int nrows, int D, int K, int S, int link, const float* EV, const float* PH,
+                  const float* z, unsigned long long seed, long long row_offset, long long* row_total, int* row_nnz,
+                  double* row_disc, unsigned long long* col_total, unsigned long long* col_sumsq,
+                  unsigned int* col_nnz, unsigned int* draw_max, unsigned long long* draw_invalid, int* out,
+                  double* disc_sum, double* scratch, void* stream);
+/* observed statistics of a CSR batch (column ids = features): row_total[nrows], row_nnz[nrows] written;
+ * col_total[D], col_sumsq[D] (fp64, exact for integer counts) and col_nnz[D] accumulated (caller zeroes) */
+int spmf_ppc_observed(const long long* rowptr, const int* cols, const float* vals, int nrows, int D,
+                      double* row_total, int* row_nnz, double* col_total, double* col_sumsq, unsigned int* col_nnz,
+                      void* stream);
 
 const char* spmf_version(void);
 

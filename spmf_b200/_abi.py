@@ -16,6 +16,7 @@ NUM_VARS = 12
 NUM_PARTS = 16
 MAX_K = 512        # latent dimensions of the gather / dense kernels (SPMF_MAX_K)
 MAX_TILE_K = 128   # latent dimensions of the tensor-core hybrid path (SPMF_MAX_TILE_K)
+PPC_MAX_S = 65535  # draws of one posterior predictive check (SPMF_PPC_MAX_S)
 
 
 class SpmfError(RuntimeError):
@@ -67,6 +68,7 @@ _SIGS = {
     "spmf_unpack_parts": (i32, [p, i32, i32, f32, f32, p, p, p]),
     "spmf_sumsq": (i32, [p, i64, p, p, p, p]),
     "spmf_colsum": (i32, [p, i64, i32, i32, p, p, p]),
+    "spmf_colsum_f64": (i32, [p, i64, i32, i32, p, p, p]),
     "spmf_csr_colstats": (i32, [p, p, i64, i32, p, p, p]),
     "spmf_csc_scratch_ints": (i64, [i32]),
     "spmf_csr_to_csc": (i32, [p, p, p, i32, i32, p, p, p, p, p]),
@@ -112,6 +114,9 @@ _SIGS = {
     "spmf_zero_col_grads": (i32, [p, p, p, i32, i32, i32, p]),
     "spmf_csc_cols_accum": (i32, [p, p, p, i32, i32, i32, i32, i32, p, p, p, p, p, p, p, p]),
     "spmf_csr_to_csc_part": (i32, [p, p, i32, p, p, i32, i32, p, p, p, p, p]),
+    # posterior predictive check (spmf_ppc.cu)
+    "spmf_ppc_rows": (i32, [p, i32, i32, i32, i32, i32, p, p, p, u64, i64, p, p, p, p, p, p, p, p, p, p, p, p]),
+    "spmf_ppc_observed": (i32, [p, p, p, i32, i32, p, p, p, p, p, p]),
 }
 
 

@@ -284,4 +284,103 @@ SPMF_HD float gamma_draw(float alpha, uint32_t elem_lo, uint32_t elem_hi, uint32
   return fmaxf(g, 1.17549435e-38f);
 }
 
+// ---------------------------------------------------------------------------
+// Poisson and Bernoulli draws of the posterior predictive replicates (csrc/spmf_ppc.cu).  Pure functions
+// of the parameter, a Philox key and a counter: the i-th Philox call of a draw uses `ctr` with ctr.w + i.
+// ---------------------------------------------------------------------------
+struct Key2 { uint32_t k0, k1; };
+
+constexpr float kPoissonInvMax = 10.f;        // inversion below this rate, PTRS from it on
+constexpr int kPoissonInvCap = 64;            // inversion search stops at this count
+constexpr int kPoissonPtrsCalls = 8;          // Philox calls of one PTRS draw: 2 candidates each
+// Largest valid Poisson rate: keeps every replicate an exact int32 and the per-column sums of squares
+// of a batch well inside 64 bits.
+constexpr float kPoissonMaxRate = 16777216.f;  // 2^24
+
+SPMF_HD bool poisson_rate_ok(float lam) { return lam >= 0.f && lam <= kPoissonMaxRate; }   // false for NaN
+
+// Sequential-search inversion of the CDF at u in (0,1].  The search stops where the next pmf term no
+// longer changes F in fp32 (or at kPoissonInvCap): the tail mass beyond that point -- a few times 2^-24,
+// the resolution of u01 -- lands on the count reached there.
+SPMF_HD int poisson_inversion(float lam, float u) {
+  float p = expf(-lam), F = p;
+  int k = 0;
+  while (u > F && k < kPoissonInvCap) {
+    ++k;
+    p *= lam / (float)k;
+    const float Fn = F + p;
+    if (Fn == F) break;
+    F = Fn;
+  }
+  return k;
+}
+
+// log k! in double for integer k >= 0 (numpy's random_loggam: Stirling series from 7 on, the recurrence below)
+SPMF_HD double log_factorial(double k) {
+  double x = k + 1.0, shift = 0.0;
+  if (x <= 2.0) return 0.0;
+  while (x < 7.0) {
+    shift += log(x);
+    x += 1.0;
+  }
+  const double x2 = 1.0 / (x * x);
+  const double g = 8.333333333333333e-02 + x2 * (-2.777777777777778e-03 + x2 * (7.936507936507937e-04 +
+                   x2 * (-5.952380952380952e-04 + x2 * (8.417508417508418e-04 + x2 * (-1.917526917526918e-03 +
+                   x2 * (6.410256410256410e-03 + x2 * (-2.955065359477124e-02 + x2 * (1.796443723688307e-01 +
+                   x2 * -1.39243221690590e+00))))))));
+  return g / x + 0.9189385332046727 + (x - 0.5) * log(x) - x - shift;
+}
+
+// Transformed rejection with squeeze (PTRS, Hoermann 1993; the method of numpy's random_poisson_ptrs)
+// for lam >= kPoissonInvMax.  The acceptance test -lam + k log lam - log k! is evaluated in double: in fp32
+// the two large terms (~1e6 at lam = 1e5) cancel to O(1) and lgammaf alone is off by about one unit.  A
+// candidate is accepted with probability above 0.9, so all 2*kPoissonPtrsCalls candidates are rejected with
+// probability below 1e-15; the draw then returns floor(lam), the mode.
+SPMF_HD int poisson_ptrs(float lam, Key2 key, U4 ctr) {
+  const float slam = sqrtf(lam);
+  const double dlam = (double)lam, dloglam = log(dlam);
+  const float b = 0.931f + 2.53f * slam;
+  const float a = -0.059f + 0.02483f * b;
+  const float log_invalpha = logf(1.1239f + 1.1328f / (b - 3.4f));
+  const float vr = 0.9277f - 3.6224f / (b - 2.f);
+  for (int call = 0; call < kPoissonPtrsCalls; ++call) {
+    U4 c = ctr;
+    c.w += (uint32_t)call;
+    const U4 r = philox4x32_10(c, key.k0, key.k1);
+    for (int h = 0; h < 2; ++h) {
+      const float U = u01(h ? r.z : r.x) - 0.5f, V = u01(h ? r.w : r.y);
+      const float us = 0.5f - fabsf(U);
+      if (us < 0.013f && V > us) continue;          // (also every us == 0, before 2a/us is formed)
+      const double k = floor((double)(2.f * a / us + b) * (double)U + dlam + 0.43);
+      if (us >= 0.07f && V <= vr) return (int)k;
+      if (k < 0.0) continue;
+      const double rhs = -dlam + k * dloglam - log_factorial(k);
+      if ((double)(logf(V) + log_invalpha - logf(a / (us * us) + b)) <= rhs) return (int)k;
+    }
+  }
+  return (int)floorf(lam);
+}
+
+// Poisson(lam) for a valid rate (poisson_rate_ok); 0 for lam == 0 and for anything invalid.
+SPMF_HD int poisson_draw(float lam, Key2 key, U4 ctr) {
+  if (!(lam > 0.f) || !(lam <= kPoissonMaxRate)) return 0;
+  if (lam < kPoissonInvMax) return poisson_inversion(lam, u01(philox4x32_10(ctr, key.k0, key.k1).x));
+  return poisson_ptrs(lam, key, ctr);
+}
+
+// Bernoulli(p): 1 iff u01 <= p, so P(1) = floor(p * 2^24) / 2^24 -- p is resolved to 2^-24 (p = 0 never
+// gives 1, p = 1 always does).
+SPMF_HD int bernoulli_draw(float p, Key2 key, U4 ctr) {
+  return u01(philox4x32_10(ctr, key.k0, key.k1).x) <= p ? 1 : 0;
+}
+
+// Replicate stream of entry (draw s, global row, feature d) under a check seed.  The seed is mixed with a
+// constant, so the key differs from the training noise key (the model seed) even for equal seeds; the
+// counter holds (d, row bits 0-31, row bits 32-47 | s << 16, call).  Needs s < 2^16 and row < 2^48.
+SPMF_HD Key2 ppc_key(uint64_t seed) { return Key2{(uint32_t)seed, (uint32_t)(seed >> 32) ^ 0x50504331u}; }
+SPMF_HD U4 ppc_counter(int s, long long row, int d) {
+  const uint64_t r = (uint64_t)row;
+  return U4{(uint32_t)d, (uint32_t)r, (uint32_t)((r >> 32) & 0xffffu) | ((uint32_t)s << 16), 0u};
+}
+
 }  // namespace spmf

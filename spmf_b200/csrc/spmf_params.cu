@@ -1247,4 +1247,9 @@ int spmf_colsum(const float* in, long long n, int c, int q, double* out, double*
   return reduce_rows<float>(in, out, scratch, n, c, q, (cudaStream_t)stream);
 }
 
+int spmf_colsum_f64(const double* in, long long n, int c, int q, double* out, double* scratch, void* stream) {
+  if (!in || !out || !scratch) return SPMF_ERR_BAD_ARG;
+  return reduce_rows<double>(in, out, scratch, n, c, q, (cudaStream_t)stream);
+}
+
 }  // extern "C"

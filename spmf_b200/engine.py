@@ -82,6 +82,8 @@ class StepWorkspace:
         return False
 
     def ensure_rows(self, nrows):
+        """Grow the per-row buffers to `nrows` rows; True if they moved.  Callers outside __init__ go through
+        AdviEngine.ensure_rows, which also invalidates what points into the old buffers."""
         if nrows <= self.max_rows:
             return False
         C = self.KP * self.SV
@@ -89,6 +91,7 @@ class StepWorkspace:
         self.z = torch.empty(self.NQ * nrows * C, dtype=torch.float32, device=self.device)
         self.dzr = torch.empty(self.NQ * nrows * C, dtype=torch.float32, device=self.device)
         self.rowacc = torch.empty(self.NQ * nrows * 4 * self.SV, dtype=torch.float32, device=self.device)
+        return True
 
 
 class AdviEngine:
@@ -192,13 +195,31 @@ class AdviEngine:
         _abi.call("spmf_guard_decode", C.cast(buf, C.c_void_p), C.byref(flag), C.byref(nbad), C.byref(mv))
         return flag.value, nbad.value, mv.value
 
+    def _workspace_moved(self):
+        """A workspace buffer was reallocated: the cached step arguments and every captured step graph point into
+        the old one (the generation is part of the graph cache key)."""
+        self._args = None
+        self._ws_gen += 1
+
+    def ensure_rows(self, nrows):
+        """Per-row workspace (z, dzr, rowacc) for batches of `nrows` rows.  Every user of the workspace grows
+        it here -- the step, and the evaluation paths (encode, data_term, row_log_likelihood, the predictive
+        check) -- so that a later graph replay never reads freed buffers."""
+        if self.ws.ensure_rows(nrows):
+            self._workspace_moved()
+
+    def dense_scratch(self, nrows):
+        """fp32 [nrows][D] scratch of the dense kernels (grown like ensure_rows)."""
+        w = self.ws
+        if w.ensure_dense(max(int(nrows), w.max_rows)):
+            self._workspace_moved()
+        return w.xdense
+
     def _guard_scratch(self, nrows):
         """Dense scratch pointer for the exact guard / dense links, or None (guard degrades to drop-and-count)."""
-        w = self.ws
         if self.link == 0 and (not self.exact_guard or 4 * int(nrows) * self.D > self.GUARD_SCRATCH_LIMIT):
             return None
-        w.ensure_dense(max(int(nrows), w.max_rows))
-        return w.xdense
+        return self.dense_scratch(nrows)
 
     def fill_noise(self, step=None, which=3, advance=True):
         """Philox draws for `step`: N(0,1) for v,w,u,s (which&1), Gamma(alpha,1) for the rest (which&2)."""
@@ -221,7 +242,7 @@ class AdviEngine:
         path: unormalized_log_prob_parts; the training step issues the same sequence natively), including
         the exact non-finite guard / the dense links."""
         w = self.ws
-        w.ensure_rows(b.nrows)
+        self.ensure_rows(b.nrows)
         st = _stream()
         self.reset_guard()
         xd = self._guard_scratch(b.nrows)
@@ -385,7 +406,7 @@ class AdviEngine:
         if self.world_size > 1:
             raise _abi.SpmfError("custom encoder / decoder callables are single-GPU only")
         w = self.ws
-        w.ensure_rows(batch.nrows)
+        self.ensure_rows(batch.nrows)
         xd = self._guard_scratch(batch.nrows)
         if fresh_noise:
             self.fill_noise()
@@ -494,16 +515,12 @@ class AdviEngine:
         if self.custom_link is not None:
             return self._step_custom(batch, fresh_noise, lr, clip_value, beta1, beta2, eps)
         w = self.ws
-        if batch.nrows > w.max_rows:
-            w.ensure_rows(batch.nrows)
-            self._args = None
-            self._ws_gen += 1
+        self.ensure_rows(batch.nrows)
         hybrid = self._runs_hybrid(batch)
         if hybrid:
             h = batch.ensure_hot(self.rank, self.hot_cols, version=getattr(self, "rank_version", 0))
             if w.ensure_hybrid(self.hot_cols, batch.nrows):
-                self._args = None
-                self._ws_gen += 1
+                self._workspace_moved()
         else:
             if batch.dense_raw is not None:
                 raise _abi.SpmfError("this batch was ingested dense for the tile-hybrid step, but the engine for "
@@ -513,10 +530,7 @@ class AdviEngine:
                                      f"for S={self.S} runs the gather step; upload it without a hot split")
             if self.link == 0:
                 batch.ensure_csc()
-        xd_before = getattr(w, "xdense", None)
         xd = self._guard_scratch(batch.nrows)
-        if xd is not xd_before:
-            self._ws_gen += 1
         a = self._step_args()
         a.step_state = _ptr(self.step_state)
         a.link, a.gs, a.xdense, a.xdense_in = self.link, _ptr(self.gs), _ptr(xd), None

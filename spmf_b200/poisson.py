@@ -63,6 +63,33 @@ def waic_terms(ll):
     return lppd, pwaic
 
 
+PPC_SAMPLE_LIMIT = 1 << 30      # replicates posterior_predictive_sample materialises at most (4 GiB of int32)
+PPC_INTEGER_STATS = ('row_total', 'row_nnz', 'col_total', 'col_sumsq', 'col_nnz', 'total', 'nnz', 'max')
+
+
+def ppc_p_values(observed, replicated):
+    """Posterior predictive p-values from the statistics of posterior_predictive_check.
+
+    Every statistic T uses the mid-p  (#{s: T_rep_s > T_obs} + 0.5 #{s: T_rep_s == T_obs}) / S,  elementwise over
+    rows / columns.  The discrepancy is paired per draw: D(x_rep_s, theta_s) against D(x, theta_s).  'col_var' is
+    the per-column sample variance over the N rows, (sumsq - total^2 / N) / (N - 1), computed in fp64 from the
+    exact integer sums on both sides."""
+    S = replicated['discrepancy'].shape[0]
+
+    def mid_p(rep, obs):
+        rep, obs = rep.to(torch.float64), obs.to(torch.float64)
+        return ((rep > obs).sum(0, dtype=torch.float64) + 0.5 * (rep == obs).sum(0, dtype=torch.float64)) / S
+
+    def col_var(t):
+        n = float(observed['row_total'].shape[-1])
+        tot, sq = t['col_total'].to(torch.float64), t['col_sumsq'].to(torch.float64)
+        return (sq - tot * tot / n) / max(n - 1.0, 1.0)
+
+    out = {k: mid_p(replicated[k], observed[k]) for k in PPC_INTEGER_STATS + ('discrepancy',)}
+    out['col_var'] = mid_p(col_var(replicated), col_var(observed))
+    return out
+
+
 class _SurrogateDistribution:
     """Stand-in for `self.surrogate_distribution` (a tfd.JointDistributionNamed in the reference,
     poisson.py:567-569): `.sample(n)` returns a dict of reference-shaped draws."""
@@ -442,7 +469,7 @@ class PoissonFactorization:
         S = u.shape[0] if batched else 1
         eng = self._engine_for(S)
         b = as_device_batch(x, self.device, self.feature_dim)
-        eng.ws.ensure_rows(b.nrows)
+        eng.ensure_rows(b.nrows)
         D, K = self.feature_dim, self.latent_dim
         zeros_v = torch.zeros((S, K, D) if batched else (K, D), device=self.device)
         zeros_w = torch.zeros((S, 1, D) if batched else (1, D), device=self.device)
@@ -581,8 +608,8 @@ class PoissonFactorization:
         b = c if isinstance(c, DeviceBatch) else as_device_batch(c, self.device, self.feature_dim)
         if b.cols is None:
             raise ValueError("row_log_likelihood needs a batch with its CSR arrays (not a hybrid-only upload)")
+        eng.ensure_rows(b.nrows)
         ws = eng.ws
-        ws.ensure_rows(b.nrows)
         self._operands_from_theta(eng, params['u'], params['v'], params['w'], params['s'])
         if self._custom_link:
             eng.reset_guard()
@@ -608,16 +635,8 @@ class PoissonFactorization:
         (lppd_i - pwaic_i), se = 2 sqrt(n var_i(lppd_i - pwaic_i)).  Returns the reference's dict
         {'waic', 'se', 'lppd', 'pwaic'}.  `data`: a batch factory as for fit(), a CsrShard, or one
         batch / array; default: the factory last given to fit() / compute_scales()."""
-        data = self._last_data_factory if data is None else data
-        if data is None:
-            raise ValueError("waic() needs data (none was seen by fit / compute_scales yet)")
+        batches = self._batches_of(data, batch_size, "waic()")
         draws = self.surrogate_distribution.sample(int(sample_size), seed=seed)
-        if isinstance(data, CsrShard):
-            batches = data.iter_batches(batch_size or min(data.nrows, 8192))
-        elif callable(data):
-            batches = iter(data())
-        else:
-            batches = [data]
         acc = torch.zeros(4, dtype=torch.float64, device=self.device)     # lppd, pwaic, elpd, elpd^2
         n = 0
         for batch in batches:
@@ -629,6 +648,152 @@ class PoissonFactorization:
         lppd, pwaic, e1, e2 = (float(t) for t in acc.cpu())
         var = max(e2 / n - (e1 / n) ** 2, 0.0) * (n / (n - 1.0) if n > 1 else 1.0)
         return {'waic': -2.0 * e1, 'se': 2.0 * math.sqrt(n * var), 'lppd': lppd, 'pwaic': pwaic}
+
+    def _batches_of(self, data, batch_size, who):
+        """The batches of `data` for the evaluation passes: a CsrShard cut into `batch_size` rows (default
+        min(N, 8192)), a batch factory as for fit(), or one batch / array; default: the factory last given to
+        fit() / compute_scales()."""
+        data = self._last_data_factory if data is None else data
+        if data is None:
+            raise ValueError(f"{who} needs data (none was seen by fit / compute_scales yet)")
+        if isinstance(data, CsrShard):
+            return data.iter_batches(batch_size or min(data.nrows, 8192))
+        if callable(data):
+            return iter(data())
+        return [data]
+
+    # ------------------------------------------------------------------ posterior predictive check
+    def _ppc_engine(self, params, sample_size, seed):
+        """Engine holding the operands of the check's draws: explicit `params` (leading sample axis) or
+        `sample_size` surrogate draws from `seed`.  Neither moves rng_step or opt_step."""
+        if self._custom_link:
+            raise _abi.SpmfError("the posterior predictive check has no CUDA path for custom encoder / decoder "
+                                 "callables")
+        if not params:
+            params = self.surrogate_distribution.sample(int(sample_size), seed=seed)
+        u = torch.as_tensor(params['u'])
+        S = u.shape[0] if u.dim() == 3 else 1
+        if S > _abi.PPC_MAX_S:
+            raise ValueError(f"the check takes at most {_abi.PPC_MAX_S} draws, got {S}")
+        eng = self._engine_for(S)
+        self._operands_from_theta(eng, params['u'], params['v'], params['w'], params['s'])
+        return eng
+
+    def _ppc_device_batch(self, batch):
+        c = batch[self.count_key] if isinstance(batch, dict) else batch
+        b = c if isinstance(c, DeviceBatch) else as_device_batch(c, self.device, self.feature_dim)
+        if b.cols is None:
+            raise ValueError("the posterior predictive check needs a batch with its CSR arrays "
+                             "(not a hybrid-only upload)")
+        return b
+
+    def _ppc_pass(self, eng, b, seed, row_offset, acc, out=None):
+        """Replicates of batch `b` and their statistics (spmf_ppc_rows): per-row results are returned,
+        per-column / per-draw ones accumulate into `acc`."""
+        S, D, B = eng.S, self.feature_dim, b.nrows
+        eng.ensure_rows(B)
+        xd = eng.dense_scratch(B)
+        ws, st = eng.ws, _stream()
+        eng.dense_scatter(b, xd)
+        if self.link & 1:                  # log(x/eta + 1) encoder: dense kernel, as encode()
+            eng.dense_encode(b, xd)
+        else:
+            _abi.call("spmf_csr_encode", _ptr(b.rowptr), _ptr(b.cols), _ptr(b.vals), _ptr(b.rowsum),
+                      eng.inv_xi, int(self.scale_rows), B, D, self.latent_dim, S, _ptr(ws.Ap), _ptr(ws.z), st)
+        dev = self.device
+        row_total = torch.empty(S, B, dtype=torch.int64, device=dev)
+        row_nnz = torch.empty(S, B, dtype=torch.int32, device=dev)
+        row_disc = torch.empty(S, B, 2, dtype=torch.float64, device=dev)
+        disc = torch.empty(S, 2, dtype=torch.float64, device=dev)
+        _abi.call("spmf_ppc_rows", _ptr(xd), B, D, self.latent_dim, S, self.link, _ptr(ws.EV), _ptr(ws.PH),
+                  _ptr(ws.z), int(seed) & 0xFFFFFFFFFFFFFFFF, int(row_offset), _ptr(row_total), _ptr(row_nnz),
+                  _ptr(row_disc), _ptr(acc['col_total']), _ptr(acc['col_sumsq']), _ptr(acc['col_nnz']),
+                  _ptr(acc['max']), _ptr(acc['invalid']), _ptr(out), _ptr(disc), _ptr(acc['scratch']), st)
+        return row_total, row_nnz, disc
+
+    def _ppc_acc(self, S):
+        z = lambda *shape, dt=torch.int64: torch.zeros(*shape, dtype=dt, device=self.device)
+        return dict(col_total=z(S, self.feature_dim), col_sumsq=z(S, self.feature_dim),
+                    col_nnz=z(S, self.feature_dim, dt=torch.int32), max=z(S, dt=torch.int32), invalid=z(S),
+                    scratch=torch.empty(128 * S, dtype=torch.float64, device=self.device))
+
+    def posterior_predictive_check(self, data=None, sample_size=32, batch_size=None, seed=12345, **params):
+        """Posterior predictive check over the rows of `data`: for every draw theta_s a replicated count matrix
+        x_rep ~ p(x | theta_s) (Poisson(rate), or Bernoulli(sigmoid(logit)) for BernoulliFactorization) is drawn
+        by a fused CUDA pass over every entry (csrc/spmf_ppc.cu) and reduced to check statistics on the fly; the
+        (S,B,D) rate and replicate tensors never exist.
+
+        `data` is taken as by waic(): a batch factory, a CsrShard (cut into `batch_size` rows), one batch or an
+        array; default: the factory last given to fit() / compute_scales().  Draws: explicit s, u, v, w with a
+        leading sample axis (as for row_log_likelihood), else `sample_size` surrogate draws from `seed`; the same
+        draws serve every batch.  The replicate of entry (s, row, d) comes from a Philox stream keyed by (seed, s,
+        global row, d) -- rows are numbered across the batches in order -- so the result does not depend on the
+        batch size, and two calls with the same arguments give bit-identical results.  Neither rng_step nor
+        opt_step moves.  Under torch.distributed each rank checks its own shard (no aggregation across ranks).
+
+        Returns (observed, replicated, p_value, invalid):
+          observed:   'row_total', 'row_nnz' (N,); 'col_total', 'col_sumsq', 'col_nnz' (D,); 'total', 'nnz',
+                      'max' (scalars); 'discrepancy' (S,) = D(x, theta_s)
+          replicated: the same keys with a leading S axis (integers, exact); 'discrepancy' (S,) = D(x_rep_s, theta_s)
+          p_value:    ppc_p_values(observed, replicated): the mid-p (#{T_rep > T_obs} + 0.5 #{T_rep == T_obs}) / S of
+                      every statistic, the discrepancy paired per draw, plus 'col_var'
+          invalid:    (S,) entries whose rate is negative, not finite or above 2^24 (Poisson) or whose logit is
+                      not finite (Bernoulli): their replicate is 0 and they are left out of both discrepancies.
+        The discrepancy is D(y, theta) = sum (y - rate)^2 / rate (Poisson) or sum (y - p)^2 / (p (1 - p))
+        (Bernoulli) over the valid entries, summed in fp64 in a fixed order; an entry with rate (or p (1 - p))
+        0 adds 0 where y equals it and +inf elsewhere."""
+        batches = self._batches_of(data, batch_size, "posterior_predictive_check()")
+        eng = self._ppc_engine(params, sample_size, seed)
+        S, D, dev = eng.S, self.feature_dim, self.device
+        acc = self._ppc_acc(S)
+        obs_col = dict(col_total=torch.zeros(D, dtype=torch.float64, device=dev),
+                       col_sumsq=torch.zeros(D, dtype=torch.float64, device=dev),
+                       col_nnz=torch.zeros(D, dtype=torch.int32, device=dev))
+        rep_rows, rep_nnz, obs_rows, obs_nnz = [], [], [], []
+        disc = torch.zeros(S, 2, dtype=torch.float64, device=dev)
+        obs_max = torch.zeros((), dtype=torch.float32, device=dev)
+        row_offset = 0
+        for batch in batches:
+            b = self._ppc_device_batch(batch)
+            rt, rn, d = self._ppc_pass(eng, b, seed, row_offset, acc)
+            rep_rows.append(rt)
+            rep_nnz.append(rn)
+            disc += d                                       # batch order: a fixed summation order
+            ot = torch.empty(b.nrows, dtype=torch.float64, device=dev)
+            on = torch.empty(b.nrows, dtype=torch.int32, device=dev)
+            _abi.call("spmf_ppc_observed", _ptr(b.rowptr), _ptr(b.cols), _ptr(b.vals), b.nrows, D, _ptr(ot),
+                      _ptr(on), _ptr(obs_col['col_total']), _ptr(obs_col['col_sumsq']), _ptr(obs_col['col_nnz']),
+                      _stream())
+            obs_rows.append(ot)
+            obs_nnz.append(on)
+            obs_max = torch.maximum(obs_max, eng.ws.xdense[:b.nrows * D].max())
+            row_offset += b.nrows
+        if row_offset == 0:
+            raise ValueError("posterior_predictive_check(): the data holds no rows")
+        rep_rows, rep_nnz = torch.cat(rep_rows, 1), torch.cat(rep_nnz, 1)
+        obs_rows, obs_nnz = torch.cat(obs_rows), torch.cat(obs_nnz)
+        observed = dict(row_total=obs_rows, row_nnz=obs_nnz, **obs_col, total=obs_rows.sum(),
+                        nnz=obs_nnz.sum(dtype=torch.int64), max=obs_max.to(torch.float64), discrepancy=disc[:, 1])
+        replicated = dict(row_total=rep_rows, row_nnz=rep_nnz, col_total=acc['col_total'],
+                          col_sumsq=acc['col_sumsq'], col_nnz=acc['col_nnz'], total=rep_rows.sum(1),
+                          nnz=rep_nnz.sum(1, dtype=torch.int64), max=acc['max'], discrepancy=disc[:, 0])
+        return observed, replicated, ppc_p_values(observed, replicated), acc['invalid']
+
+    def posterior_predictive_sample(self, data, sample_size=8, seed=12345, row_offset=0, **params):
+        """The replicates x_rep of one batch as an int32 (S, B, D) device tensor: the same kernel, draws and
+        Philox streams as posterior_predictive_check (rows numbered from `row_offset`), so the statistics of these
+        replicates are the check's statistics.  Draws as for the check.  Raises ValueError above PPC_SAMPLE_LIMIT
+        (2^30) entries."""
+        b = self._ppc_device_batch(data)
+        u = torch.as_tensor(params['u']) if params else None
+        S = int(sample_size) if u is None else (u.shape[0] if u.dim() == 3 else 1)
+        if S * b.nrows * self.feature_dim > PPC_SAMPLE_LIMIT:
+            raise ValueError(f"{S} x {b.nrows} x {self.feature_dim} replicates exceed the limit of {PPC_SAMPLE_LIMIT} "
+                             "entries: use posterior_predictive_check, or fewer rows / draws")
+        eng = self._ppc_engine(params, sample_size, seed)
+        out = torch.empty(eng.S, b.nrows, self.feature_dim, dtype=torch.int32, device=self.device)
+        self._ppc_pass(eng, b, seed, row_offset, self._ppc_acc(eng.S), out=out)
+        return out
 
     def sample(self, n=None, seed=None):
         """[EXT] BayesianModel.sample: draws of every latent variable from the surrogate posterior."""
