@@ -46,13 +46,23 @@ def _as_csr(x):
     return m
 
 
-def analytic_loss_and_grads(model, params, noise, x, c_gamma=False):
+def analytic_loss_and_grads(model, params, noise, x, c_gamma=False, magnitudes=False):
     """Returns (loss, grads dict, parts dict of (S,) arrays).  `model` is an
     OraclePoissonFactorization (only its hyper-parameters / eta / xi are read).  `x`: the (B,D)
     counts, dense or scipy.sparse -- only the nonzeros are visited (the same sparse closed form
     the kernels use), so a bench-sized batch (8192 x 20000, ~8e6 nonzeros) is evaluated in float64
     on the CPU without the (S,B,D) rate tensor.  c_gamma: use the C helper (oracle/gamma_der.c) for
-    the implicit Gamma gradient instead of the vectorised python series (same expansions)."""
+    the implicit Gamma gradient instead of the vectorised python series (same expansions).
+
+    magnitudes=True returns (loss, grads, parts, mags, rows) for an element-wise check of an fp32 kernel:
+      mags: for every gradient of v, w, u, s ('<var>/loc', '<var>/scale_raw'), a float64 array M of the same
+            shape: the same formulas evaluated with every summand of every signed sum replaced by its absolute
+            value, data term, chain and prior terms alike.  M bounds the cancellation at each element, so
+            |got - ref| <= rtol * M is a test whose strength does not depend on the element's size.  Also the
+            data-term sums alone, summed over the draws: 'data/GAp' (D,K), 'data/GEV' (D,K), 'data/Gphi' (D,).
+      rows: {'z': (z, Mz) of shape (S,B,K), 'row_ll': (ll, Mll) of shape (S,B)} -- the encoding and the
+            per-row Poisson log-likelihood with their magnitudes.  Mll counts x (|log lambda| + 1) per
+            nonzero: an error relative to lambda is an absolute error in log lambda."""
     import scipy.sparse as sp
     import torch
     P = {k: v.detach().numpy().astype(np.float64) for k, v in params.items()}
@@ -164,6 +174,11 @@ def analytic_loss_and_grads(model, params, noise, x, c_gamma=False):
     Xr = sp.diags(r) @ X                                          # rows scaled by r_b
     Lx = np.zeros(S); Lz = np.zeros(S)
     GAp = np.zeros_like(Ap); GEV = np.zeros_like(EV); Gphi = np.zeros_like(phi)
+    # magnitudes: every operand is >= 0 here (x, r, A', eta*v, phi, z, lambda), so only the signed
+    # sums (dz, GEV, Gphi) and what they feed need the absolute-value restatement
+    MGAp = np.zeros_like(Ap); MGEV = np.zeros_like(EV); MGphi = np.zeros_like(phi)
+    Z = np.zeros((S, B, K)); ROW_LL = np.zeros((S, B)); MROW_LL = np.zeros((S, B))
+    lgam_row = np.asarray(sp.csr_matrix((gammaln(xv + 1.0), di, indptr), shape=(B, D)).sum(1)).reshape(B)
     CH = 1 << 20                                                  # nonzeros per chunk (bounds temporaries)
     for s in range(S):
         z = Xr @ Ap[s]                                            # (B,K) = r_b * (x @ A')
@@ -180,6 +195,17 @@ def analytic_loss_and_grads(model, params, noise, x, c_gamma=False):
         GEV[s] = W.T @ z - z.sum(0)[None, :]
         Gphi[s] = np.asarray(W.sum(0)).reshape(D) - B
         GAp[s] = Xr.T @ dz
+        if magnitudes:
+            Mdz = W @ EV[s] + vsum[None, :] + z
+            MGEV[s] = W.T @ z + z.sum(0)[None, :]
+            MGphi[s] = np.asarray(W.sum(0)).reshape(D) + B
+            MGAp[s] = Xr.T @ Mdz
+            Z[s] = z
+            xl = sp.csr_matrix((xv * np.log(lam), di, indptr), shape=(B, D))
+            xm = sp.csr_matrix((xv * (np.abs(np.log(lam)) + 1.0), di, indptr), shape=(B, D))
+            rate_sum = z @ vsum + phi[s].sum()
+            ROW_LL[s] = np.asarray(xl.sum(1)).reshape(B) - lgam_row - rate_sum
+            MROW_LL[s] = np.asarray(xm.sum(1)).reshape(B) + lgam_row + rate_sum
     parts['z'] = Lz
     parts['x'] = Lx
 
@@ -192,11 +218,24 @@ def analytic_loss_and_grads(model, params, noise, x, c_gamma=False):
     den = (s0 + s1) ** 2
     dth['s'][:, 0, :] += (da - db) * s1 / den
     dth['s'][:, 1, :] += (db - da) * s0 / den
+    if magnitudes:
+        # prior terms of v, w, u, s in absolute value (the InverseGamma family is not checked element-wise)
+        sig_u = th['u_eta'] * th['u_tau'] * c_k
+        sig_s = th['s_eta'] * th['s_tau']
+        mth = {'v': th['v'] / 0.01, 'w': th['w'].copy(), 'u': th['u'] / sig_u ** 2, 's': th['s'] / sig_s ** 2}
+        mth['u'] += MGAp * a_d[:, :, None] / eta[None, :, None]
+        Mda = (MGAp * th['u']).sum(-1) / eta[None, :]
+        mth['v'] += np.swapaxes(MGEV * eta[None, :, None], -1, -2)
+        mth['w'] += (eta[None, :] * b_d * MGphi)[:, None, :]
+        Mdb = eta[None, :] * th['w'][:, 0, :] * MGphi
+        mth['s'][:, 0, :] += (Mda + Mdb) * s1 / den
+        mth['s'][:, 1, :] += (Mda + Mdb) * s0 / den
 
     # ---------------- loss and grads of the 24 variational tensors ----------------
     target = sum(parts.values())
     loss = float((logq - target).mean())
     grads = {}
+    mags = {}
     for k in VAR_LIST:
         # d loss_s / d t  with loss_s = logq_s - target_s ;  y = softplus(t)
         Gy = -dth[k]
@@ -206,6 +245,10 @@ def analytic_loss_and_grads(model, params, noise, x, c_gamma=False):
             grads[k + '/loc'] = dt.mean(0)
             srho = sigmoid(P[k + '/scale_raw'])
             grads[k + '/scale_raw'] = (dt * Nz[k]).mean(0) * srho - srho / sig
+            if magnitudes:
+                Mdt = mth[k] * sg[k] + (1.0 - sg[k])
+                mags[k + '/loc'] = Mdt.mean(0)
+                mags[k + '/scale_raw'] = (Mdt * np.abs(Nz[k])).mean(0) * srho + srho / sig
         else:
             al, be, g = aux[k]
             t = t_pre[k]
@@ -224,4 +267,9 @@ def analytic_loss_and_grads(model, params, noise, x, c_gamma=False):
             grads[k + '/conc_raw'] = dal.mean(0) * sigmoid(P[k + '/conc_raw'])
             grads[k + '/scale_raw'] = dbe.mean(0) * sigmoid(P[k + '/scale_raw'])
     parts['logq'] = logq
-    return loss, grads, parts
+    if not magnitudes:
+        return loss, grads, parts
+    mags['data/GAp'] = MGAp.sum(0)
+    mags['data/GEV'] = MGEV.sum(0)
+    mags['data/Gphi'] = MGphi.sum(0)
+    return loss, grads, parts, mags, {'z': (Z, Z.copy()), 'row_ll': (ROW_LL, MROW_LL)}
