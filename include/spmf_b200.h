@@ -564,6 +564,30 @@ int spmf_ppc_observed(const long long* rowptr, const int* cols, const float* val
                       double* row_total, int* row_nnz, double* col_total, double* col_sumsq, unsigned int* col_nnz,
                       void* stream);
 
+/* ---- PSIS leave-one-out (csrc/spmf_loo.cu) ----
+ * ll: row-major [nrows][ld] fp64 (ld >= S), ll[b][s] = log p(x_b | theta_s).  Per row b:
+ * elpd[b] = PSIS-LOO log predictive density, lppd[b] = log mean_s exp(ll[b][s]), khat[b] = Pareto k-hat.
+ * 1 <= S <= SPMF_LOO_MAX_S (8192).  Deterministic: bit-identical from run to run, and independent of nrows.
+ *
+ * The algorithm is ArviZ's _psislw / _gpdfit with r_eff = 1 (the surrogate draws are independent); all in fp64:
+ *  1. r_s = -ll_s - max_s(-ll_s).  M = ceil(min(0.2 S, 3 sqrt(S))), capped at S - 1.  cutoff = max(r_(S-M),
+ *     log(DBL_MIN)), r_(S-M) the (M+1)-th largest value; the tail is the n values strictly above the cutoff.
+ *  2. n <= 4: khat = +inf, no smoothing.  Otherwise the generalised Pareto fit (Zhang & Stephens 2009, Vehtari's
+ *     prior) to y = exp(tail) - exp(cutoff), ascending: m = 30 + floor(sqrt(n)) grid points
+ *     b_j = 1/y_n + (1 - sqrt(m/(j - 1/2))) / (3 y_floor(n/4 + 1/2)), k_j = mean_i log1p(-b_j y_i),
+ *     L_j = n (log(-b_j/k_j) - k_j - 1), w_j = 1 / sum_i exp(L_i - L_j) (an exp that overflows gives w_j = 0);
+ *     w_j < 10 DBL_EPSILON is dropped and the rest renormalised; b = sum_j w_j b_j, k = mean_i log1p(-b y_i),
+ *     sigma = -k/b, khat = (n k + 5)/(n + 10).
+ *  3. If khat and sigma > 0 are finite, the i-th smallest tail value becomes
+ *     log(sigma expm1(-khat log1p(-(i - 1/2)/n)) / khat + exp(cutoff)) (-log1p(-p) when |khat| < DBL_EPSILON), and
+ *     every log weight is clamped at 0, the largest raw one.  Otherwise khat = +inf and the raw weights stay.
+ *  4. lw = r - logsumexp(r); elpd = logsumexp(lw + ll); lppd = logsumexp(ll) - log S.
+ *  5. A row holding -inf (and no NaN / +inf): elpd = -inf (the estimate 1/mean(1/p) = 0), khat = +inf, lppd as in 4.
+ *     A row holding NaN or +inf: NaN in all three outputs. */
+#define SPMF_LOO_MAX_S 8192
+int spmf_psis_loo(const double* ll, long long ld, int nrows, int S, double* elpd, double* lppd, float* khat,
+                  void* stream);
+
 const char* spmf_version(void);
 
 #ifdef __cplusplus

@@ -17,6 +17,7 @@ NUM_PARTS = 16
 MAX_K = 512        # latent dimensions of the gather / dense kernels (SPMF_MAX_K)
 MAX_TILE_K = 128   # latent dimensions of the tensor-core hybrid path (SPMF_MAX_TILE_K)
 PPC_MAX_S = 65535  # draws of one posterior predictive check (SPMF_PPC_MAX_S)
+LOO_MAX_S = 8192   # draws of one PSIS leave-one-out evaluation (SPMF_LOO_MAX_S)
 
 
 class SpmfError(RuntimeError):
@@ -117,6 +118,8 @@ _SIGS = {
     # posterior predictive check (spmf_ppc.cu)
     "spmf_ppc_rows": (i32, [p, i32, i32, i32, i32, i32, p, p, p, u64, i64, p, p, p, p, p, p, p, p, p, p, p, p]),
     "spmf_ppc_observed": (i32, [p, p, p, i32, i32, p, p, p, p, p, p]),
+    # PSIS leave-one-out (spmf_loo.cu)
+    "spmf_psis_loo": (i32, [p, i64, i32, i32, p, p, p, p]),
 }
 
 

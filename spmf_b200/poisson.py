@@ -63,6 +63,21 @@ def waic_terms(ll):
     return lppd, pwaic
 
 
+LOO_DRAW_CHUNK = 64     # surrogate draws loo() regenerates at a time (bounds its engine memory whatever S is)
+
+
+def loo_compare(a, b):
+    """Difference of two loo() results over the same rows (e.g. two latent dimensions or links):
+    'elpd_diff' = sum_i (a_i - b_i) and 'se_diff' = sqrt(n var(a_i - b_i)) of the pointwise elpd_loo."""
+    ea, eb = a['pointwise']['elpd_loo'], b['pointwise']['elpd_loo']
+    if ea.numel() != eb.numel():
+        raise ValueError(f"loo_compare: the results cover {ea.numel()} and {eb.numel()} rows; they must be the same rows")
+    d = ea.to(torch.float64) - eb.to(device=ea.device, dtype=torch.float64)
+    n = d.numel()
+    var = float(d.var(unbiased=True)) if n > 1 else 0.0
+    return {'elpd_diff': float(d.sum()), 'se_diff': math.sqrt(n * var)}
+
+
 PPC_SAMPLE_LIMIT = 1 << 30      # replicates posterior_predictive_sample materialises at most (4 GiB of int32)
 PPC_INTEGER_STATS = ('row_total', 'row_nnz', 'col_total', 'col_sumsq', 'col_nnz', 'total', 'nnz', 'max')
 
@@ -604,13 +619,24 @@ class PoissonFactorization:
         u = torch.as_tensor(params['u'])
         S = u.shape[0] if u.dim() == 3 else 1
         eng = self._engine_for(S)
+        b = self._csr_batch(data, "row_log_likelihood")
+        self._operands_from_theta(eng, params['u'], params['v'], params['w'], params['s'])
+        return self._row_ll(eng, b)
+
+    def _csr_batch(self, data, who):
         c = data[self.count_key] if isinstance(data, dict) else data
         b = c if isinstance(c, DeviceBatch) else as_device_batch(c, self.device, self.feature_dim)
         if b.cols is None:
-            raise ValueError("row_log_likelihood needs a batch with its CSR arrays (not a hybrid-only upload)")
+            raise ValueError(f"{who} needs a batch with its CSR arrays (not a hybrid-only upload)")
+        return b
+
+    def _row_ll(self, eng, b):
+        """(S, B) float64 per-row log-likelihoods of batch `b` for the operand tables currently in `eng`'s
+        workspace: the CUDA row pass (sparse link), the dense row pass (other links) or the torch data term of
+        custom callables."""
+        S = eng.S
         eng.ensure_rows(b.nrows)
         ws = eng.ws
-        self._operands_from_theta(eng, params['u'], params['v'], params['w'], params['s'])
         if self._custom_link:
             eng.reset_guard()
             eng.custom_data_term(b, eng._guard_scratch(b.nrows), forward_only=True)
@@ -648,6 +674,80 @@ class PoissonFactorization:
         lppd, pwaic, e1, e2 = (float(t) for t in acc.cpu())
         var = max(e2 / n - (e1 / n) ** 2, 0.0) * (n / (n - 1.0) if n > 1 else 1.0)
         return {'waic': -2.0 * e1, 'se': 2.0 * math.sqrt(n * var), 'lppd': lppd, 'pwaic': pwaic}
+
+    def loo(self, data=None, sample_size=1000, batch_size=None, seed=12345, **params):
+        """Pareto-smoothed importance-sampling leave-one-out cross-validation (PSIS-LOO, Vehtari, Gelman & Gabry
+        2017) over the ROWS of `data`, with the Pareto k-hat diagnostic of every row: where k-hat is above
+        `khat_threshold`, that row's estimate is not to be trusted.
+
+        `data` is taken as by waic().  Draws: explicit s, u, v, w with a leading sample axis, else `sample_size`
+        surrogate draws; the same draws serve every batch.  Surrogate draws are taken in chunks of LOO_DRAW_CHUNK:
+        chunk c holds exactly the draws surrogate_distribution.sample(n_c, seed=seed + c) returns.  Draws are
+        regenerated per batch and chunk, so memory stays at one chunk's engine and one batch's [B][S] fp64
+        log-likelihoods whatever S is (at most LOO_MAX_S).  The per-row log-likelihoods come from the row pass of
+        row_log_likelihood; the smoothing runs in one CUDA kernel per batch (spmf_psis_loo, csrc/spmf_loo.cu).
+        Neither rng_step nor opt_step moves.  Under torch.distributed each rank evaluates its own shard.
+
+        Returns a dict: 'elpd_loo' = sum_i elpd_i, 'se' = sqrt(n var(elpd_i)), 'p_loo' = sum_i (lppd_i - elpd_i),
+        'looic' = -2 elpd_loo, 'lppd' = sum_i lppd_i, 'khat_threshold' = min(1 - 1/log10(S), 0.7),
+        'n_khat_above' (rows above it, k-hat = inf included), 'n_nonfinite' (rows whose elpd is not finite: a
+        draw of zero likelihood gives -inf, a NaN or +inf log-likelihood gives NaN), and 'pointwise': device
+        tensors 'elpd_loo', 'p_loo' (float64) and 'khat' (float32) of shape (N,), in row order.  Sums over rows
+        run in batch order."""
+        batches = self._batches_of(data, batch_size, "loo()")
+        if params:
+            theta = {k: torch.as_tensor(params[k]) for k in ('s', 'u', 'v', 'w')}
+            if theta['u'].dim() == 2:
+                theta = {k: t[None] for k, t in theta.items()}
+            S = theta['u'].shape[0]
+        else:
+            theta, S = None, int(sample_size)
+        if not 1 <= S <= _abi.LOO_MAX_S:
+            raise ValueError(f"loo() takes 1 to {_abi.LOO_MAX_S} draws, got {S}")
+        dev, f64 = self.device, torch.float64
+        acc = torch.zeros(4, dtype=f64, device=dev)     # elpd, elpd^2, lppd, p_loo
+        elpd_all, ploo_all, khat_all = [], [], []
+        for batch in batches:
+            b = self._csr_batch(batch, "loo()")
+            if b.nrows == 0:
+                continue
+            ll = self._loo_row_ll(b, S, seed, theta)
+            elpd = torch.empty(b.nrows, dtype=f64, device=dev)
+            lppd = torch.empty(b.nrows, dtype=f64, device=dev)
+            khat = torch.empty(b.nrows, dtype=torch.float32, device=dev)
+            _abi.call("spmf_psis_loo", _ptr(ll), S, b.nrows, S, _ptr(elpd), _ptr(lppd), _ptr(khat), _stream())
+            ploo = lppd - elpd
+            acc += torch.stack([elpd.sum(), (elpd * elpd).sum(), lppd.sum(), ploo.sum()])
+            elpd_all.append(elpd)
+            ploo_all.append(ploo)
+            khat_all.append(khat)
+        if not elpd_all:
+            raise ValueError("loo(): the data holds no rows")
+        elpd, ploo, khat = torch.cat(elpd_all), torch.cat(ploo_all), torch.cat(khat_all)
+        n = elpd.numel()
+        e1, e2, lppd, p_loo = (float(t) for t in acc.cpu())
+        var = max(e2 / n - (e1 / n) ** 2, 0.0) * (n / (n - 1.0) if n > 1 else 1.0)
+        threshold = min(1.0 - 1.0 / math.log10(S), 0.7) if S > 1 else -math.inf
+        return {'elpd_loo': e1, 'se': math.sqrt(n * var), 'p_loo': p_loo, 'looic': -2.0 * e1, 'lppd': lppd,
+                'khat_threshold': threshold, 'n_khat_above': int((khat > threshold).sum()),
+                'n_nonfinite': int((~torch.isfinite(elpd)).sum()),
+                'pointwise': {'elpd_loo': elpd, 'p_loo': ploo, 'khat': khat}}
+
+    def _loo_row_ll(self, b, S, seed, theta):
+        """[B][S] fp64 per-row log-likelihoods of batch `b` for loo(): draws in chunks of LOO_DRAW_CHUNK, chunk c
+        either the Normal draws sample(n_c, seed + c) makes (theta None, regenerated here without moving rng_step)
+        or the slice of the explicit draws `theta` (dict of s, u, v, w with a leading sample axis)."""
+        ll = torch.empty(b.nrows, S, dtype=torch.float64, device=self.device)
+        for c, c0 in enumerate(range(0, S, LOO_DRAW_CHUNK)):
+            nc = min(LOO_DRAW_CHUNK, S - c0)
+            eng = self._engine_for(nc)
+            if theta is None:
+                eng.fill_noise(step=int(seed) + c, which=AdviEngine.NOISE_NORMAL, advance=False)
+                eng.draw_operands()
+            else:
+                self._operands_from_theta(eng, *(theta[k][c0:c0 + nc] for k in ('u', 'v', 'w', 's')))
+            ll[:, c0:c0 + nc].copy_(self._row_ll(eng, b).t())
+        return ll
 
     def _batches_of(self, data, batch_size, who):
         """The batches of `data` for the evaluation passes: a CsrShard cut into `batch_size` rows (default
