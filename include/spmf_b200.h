@@ -587,6 +587,42 @@ int spmf_ppc_observed(const long long* rowptr, const int* cols, const float* val
 #define SPMF_LOO_MAX_S 8192
 int spmf_psis_loo(const double* ll, long long ld, int nrows, int S, double* elpd, double* lppd, float* khat,
                   void* stream);
+/* The same, and lw[b][s] (row stride ldw >= S) = the normalised log weights of step 4, smoothed and truncated, in
+ * draw order (sum_s exp(lw[b][s]) = 1); a tied draw of the tail takes the smoothed weight a stable sort of the
+ * log-ratios gives it.  Rows of step 5 (elpd not finite) get lw = NaN.  elpd, lppd and khat are bit-identical to
+ * spmf_psis_loo's. */
+int spmf_psis_loo_lw(const double* ll, long long ld, int nrows, int S, double* elpd, double* lppd, float* khat,
+                     double* lw, long long ldw, void* stream);
+
+/* ---- LOO-PIT (csrc/spmf_pit.cu, CDFs and binning in csrc/spmf_pit.cuh) ----
+ * The probability integral transform of every entry under its row's leave-one-out predictive, non-randomised
+ * (Czado, Gneiting & Held 2009) for counts.
+ * spmf_loo_pit_accum: one chunk of S <= SPMF_LOO_PIT_MAX_DRAWS draws; xd, z, EV, PH as for spmf_ppc_rows (any link,
+ * K <= SPMF_MAX_K); lw = the chunk's first column of spmf_psis_loo_lw's weights (lw[b * ldw + s], s < S).  For
+ * every entry (b, d), adds in fp64
+ *   acc[b][d][0] += sum_s exp(lw[b][s]) F(x_bd - 1 | theta_s),   acc[b][d][1] += sum_s exp(lw[b][s]) F(x_bd | theta_s)
+ * with F the Poisson CDF of the rate (links 0, 1) or the Bernoulli CDF of the logit (links 2, 3) that link_rate
+ * forms, and adds to inv[b][d] the draws at which the entry is invalid: a Poisson rate that is negative, not
+ * finite or above 2^24, a logit that is not finite, or an observed value that is not an integer of the support
+ * (0 <= x <= 2^24, or x in {0, 1} for Bernoulli).  Invalid draws add nothing to acc.  Within the chunk the draws
+ * are added in ascending s, into the value acc held before the call: calling the chunks in order sums every entry
+ * in one fixed order, independent of nrows, the batch split and the launch geometry, so acc is bit-identical from
+ * run to run.  rate_out[S][nrows][D] (fp32, may be NULL) = the rate (or logit) of every entry.
+ * spmf_loo_pit_hist: for every entry with inv == 0 and finite acc (a row of NaN weights is left out), the PIT
+ * distribution F(u) = 0 (u <= P-), (u - P-)/(P+ - P-) (P- < u < P+), 1 (u >= P+) with P-, P+ = acc clamped to
+ * [0, 1]; bin j = 0..J-1 gets F((j+1)/J) - F(j/J), or, if P+ <= P-, unit mass in bin min(J - 1, floor(P+ J)).
+ * Adds (the caller zeroes) col_hist[D][J], col_n[D] (valid entries) and col_pit_sum[D] (sum of (P- + P+)/2).
+ * The sums over the rows run in a fixed order (blocks of 1024 rows, then the blocks in order; no atomics), so the
+ * outputs are bit-identical from run to run.  1 <= J <= SPMF_LOO_PIT_MAX_BINS; scratch: spmf_loo_pit_hist_scratch
+ * _doubles(nrows, D, J) doubles. */
+#define SPMF_LOO_PIT_MAX_DRAWS 64
+#define SPMF_LOO_PIT_MAX_BINS 1000
+int spmf_loo_pit_accum(const float* xd, int nrows, int D, int K, int S, int link, const float* EV, const float* PH,
+                       const float* z, const double* lw, long long ldw, double* acc, int* inv, float* rate_out,
+                       void* stream);
+long long spmf_loo_pit_hist_scratch_doubles(int nrows, int D, int J);
+int spmf_loo_pit_hist(const double* acc, const int* inv, int nrows, int D, int J, double* col_hist,
+                      long long* col_n, double* col_pit_sum, double* scratch, void* stream);
 
 const char* spmf_version(void);
 

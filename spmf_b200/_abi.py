@@ -18,6 +18,8 @@ MAX_K = 512        # latent dimensions of the gather / dense kernels (SPMF_MAX_K
 MAX_TILE_K = 128   # latent dimensions of the tensor-core hybrid path (SPMF_MAX_TILE_K)
 PPC_MAX_S = 65535  # draws of one posterior predictive check (SPMF_PPC_MAX_S)
 LOO_MAX_S = 8192   # draws of one PSIS leave-one-out evaluation (SPMF_LOO_MAX_S)
+LOO_PIT_MAX_DRAWS = 64    # draws of one spmf_loo_pit_accum chunk (SPMF_LOO_PIT_MAX_DRAWS)
+LOO_PIT_MAX_BINS = 1000   # PIT histogram bins (SPMF_LOO_PIT_MAX_BINS)
 
 
 class SpmfError(RuntimeError):
@@ -120,6 +122,11 @@ _SIGS = {
     "spmf_ppc_observed": (i32, [p, p, p, i32, i32, p, p, p, p, p, p]),
     # PSIS leave-one-out (spmf_loo.cu)
     "spmf_psis_loo": (i32, [p, i64, i32, i32, p, p, p, p]),
+    "spmf_psis_loo_lw": (i32, [p, i64, i32, i32, p, p, p, p, i64, p]),
+    # LOO-PIT (spmf_pit.cu)
+    "spmf_loo_pit_accum": (i32, [p, i32, i32, i32, i32, i32, p, p, p, p, i64, p, p, p, p]),
+    "spmf_loo_pit_hist_scratch_doubles": (i64, [i32, i32, i32]),
+    "spmf_loo_pit_hist": (i32, [p, p, i32, i32, i32, p, p, p, p, p]),
 }
 
 

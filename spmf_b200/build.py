@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libspmf_b200.so")
-SOURCES = ["spmf_params.cu", "spmf_sparse.cu", "spmf_umma.cu", "spmf_hot_tile.cu", "spmf_dense.cu", "spmf_ppc.cu", "spmf_loo.cu",
+SOURCES = ["spmf_params.cu", "spmf_sparse.cu", "spmf_umma.cu", "spmf_hot_tile.cu", "spmf_dense.cu", "spmf_ppc.cu", "spmf_loo.cu", "spmf_pit.cu",
            "spmf_p2p.cu", "spmf_step.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]

@@ -9,6 +9,9 @@
 // thread 0 for the weighted grid mean.  Every reduction has a fixed order: a strided per-thread partial, a warp
 // butterfly, then the warps' results in warp order.  Nothing is accumulated with atomics, so the outputs are
 // bit-identical from run to run and a row's result does not depend on the other rows or on nrows.
+// With `lw` given, each thread then writes the normalised log weights of its draws in draw order: a draw of the
+// tail finds its sorted position by a binary search of the sorted row (tied draws of the tail are ranked by
+// draw index, as a stable sort of the log-ratios ranks them).
 #include <cuda_runtime.h>
 #include <float.h>
 #include <math.h>
@@ -51,9 +54,12 @@ __device__ __forceinline__ double loo_block_max(double v, double* red) {
   return t;
 }
 
+// LW: also write the log weights (spmf_psis_loo_lw).  A template argument rather than a run-time test of lw, so
+// that the instance without them compiles to the kernel spmf_psis_loo always ran (60 registers, no spills).
+template <bool LW>
 __global__ void __launch_bounds__(kLooThreads)
 psis_loo_kernel(const double* __restrict__ ll, long long ld, int S, int P, double* __restrict__ elpd,
-                double* __restrict__ lppd, float* __restrict__ khat) {
+                double* __restrict__ lppd, float* __restrict__ khat, double* __restrict__ lw, long long ldw) {
   extern __shared__ double sv[];                     // [P] the row, sorted ascending (padding +inf)
   __shared__ double red[kLooWarps];
   __shared__ double tl[kLooMaxTail];                 // tail: y ascending, then its smoothed log weights
@@ -63,6 +69,7 @@ psis_loo_kernel(const double* __restrict__ ll, long long ld, int S, int P, doubl
   const long long row = blockIdx.x;
   const double* x = ll + row * ld;
   const double INF = __longlong_as_double(0x7ff0000000000000ll);
+  const double NaN = __longlong_as_double(0x7ff8000000000000ll);
 
   bool bad = false, neg = false;
   double mx = -INF;
@@ -78,9 +85,11 @@ psis_loo_kernel(const double* __restrict__ ll, long long ld, int S, int P, doubl
   }
   if (__syncthreads_or(bad)) {                       // NaN or +inf: nothing is defined
     if (tid == 0) {
-      elpd[row] = lppd[row] = __longlong_as_double(0x7ff8000000000000ll);
+      elpd[row] = lppd[row] = NaN;
       khat[row] = __int_as_float(0x7fc00000);
     }
+    if (LW)
+      for (int s = tid; s < S; s += kLooThreads) lw[row * ldw + s] = NaN;
     return;
   }
   neg = __syncthreads_or(neg);
@@ -96,6 +105,8 @@ psis_loo_kernel(const double* __restrict__ ll, long long ld, int S, int P, doubl
       lppd[row] = lp;
       khat[row] = __int_as_float(0x7f800000);
     }
+    if (LW)
+      for (int s = tid; s < S; s += kLooThreads) lw[row * ldw + s] = NaN;
     return;
   }
 
@@ -197,28 +208,60 @@ psis_loo_kernel(const double* __restrict__ ll, long long ld, int S, int P, doubl
     lppd[row] = lp;
     khat[row] = (float)kh;
   }
+  if (!LW) return;
+  // lw in draw order: the tail draws take their smoothed weight from their position in the sorted row
+  for (int s = tid; s < S; s += kLooThreads) {
+    const double v = __ldg(x + s);
+    double r = -v - rmax;
+    if (smooth) {
+      int lo = 0, hi = n;                            // first sorted position holding v, if v is in the tail sv[0, n)
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (sv[mid] < v) lo = mid + 1; else hi = mid;
+      }
+      if (lo < n) {
+        int t = lo;
+        if (lo + 1 < n && sv[lo + 1] == v)           // tied tail draws: a later draw takes an earlier position
+          for (int j = s + 1; j < S; ++j) t += __ldg(x + j) == v;
+        r = tl[n - 1 - t];
+      }
+    }
+    lw[row * ldw + s] = r - lse_r;
+  }
 }
 
 }  // namespace spmf
 
 using namespace spmf;
 
-extern "C" {
-
-int spmf_psis_loo(const double* ll, long long ld, int nrows, int S, double* elpd, double* lppd, float* khat,
-                  void* stream) {
+static int psis_loo_launch(const double* ll, long long ld, int nrows, int S, double* elpd, double* lppd, float* khat,
+                           double* lw, long long ldw, void* stream) {
   if (!ll || !elpd || !lppd || !khat) return SPMF_ERR_BAD_ARG;
   if (nrows <= 0 || S < 1 || S > SPMF_LOO_MAX_S || ld < S) return SPMF_ERR_BAD_ARG;
   int P = 1;
   while (P < S) P <<= 1;
   const size_t smem = sizeof(double) * (size_t)P;
+  auto kern = lw ? psis_loo_kernel<true> : psis_loo_kernel<false>;
   if (smem > 48 * 1024) {
-    const cudaError_t e = cudaFuncSetAttribute(psis_loo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
   }
-  psis_loo_kernel<<<(unsigned)nrows, kLooThreads, smem, (cudaStream_t)stream>>>(ll, ld, S, P, elpd, lppd, khat);
+  kern<<<(unsigned)nrows, kLooThreads, smem, (cudaStream_t)stream>>>(ll, ld, S, P, elpd, lppd, khat, lw, ldw);
   const cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? SPMF_OK : (int)e;
+}
+
+extern "C" {
+
+int spmf_psis_loo(const double* ll, long long ld, int nrows, int S, double* elpd, double* lppd, float* khat,
+                  void* stream) {
+  return psis_loo_launch(ll, ld, nrows, S, elpd, lppd, khat, nullptr, 0, stream);
+}
+
+int spmf_psis_loo_lw(const double* ll, long long ld, int nrows, int S, double* elpd, double* lppd, float* khat,
+                     double* lw, long long ldw, void* stream) {
+  if (!lw || ldw < S) return SPMF_ERR_BAD_ARG;
+  return psis_loo_launch(ll, ld, nrows, S, elpd, lppd, khat, lw, ldw, stream);
 }
 
 }  // extern "C"

@@ -64,6 +64,8 @@ def waic_terms(ll):
 
 
 LOO_DRAW_CHUNK = 64     # surrogate draws loo() regenerates at a time (bounds its engine memory whatever S is)
+LOO_PIT_ACC_BYTES = 1 << 30      # loo_pit()'s default batch keeps its (B, D, 2) fp64 accumulator within 1 GiB
+LOO_PIT_VALUES_LIMIT = 1 << 27   # entries loo_pit_values() returns at most (2 GiB of (P-, P+) pairs)
 
 
 def loo_compare(a, b):
@@ -695,15 +697,7 @@ class PoissonFactorization:
         tensors 'elpd_loo', 'p_loo' (float64) and 'khat' (float32) of shape (N,), in row order.  Sums over rows
         run in batch order."""
         batches = self._batches_of(data, batch_size, "loo()")
-        if params:
-            theta = {k: torch.as_tensor(params[k]) for k in ('s', 'u', 'v', 'w')}
-            if theta['u'].dim() == 2:
-                theta = {k: t[None] for k, t in theta.items()}
-            S = theta['u'].shape[0]
-        else:
-            theta, S = None, int(sample_size)
-        if not 1 <= S <= _abi.LOO_MAX_S:
-            raise ValueError(f"loo() takes 1 to {_abi.LOO_MAX_S} draws, got {S}")
+        theta, S = self._loo_draws(sample_size, params, "loo()")
         dev, f64 = self.device, torch.float64
         acc = torch.zeros(4, dtype=f64, device=dev)     # elpd, elpd^2, lppd, p_loo
         elpd_all, ploo_all, khat_all = [], [], []
@@ -748,6 +742,144 @@ class PoissonFactorization:
                 self._operands_from_theta(eng, *(theta[k][c0:c0 + nc] for k in ('u', 'v', 'w', 's')))
             ll[:, c0:c0 + nc].copy_(self._row_ll(eng, b).t())
         return ll
+
+    # ------------------------------------------------------------------ LOO-PIT
+    def _loo_draws(self, sample_size, params, who):
+        """(theta, S) of loo() and loo_pit(): explicit draws (leading sample axis) or `sample_size` surrogate draws."""
+        if params:
+            theta = {k: torch.as_tensor(params[k]) for k in ('s', 'u', 'v', 'w')}
+            if theta['u'].dim() == 2:
+                theta = {k: t[None] for k, t in theta.items()}
+            S = theta['u'].shape[0]
+        else:
+            theta, S = None, int(sample_size)
+        if not 1 <= S <= _abi.LOO_MAX_S:
+            raise ValueError(f"{who} takes 1 to {_abi.LOO_MAX_S} draws, got {S}")
+        return theta, S
+
+    def _loo_pit_batch(self, b, S, seed, theta, rates=None):
+        """(P-, P+) of every entry of batch `b` in an fp64 (B, D, 2) tensor, the per-entry invalid draw counts
+        (B, D) and the batch's (elpd, khat): _loo_row_ll, spmf_psis_loo_lw, then a second pass over the same draw
+        chunks that regenerates the operands, densifies and encodes the batch as _ppc_pass does and calls
+        spmf_loo_pit_accum (csrc/spmf_pit.cu).  `rates` (a list, for checking): receives every chunk's (n_c, B, D)
+        fp32 rates as the kernel formed them."""
+        if self._custom_link:
+            raise _abi.SpmfError("LOO-PIT has no CUDA path for custom encoder / decoder callables")
+        dev, f64, B, D = self.device, torch.float64, b.nrows, self.feature_dim
+        ll = self._loo_row_ll(b, S, seed, theta)
+        lw = torch.empty(B, S, dtype=f64, device=dev)
+        elpd = torch.empty(B, dtype=f64, device=dev)
+        lppd = torch.empty(B, dtype=f64, device=dev)
+        khat = torch.empty(B, dtype=torch.float32, device=dev)
+        st = _stream()
+        _abi.call("spmf_psis_loo_lw", _ptr(ll), S, B, S, _ptr(elpd), _ptr(lppd), _ptr(khat), _ptr(lw), S, st)
+        del ll
+        acc = torch.zeros(B, D, 2, dtype=f64, device=dev)
+        inv = torch.zeros(B, D, dtype=torch.int32, device=dev)
+        for c, c0 in enumerate(range(0, S, LOO_DRAW_CHUNK)):
+            nc = min(LOO_DRAW_CHUNK, S - c0)
+            eng = self._engine_for(nc)
+            if theta is None:
+                eng.fill_noise(step=int(seed) + c, which=AdviEngine.NOISE_NORMAL, advance=False)
+                eng.draw_operands()
+            else:
+                self._operands_from_theta(eng, *(theta[k][c0:c0 + nc] for k in ('u', 'v', 'w', 's')))
+            eng.ensure_rows(B)
+            xd = eng.dense_scratch(B)
+            ws = eng.ws
+            eng.dense_scatter(b, xd)
+            if self.link & 1:              # log(x/eta + 1) encoder: dense kernel, as encode()
+                eng.dense_encode(b, xd)
+            else:
+                _abi.call("spmf_csr_encode", _ptr(b.rowptr), _ptr(b.cols), _ptr(b.vals), _ptr(b.rowsum),
+                          eng.inv_xi, int(self.scale_rows), B, D, self.latent_dim, nc, _ptr(ws.Ap), _ptr(ws.z), st)
+            rate = None if rates is None else torch.empty(nc, B, D, dtype=torch.float32, device=dev)
+            _abi.call("spmf_loo_pit_accum", _ptr(xd), B, D, self.latent_dim, nc, self.link, _ptr(ws.EV), _ptr(ws.PH),
+                      _ptr(ws.z), _ptr(lw) + 8 * c0, S, _ptr(acc), _ptr(inv), _ptr(rate), st)
+            if rates is not None:
+                rates.append(rate)
+        return acc, inv, elpd, khat
+
+    def loo_pit(self, data=None, sample_size=1000, batch_size=None, seed=12345, bins=20, **params):
+        """LOO-PIT calibration check (Gabry et al. 2019): the probability integral transform of every entry
+        (row, feature) under the leave-one-ROW-out predictive, which PSIS-LOO approximates by weighting the posterior
+        draws with the row's Pareto-smoothed importance weights.  For counts the PIT is non-randomised (Czado,
+        Gneiting & Held 2009): entry (b, d) has P- = sum_s w_bs F(x_bd - 1 | theta_s) and P+ = sum_s w_bs
+        F(x_bd | theta_s), and its PIT is uniform on [P-, P+].  Under a calibrated model the PIT values are uniform:
+        a U-shaped histogram means the data are over-dispersed against the predictive, a hump under-dispersed, a
+        tilt biased.  Zeros are included.  The (S, B, D) rates are never materialised: a fused CUDA pass
+        (csrc/spmf_pit.cu) weights each entry's CDFs as it forms them.
+
+        `data`, the draws, their chunking and seeds are exactly loo()'s, so the weights are those loo() reports k-hat
+        for.  `batch_size` cuts a CsrShard; by default it keeps the (B, D, 2) fp64 accumulator at or below 1 GiB.
+        `bins` = J, 1 to LOO_PIT_MAX_BINS.  Neither rng_step nor opt_step moves.  Under torch.distributed each rank
+        checks its own shard.  Custom encoder / decoder callables raise SpmfError.
+
+        Returns a dict:
+          'hist' (J,), 'col_hist' (D, J): summed PIT distributions of the valid entries (bin j covers (j/J, (j+1)/J]);
+          'n', 'col_n' (D,): valid entries;  'col_mean_pit' (D,): their mean PIT (P- + P+)/2;
+          'ecdf_dev', 'col_ecdf_dev' (D,): max_j |cumulative histogram_j / n - (j+1)/J|, overall and per feature;
+          'n_invalid': entries left out because a draw gave an invalid rate / logit or the count is not in the
+                       support (see posterior_predictive_check), in the rows not excluded;
+          'n_rows_excluded': rows whose elpd is not finite (their weights are undefined: all their entries);
+          'khat_threshold', 'n_khat_above': as loo() defines them -- these rows' weights are used, and counted.
+        Device tensors are float64 (col_n int64).  Sums over the rows run in batch order."""
+        if self._custom_link:
+            raise _abi.SpmfError("LOO-PIT has no CUDA path for custom encoder / decoder callables")
+        J = int(bins)
+        if not 1 <= J <= _abi.LOO_PIT_MAX_BINS:
+            raise ValueError(f"loo_pit() takes 1 to {_abi.LOO_PIT_MAX_BINS} bins, got {bins}")
+        D, dev, f64 = self.feature_dim, self.device, torch.float64
+        if batch_size is None:
+            batch_size = max(1, LOO_PIT_ACC_BYTES // (16 * D))
+        batches = self._batches_of(data, batch_size, "loo_pit()")
+        theta, S = self._loo_draws(sample_size, params, "loo_pit()")
+        col_hist = torch.zeros(D, J, dtype=f64, device=dev)
+        col_n = torch.zeros(D, dtype=torch.int64, device=dev)
+        col_pit = torch.zeros(D, dtype=f64, device=dev)
+        threshold = min(1.0 - 1.0 / math.log10(S), 0.7) if S > 1 else -math.inf
+        n_invalid = n_excl = n_khat = rows = 0
+        for batch in batches:
+            b = self._csr_batch(batch, "loo_pit()")
+            if b.nrows == 0:
+                continue
+            acc, inv, elpd, khat = self._loo_pit_batch(b, S, seed, theta)
+            scratch = torch.empty(_abi._lib.spmf_loo_pit_hist_scratch_doubles(b.nrows, D, J), dtype=f64, device=dev)
+            _abi.call("spmf_loo_pit_hist", _ptr(acc), _ptr(inv), b.nrows, D, J, _ptr(col_hist), _ptr(col_n),
+                      _ptr(col_pit), _ptr(scratch), _stream())
+            ok = torch.isfinite(elpd)
+            n_invalid += int(((inv != 0) & ok[:, None]).sum())
+            n_excl += int((~ok).sum())
+            n_khat += int((khat > threshold).sum())
+            rows += b.nrows
+        if rows == 0:
+            raise ValueError("loo_pit(): the data holds no rows")
+        hist = col_hist.sum(0)
+        n = int(col_n.sum())
+        edges = torch.arange(1, J + 1, dtype=f64, device=dev) / J
+
+        def ecdf_dev(h, cnt):
+            return (h.cumsum(-1) / cnt.unsqueeze(-1) - edges).abs().amax(-1)
+        cn = col_n.to(f64)
+        return {'hist': hist, 'col_hist': col_hist, 'n': n, 'col_n': col_n,
+                'col_mean_pit': col_pit / cn,
+                'ecdf_dev': float(ecdf_dev(hist, torch.tensor(float(n), dtype=f64, device=dev))),
+                'col_ecdf_dev': ecdf_dev(col_hist, cn),
+                'n_invalid': n_invalid, 'n_rows_excluded': n_excl,
+                'khat_threshold': threshold, 'n_khat_above': n_khat}
+
+    def loo_pit_values(self, batch, sample_size=1000, seed=12345, **params):
+        """The (B, D, 2) fp64 device tensor of (P-, P+) of every entry of one batch, from the kernels of loo_pit()
+        with the same draws and weights.  Entries left out by loo_pit() hold NaN: an invalid draw or count, or a
+        row whose elpd is not finite.  Raises ValueError above LOO_PIT_VALUES_LIMIT (2^27) entries."""
+        b = self._csr_batch(batch, "loo_pit_values()")
+        if b.nrows * self.feature_dim > LOO_PIT_VALUES_LIMIT:
+            raise ValueError(f"{b.nrows} x {self.feature_dim} entries exceed the limit of {LOO_PIT_VALUES_LIMIT}: "
+                             "use loo_pit(), or fewer rows")
+        theta, S = self._loo_draws(sample_size, params, "loo_pit_values()")
+        acc, inv, elpd, khat = self._loo_pit_batch(b, S, seed, theta)
+        bad = (inv != 0) | ~torch.isfinite(elpd)[:, None]
+        return acc.masked_fill_(bad[..., None], math.nan)
 
     def _batches_of(self, data, batch_size, who):
         """The batches of `data` for the evaluation passes: a CsrShard cut into `batch_size` rows (default
